@@ -309,6 +309,33 @@ def run_reference(args, name):
     print(json.dumps(line), flush=True)
 
 
+DUMP_LIMIT_BYTES = 64_000_000      # --dump-outputs: every file together, .npy headers included
+DUMP_SAMPLE_SEED = 2026
+
+
+def dump_outputs(out, path):
+    """Writes the arrays a caller of ob.bootstrap receives (the dict of one step) as <path>/<name>.npy in float64, so
+    that two builds can be compared output for output; total_gap and n_ok become 0-d arrays.  An array that does not
+    fit the share of DUMP_LIMIT_BYTES left to it is replaced by a seeded sample of its flattened elements (sorted
+    indices, the same on every run of the same workload).  Returns {name: [elements written, elements]} of those."""
+    arrays = {k: np.asarray(v, dtype=np.float64) for k, v in out.items()
+              if isinstance(v, np.ndarray) or k in ("total_gap", "n_ok")}
+    os.makedirs(path, exist_ok=True)
+    left = DUMP_LIMIT_BYTES - 128 * len(arrays)        # 128 bytes of .npy header per file at these ranks
+    names = sorted(arrays, key=lambda k: (arrays[k].size, k))
+    sampled = {}
+    for i, k in enumerate(names):
+        a = arrays[k]
+        cap = left // a.itemsize // (len(names) - i)   # the smaller arrays before it have left their unused share
+        if a.size > cap:
+            idx = np.sort(np.random.default_rng(DUMP_SAMPLE_SEED).choice(a.size, cap, replace=False))
+            sampled[k] = [int(cap), int(a.size)]
+            a = a.reshape(-1)[idx]
+        np.save(os.path.join(path, k + ".npy"), a)
+        left -= a.nbytes
+    return sampled
+
+
 def readme_shape_gpu(ob, ctx):
     """Same README shape end to end on the GPU (host columns -> pack -> point + 500 replicates -> results), best of 3."""
     from oaxaca_blinder_rs_b200 import synth
@@ -579,7 +606,15 @@ def main():
                          "row shards (rowshard: mode N, a rank never needs the other rows); auto = rowshard")
     ap.add_argument("--also", default="auto", choices=["auto", "on", "off"],
                     help="N > 1: also measure the row-sharded config 5 and the RIF config 4 at the same N (key `also`)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last of them returned (point statistics, SE / p / CI / t, "
+                         "coefficients, means, residuals) as DIR/<name>.npy in float64, at most 64 MB in all: arrays "
+                         "beyond that are a fixed seeded sample.  Rank 0 only")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the b200 path")
     name = args.workload
     if args.impl == "reference":
         return run_reference(args, name)
@@ -711,6 +746,11 @@ def main():
     sampler.stop_flag.set()
     sampler.step_flag.set()
     sampler.join()
+    if args.dump_outputs and rank == 0:
+        # here, before the legs below write into the same page-locked residuals buffer
+        sampled = dump_outputs(out, args.dump_outputs)
+        print(f"bench: outputs of timed step {args.steps} in {args.dump_outputs}"
+              + (f"; sampled (written, of): {sampled}" if sampled else ""), file=sys.stderr, flush=True)
     design.close()
 
     # ---- end-to-end leg: pinned host columns -> H2D + pack + bootstrap + D2H, every step ----

@@ -1,8 +1,8 @@
 """The C-ABI library loads without a GPU and exports every symbol include/obboot.h declares (no compute calls)."""
 import os
 import re
-
-import pytest
+import subprocess
+import sys
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
@@ -26,14 +26,17 @@ def test_library_exports_every_declared_symbol():
 
 
 def test_no_cpu_fallback():
-    """Without a CUDA device every compute entry point must fail loudly (never route to the oracle)."""
-    import torch
-    if torch.cuda.is_available():
-        pytest.skip("GPU present")
-    import oaxaca_blinder_rs_b200 as ob
-    with pytest.raises(ob.OaxacaError) as e:
-        ob.Context(0)
-    assert e.value.kind == "NoDevice"
+    """Without a CUDA device every compute entry point must fail loudly (never route to the oracle).  Checked in a
+    child process that sees no device, so that it holds on GPU machines too."""
+    code = ("import oaxaca_blinder_rs_b200 as ob\n"
+            "try:\n"
+            "    ob.Context(0)\n"
+            "except ob.OaxacaError as e:\n"
+            "    print(e.kind)\n")
+    r = subprocess.run([sys.executable, "-c", code], cwd=ROOT, env={**os.environ, "CUDA_VISIBLE_DEVICES": ""},
+                       capture_output=True, text=True, timeout=300)
+    assert r.returncode == 0, r.stderr
+    assert r.stdout.strip() == "NoDevice", (r.stdout, r.stderr)
 
 
 def test_product_never_imports_the_oracle():
