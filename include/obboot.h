@@ -268,6 +268,34 @@ int32_t ob_num_stats(int32_t K, int32_t n_norm, const int32_t* norm_has_base);
 
 ob_status ob_bootstrap_run(ob_ctx* ctx, const ob_design* design, const ob_boot_opts* opts, ob_result* res);
 
+/* ---- outcome sweeps over fixed resamples: the per-replicate Gram cache --------------------------------------------
+ * The replicates of the native stream depend only on (seed, global replicate id, group sizes), so re-running the
+ * bootstrap on the same design with a new outcome (ob_design_update_outcome, ob_design_apply_rif*) resamples exactly the
+ * same rows: every replicate's X'WX is unchanged, only X'Wy is new.  A cache keeps, for every slot of a run (the point
+ * estimate and this rank's replicates) and both groups, the reduced X'WX upper triangle and the X'Wy cells of the last
+ * outcome.  ob_bootstrap_run_cached takes the same inputs and returns the same outputs as ob_bootstrap_run, bit for bit;
+ * it contracts only what the cache does not hold:
+ *   OB_CACHE_FILLED        nothing reusable (another design, X / weights / row shard changed, another seed, reps, replicate
+ *                          range or sharding): the full contraction, the cache is (re)filled;
+ *   OB_CACHE_OUTCOME_ONLY  X'WX reusable: only the K T + 1 outcome columns are contracted (also when T changed);
+ *   OB_CACHE_SOLVE_ONLY    X'WX and the outcome unchanged (another ref_kind or normalisation): no resampling and no
+ *                          contraction, only the solves and the reduction.
+ * ref_kind, normalisation, skip_reduce, max_workspace_bytes and count_bits are not part of the key.  Explicit index
+ * streams and designs with a selection equation are refused (OB_ERR_UNSUPPORTED); a cache belongs to the context that
+ * created it (another context: OB_ERR_INVALID_ARG).  A call that fails leaves the cache empty.  Sharded runs (mode R and
+ * mode N) agree on the use over the communicator, every rank takes the same path.  The device memory (about
+ * 16 K(K+1)/2 + 16 (K T + 1) bytes per slot, from the context's design pool) is released by ob_gram_cache_destroy or by
+ * ob_ctx_destroy, whichever comes first; a cache outliving its context only frees its host struct. */
+typedef struct ob_gram_cache ob_gram_cache;
+typedef enum { OB_CACHE_NONE = 0, OB_CACHE_FILLED = 1, OB_CACHE_OUTCOME_ONLY = 2, OB_CACHE_SOLVE_ONLY = 3 } ob_cache_use;
+ob_status ob_gram_cache_create(ob_ctx* ctx, ob_gram_cache** out);
+void ob_gram_cache_destroy(ob_gram_cache* c);
+/* what the last ob_bootstrap_run_cached on c did (ob_cache_use; OB_CACHE_NONE before the first call or after a failed one)
+ * and the device memory the cache holds */
+ob_status ob_gram_cache_last_use(const ob_gram_cache* c, int32_t* use, int64_t* bytes);
+ob_status ob_bootstrap_run_cached(ob_ctx* ctx, const ob_design* design, const ob_boot_opts* opts, ob_gram_cache* cache,
+                                  ob_result* res);
+
 /* Reduction alone, on host arrays gathered from several shards, in replicate order
  * (process_component, builder.rs:849-865): out arrays [S] each. */
 ob_status ob_reduce_stats(ob_ctx* ctx, const double* rep_stats, const int32_t* rep_status, int64_t reps, int32_t S,
@@ -403,6 +431,10 @@ int64_t ob_debug_gram_schedule(int32_t K, int64_t n_a, int64_t n_b, int64_t slot
  * Returns the table length (tiles x 128) or -1 on bad arguments. */
 int64_t ob_debug_gram_columns(int32_t K, int32_t T, int32_t n_cont, const int32_t* cat_levels, int32_t n_cat,
                               uint16_t* pairs_out, int32_t* colmap_out, int64_t cap, int32_t* tiling_out);
+/* The same for the outcome-only contraction of ob_bootstrap_run_cached (OB_CACHE_OUTCOME_ONLY): the K T columns of X'Wy
+ * and the (y_0, y_0) cell, in the order of the full table, tiled like it. */
+int64_t ob_debug_gram_outcome_columns(int32_t K, int32_t T, uint16_t* pairs_out, int32_t* colmap_out, int64_t cap,
+                                      int32_t* tiling_out);
 
 /* Multiplicity counts of one replicate of the native stream (for the statistical validation
  * tests): counts_out [n] for group g (0 = A, 1 = B) of design d. */

@@ -49,6 +49,11 @@ ob_status ob_builder_device(ob_builder* b, int32_t device);
 ob_status ob_builder_index_stream(ob_builder* b, const uint32_t* idx_a, const uint32_t* idx_b);
 
 ob_status ob_builder_run(ob_builder* b, ob_results** out);
+/* run() once per outcome column names[n] (f64 columns) on ONE ingest: rows are cleaned over every listed column (plus the
+ * configured ones), the first run fills a per-replicate Gram cache and the others contract only their outcome columns
+ * (ob_bootstrap_run_cached).  outs[n] receives one results object per outcome, each equal to run() with that column as
+ * the outcome when the columns share their nulls.  Unsupported with heckman_selection or index_stream. */
+ob_status ob_builder_run_outcomes(ob_builder* b, const char* const* names, int32_t n, ob_results** outs);
 ob_status ob_builder_decompose_quantile(ob_builder* b, double quantile, ob_results** out);
 /* get_data_matrices(): sizes first (any out pointer may be NULL), then the row-major copies */
 ob_status ob_builder_get_data_matrices(ob_builder* b, int64_t* n_a, int64_t* n_b, int32_t* k,

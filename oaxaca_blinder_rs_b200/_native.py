@@ -30,7 +30,8 @@ SYMBOLS = ["ob_abi_version", "ob_device_count", "ob_ctx_create", "ob_ctx_destroy
            "ob_host_register", "ob_host_unregister", "ob_replicate_shard", "ob_design_pack_async", "ob_design_wait",
            "ob_design_redistribute_rows", "ob_design_row_shard", "ob_design_apply_rif_multi", "ob_design_num_outcomes",
            "ob_design_pack_row_shard_async", "ob_design_attach_selection", "ob_design_selection_cols", "ob_num_stats_heckman",
-           "ob_mm_run", "ob_debug_gram_columns"]
+           "ob_mm_run", "ob_debug_gram_columns", "ob_gram_cache_create", "ob_gram_cache_destroy", "ob_gram_cache_last_use",
+           "ob_bootstrap_run_cached", "ob_debug_gram_outcome_columns"]
 
 
 class FrameView(C.Structure):
@@ -128,6 +129,13 @@ def lib() -> C.CDLL:
         L.ob_num_stats.argtypes = [C.c_int32, C.c_int32, _IP]
         L.ob_num_stats.restype = C.c_int32
         L.ob_bootstrap_run.argtypes = [C.c_void_p, C.c_void_p, C.POINTER(BootOpts), C.POINTER(Result)]
+        L.ob_gram_cache_create.argtypes = [C.c_void_p, C.POINTER(C.c_void_p)]
+        L.ob_gram_cache_destroy.argtypes = [C.c_void_p]
+        L.ob_gram_cache_destroy.restype = None
+        L.ob_gram_cache_last_use.argtypes = [C.c_void_p, _IP, C.POINTER(C.c_int64)]
+        L.ob_bootstrap_run_cached.argtypes = [C.c_void_p, C.c_void_p, C.POINTER(BootOpts), C.c_void_p, C.POINTER(Result)]
+        L.ob_debug_gram_outcome_columns.argtypes = [C.c_int32, C.c_int32, C.POINTER(C.c_uint16), _IP, C.c_int64, _IP]
+        L.ob_debug_gram_outcome_columns.restype = C.c_int64
         L.ob_reduce_stats.argtypes = [C.c_void_p, _DP, _IP, C.c_int64, C.c_int32, _DP, C.POINTER(C.c_int64),
                                       _DP, _DP, _DP, _DP, _DP]
         L.ob_debug_counts.argtypes = [C.c_void_p, C.c_void_p, C.c_uint64, C.c_int64, C.c_int32,

@@ -17,7 +17,7 @@ import ctypes as C
 import enum
 import json
 from types import SimpleNamespace
-from typing import Iterable, Optional, Sequence
+from typing import Iterable, List, Optional, Sequence
 
 import numpy as np
 
@@ -60,6 +60,7 @@ def _blib():
         L.ob_builder_device.argtypes = [vp, i32]
         L.ob_builder_index_stream.argtypes = [vp, N._U32P, N._U32P]
         L.ob_builder_run.argtypes = [vp, C.POINTER(vp)]
+        L.ob_builder_run_outcomes.argtypes = [vp, C.POINTER(cp), i32, C.POINTER(vp)]
         L.ob_builder_decompose_quantile.argtypes = [vp, C.c_double, C.POINTER(vp)]
         L.ob_builder_get_data_matrices.argtypes = [vp, C.POINTER(i64), C.POINTER(i64), C.POINTER(i32), N._DP, N._DP, N._DP, N._DP]
         L.ob_builder_last_error.argtypes = [vp]; L.ob_builder_last_error.restype = cp
@@ -95,7 +96,7 @@ BUILDER_SYMBOLS = ["ob_frame_new", "ob_frame_free", "ob_frame_add_f64", "ob_fram
                    "ob_builder_new", "ob_builder_from_formula", "ob_builder_free", "ob_builder_predictors",
                    "ob_builder_categorical_predictors", "ob_builder_normalize", "ob_builder_weights",
                    "ob_builder_bootstrap_reps", "ob_builder_reference_coefficients", "ob_builder_heckman_selection",
-                   "ob_builder_seed", "ob_builder_device", "ob_builder_index_stream", "ob_builder_run",
+                   "ob_builder_seed", "ob_builder_device", "ob_builder_index_stream", "ob_builder_run", "ob_builder_run_outcomes",
                    "ob_builder_decompose_quantile", "ob_builder_get_data_matrices", "ob_builder_describe", "ob_builder_last_error", "ob_builder_last_status",
                    "ob_results_free", "ob_results_json", "ob_results_summary", "ob_results_markdown",
                    "ob_results_residuals",
@@ -310,6 +311,16 @@ class OaxacaBuilder:
         out = C.c_void_p()
         self._check(_blib().ob_builder_run(self._h, C.byref(out)))
         return OaxacaResults(out)
+
+    def run_outcomes(self, outcomes) -> List["OaxacaResults"]:
+        """run() once per listed outcome column on one ingest of the frame: rows are cleaned over every listed column, the
+        first run fills a per-replicate Gram cache and the others contract only their outcome columns.  When the columns
+        share their nulls, result k equals run() with outcomes[k] as the outcome."""
+        names = [str(o) for o in outcomes]
+        arr = (C.c_char_p * max(len(names), 1))(*[o.encode() for o in names])
+        outs = (C.c_void_p * max(len(names), 1))()
+        self._check(_blib().ob_builder_run_outcomes(self._h, arr, len(names), outs))
+        return [OaxacaResults(C.c_void_p(outs[k])) for k in range(len(names))]
 
     def decompose_quantile(self, quantile: float) -> OaxacaResults:  # builder.rs:711
         out = C.c_void_p()

@@ -116,6 +116,48 @@ def row_shard_plan(n_group: int, world: int, rank: int):
     return b.value, e.value
 
 
+CACHE_NONE, CACHE_FILLED, CACHE_OUTCOME_ONLY, CACHE_SOLVE_ONLY = 0, 1, 2, 3
+CACHE_USE_NAMES = {CACHE_NONE: "none", CACHE_FILLED: "filled", CACHE_OUTCOME_ONLY: "outcome_only", CACHE_SOLVE_ONLY: "solve_only"}
+
+
+class GramCache:
+    """ob_gram_cache: every replicate's X'WX (and the last outcome's X'Wy) of one bootstrap configuration, kept in HBM.
+    Pass it to bootstrap(..., cache=) on the same design across outcome changes (update_outcome, apply_rif*): the results
+    are those of an uncached call bit for bit, while only the outcome columns of the Gram are contracted again."""
+
+    def __init__(self, ctx: Context):
+        self.ctx = ctx
+        self._h = C.c_void_p()
+        ctx.check(N.lib().ob_gram_cache_create(ctx._h, C.byref(self._h)))
+
+    def _query(self):
+        use, nbytes = C.c_int32(), C.c_int64()
+        N.lib().ob_gram_cache_last_use(self._h, C.byref(use), C.byref(nbytes))
+        return use.value, nbytes.value
+
+    @property
+    def last_use(self) -> int:
+        """What the last cached bootstrap did: CACHE_FILLED, CACHE_OUTCOME_ONLY, CACHE_SOLVE_ONLY (CACHE_NONE: no call yet,
+        or the last one failed)."""
+        return self._query()[0]
+
+    @property
+    def bytes(self) -> int:
+        """Device memory the cache holds."""
+        return self._query()[1]
+
+    def close(self):
+        if self._h:
+            N.lib().ob_gram_cache_destroy(self._h)
+            self._h = C.c_void_p()
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+
 @dataclass
 class NormVar:
     m: int
@@ -439,8 +481,8 @@ def bootstrap(design: Design, reps: int, ref_kind: int = REF_GROUP_A, norm: Sequ
               seed: int = 0, idx_a=None, idx_b=None, rep_begin: int = 0, rep_end: int = 0,
               skip_reduce: bool = False, count_bits: int = 0, max_workspace_bytes: int = 0,
               want_rep: bool = False, want_residuals: bool = True, residuals_out: Optional[np.ndarray] = None,
-              shard_replicates: bool = False) -> dict:
-    """ob_bootstrap_run.  Returns point estimates, per-statistic SE/p/CI/t and (optionally) replicate detail.
+              shard_replicates: bool = False, cache: Optional[GramCache] = None) -> dict:
+    """ob_bootstrap_run (ob_bootstrap_run_cached with a GramCache: same results, and `cache_use` in the dict).  Returns point estimates, per-statistic SE/p/CI/t and (optionally) replicate detail.
     residuals_out: optional preallocated float64 [n_b] buffer for OaxacaResults.residuals (reusing one across calls
     avoids first-touch page faults on a fresh 8 n_b byte array during the device-to-host copy; a page-locked one --
     pinned_empty() -- takes the DMA directly).
@@ -494,10 +536,15 @@ def bootstrap(design: Design, reps: int, ref_kind: int = REF_GROUP_A, norm: Sequ
     for k, v in a.items():
         setattr(r, k, _ip(v) if v.dtype == np.int32 else _dp(v))
     try:
-        ctx.check(N.lib().ob_bootstrap_run(ctx._h, design._h, C.byref(o), C.byref(r)))
+        if cache is None:
+            ctx.check(N.lib().ob_bootstrap_run(ctx._h, design._h, C.byref(o), C.byref(r)))
+        else:
+            ctx.check(N.lib().ob_bootstrap_run_cached(ctx._h, design._h, C.byref(o), cache._h, C.byref(r)))
     finally:
         design._inflight = None        # an asynchronous pack has completed (or failed) by now
     out = dict(a)
+    if cache is not None:
+        out["cache_use"] = cache.last_use
     for k in ("rep_stats", "rep_status", "rep_beta_a", "rep_beta_b"):
         if k in out:
             out[k] = out[k][:nrep]

@@ -11,6 +11,7 @@
 #include <cstdio>
 #include <cstring>
 #include <memory>
+#include <atomic>
 #include <mutex>
 #include <set>
 
@@ -42,6 +43,7 @@ struct ob_ctx {
     // finalising objects in arbitrary order, possibly on another thread -- only frees the host struct.
     std::mutex designs_mu;
     std::set<ob_design*> designs;
+    std::set<ob_gram_cache*> caches;     // Gram caches of this context, orphaned the same way (under designs_mu)
 };
 
 struct ob_local_group { LocalGroup* g = nullptr; int world = 0; };
@@ -65,6 +67,28 @@ struct ob_design {
     int world = 1, rank = 0;         // row sharding (mode N): this design holds rank's rows of a world-way split
     double ms_h2d = 0.0, ms_pack = 0.0;   // device time of the column upload and of the pack kernels (ob_design_pack)
     GroupData g[2];
+    // identity for ob_gram_cache keys: a process-wide unique id (addresses are reused after destroy), the generation of
+    // the design columns / weights / rows / row-shard marking, and the generation of the outcome columns
+    uint64_t id = 0, x_gen = 0, y_gen = 0;
+};
+
+// ob_bootstrap_run_cached: the reduced Gram cells of every slot of a run, kept in HBM for the next run on the same
+// resamples (layouts: gram_cache_map in gram.cu)
+struct ob_gram_cache {
+    ob_ctx* owner = nullptr;         // context that created the cache; null once that context has been destroyed
+    int device = 0;
+    int last_use = OB_CACHE_NONE;
+    double* xx = nullptr; size_t xx_bytes = 0;   // [2][slots][K(K+1)/2]
+    double* yy = nullptr; size_t yy_bytes = 0;   // [2][slots][K T + 1]
+    // key of xx (valid while xx_ok): what decides the resamples and the design's X'WX
+    bool xx_ok = false;
+    uint64_t design_id = 0, x_gen = 0, seed = 0;
+    int64_t reps = 0, rep_begin = 0, rep_end = 0, slots = 0;
+    int shard_reps = 0, rep_world = 1, rep_rank = 0, row_world = 1, row_rank = 0, K = 0;
+    int count_bytes = 1;             // multiplicity width the fill ended with (a saturation already known)
+    // key of yy (valid while y_ok): the design's outcome generation and outcome count
+    bool y_ok = false;
+    uint64_t y_gen = 0; int T = 0;
 };
 
 namespace {
@@ -219,6 +243,8 @@ void alloc_group(ob_ctx* ctx, GroupData& g, int64_t n, int ldx, bool weighted, b
 }
 
 void design_register(ob_ctx* ctx, ob_design* d) {
+    static std::atomic<uint64_t> next_id{0};
+    d->id = ++next_id;
     d->owner = ctx;
     std::lock_guard<std::mutex> lk(ctx->designs_mu);
     ctx->designs.insert(d);
@@ -237,6 +263,17 @@ void design_release_device(ob_design* d) {
         if (g.hk_Xm) cudaFreeAsync(g.hk_Xm, st);
         g.X = g.w = g.Xs = g.y_raw = g.hk_Z = g.hk_Xm = nullptr; g.src = nullptr; g.hk_sel = nullptr;
     }
+}
+
+// empties a Gram cache (its device memory goes back to the owner's design pool)
+void cache_release_device(ob_gram_cache* c) {
+    if (c->owner) {
+        cudaStream_t st = c->owner->stream;
+        if (c->xx) cudaFreeAsync(c->xx, st);
+        if (c->yy) cudaFreeAsync(c->yy, st);
+    }
+    c->xx = c->yy = nullptr; c->xx_bytes = c->yy_bytes = 0;
+    c->xx_ok = c->y_ok = false;
 }
 
 // The one exchange of an asynchronous row-shard pack: every rank sends the rows of its slice that other ranks own (they
@@ -379,6 +416,8 @@ void ob_ctx_destroy(ob_ctx* ctx) {
         std::lock_guard<std::mutex> lk(ctx->designs_mu);
         for (ob_design* d : ctx->designs) { pending_finish(d, true); design_release_device(d); d->owner = nullptr; d->stream = nullptr; }
         ctx->designs.clear();
+        for (ob_gram_cache* c : ctx->caches) { cache_release_device(c); c->owner = nullptr; }
+        ctx->caches.clear();
     }
     if (ctx->stream) cudaStreamSynchronize(ctx->stream);
     if (ctx->stream_side) { cudaStreamSynchronize(ctx->stream_side); cudaStreamDestroy(ctx->stream_side); }
@@ -498,6 +537,7 @@ ob_status ob_design_set_row_shard(ob_design* d, int64_t n_a_global, int64_t n_b_
     if (ra.n_local != d->g[0].n || rb.n_local != d->g[1].n) return OB_ERR_INVALID_ARG;   // rows must follow ob_row_shard_plan
     d->g[0].shard = ra; d->g[1].shard = rb;
     d->world = world; d->rank = rank;
+    ++d->x_gen;
     return OB_OK;
 }
 
@@ -1196,6 +1236,7 @@ ob_status ob_design_update_outcome(ob_ctx* ctx, ob_design* d, const double* y_fr
         if (n_frame != d->n_frame) fail(OB_ERR_INVALID_ARG, "outcome length differs from the frame the design was packed from");
         if (!d->g[0].src || !d->g[1].src) fail(OB_ERR_UNSUPPORTED, "this design carries no frame-row map (gathered design)");
         g_alloc_pack = true;
+        ++d->y_gen;
         DevBuf d_y(sizeof(double) * (size_t)std::max<int64_t>(n_frame, 1));
         OB_CUDA(cudaMemcpyAsync(d_y.p, y_frame, sizeof(double) * (size_t)n_frame, cudaMemcpyHostToDevice, ctx->stream));
         for (int g = 0; g < 2; ++g) {
@@ -1223,6 +1264,7 @@ ob_status ob_design_apply_rif_multi(ob_ctx* ctx, ob_design* d, const double* tau
         if (d->K + n_tau > MAX_DESIGN_COLS) fail(OB_ERR_UNSUPPORTED, "design plus outcome columns wider than 280");
         cudaStream_t st = ctx->stream;
         const int K = d->K;
+        ++d->y_gen;
         const int ldx_new = std::max(d->ldx, design_ldx(K + n_tau));
         for (int g = 0; g < 2; ++g) {
             GroupData& G = d->g[g];
@@ -1860,10 +1902,13 @@ ob_status ob_mm_run(ob_ctx* ctx, const ob_design* d, const ob_mm_opts* o, ob_mm_
     });
 }
 
-ob_status ob_bootstrap_run(ob_ctx* ctx, const ob_design* d, const ob_boot_opts* o, ob_result* res) {
-    if (!ctx || !d || !o || !res) return OB_ERR_INVALID_ARG;
-    return guarded(ctx, [&] {
+// ob_bootstrap_run, and with a cache ob_bootstrap_run_cached: the batch loop contracts the full Gram (no cache, or a
+// cache that is (re)filled), only its outcome columns (OB_CACHE_OUTCOME_ONLY: X'WX comes from the cache) or nothing
+// (OB_CACHE_SOLVE_ONLY: the whole Gram comes from the cache, no multiplicities are generated)
+static void bootstrap_body(ob_ctx* ctx, const ob_design* d, const ob_boot_opts* o, ob_gram_cache* cache, ob_result* res) {
         design_alive(d);
+        if (cache && d->K1 > 0) fail(OB_ERR_UNSUPPORTED, "a Gram cache does not apply to designs with a selection equation (Heckman)");
+        if (cache && (o->idx_a || o->idx_b)) fail(OB_ERR_UNSUPPORTED, "a Gram cache needs the native resampling stream (explicit index streams cannot be keyed)");
         if (d->K1 > 0) {                 // a selection equation is attached: the Heckman two-step estimator per replicate
             design_ready(d);
             heckman_run(ctx, d, o, res);
@@ -1890,6 +1935,27 @@ ob_status ob_bootstrap_run(ob_ctx* ctx, const ob_design* d, const ob_boot_opts* 
             fail(OB_ERR_NCCL, "row-sharded design needs ob_comm_init_* on this context with the same world/rank");
         const int world = d->world;
         int n_base = 0, n_idx = 0;
+        // ---- Gram cache: what of this run the cache already holds ----
+        int mode = OB_CACHE_NONE;
+        const int rep_world = shard_reps ? ctx->comm->world : 1, rep_rank = shard_reps ? ctx->comm->rank : 0;
+        if (cache) {
+            const bool xx_hit = cache->xx_ok && cache->design_id == d->id && cache->x_gen == d->x_gen && cache->seed == o->seed &&
+                                cache->reps == o->reps && cache->rep_begin == rb && cache->rep_end == re &&
+                                cache->shard_reps == (shard_reps ? 1 : 0) && cache->rep_world == rep_world && cache->rep_rank == rep_rank &&
+                                cache->row_world == d->world && cache->row_rank == d->rank && cache->K == d->K &&
+                                !(o->count_bits == 8 && cache->count_bytes == 2);   // that run saturates 8-bit counts: let it fail
+            mode = !xx_hit ? OB_CACHE_FILLED : (cache->y_ok && cache->y_gen == d->y_gen && cache->T == d->T) ? OB_CACHE_SOLVE_ONLY
+                                                                                                           : OB_CACHE_OUTCOME_ONLY;
+            // sharded runs: every rank must run the same collectives -- all take the least reuse any rank can do
+            if (Comm* ac = shard_reps ? ctx->comm.get() : comm) {
+                DevBuf d_mode(sizeof(int));
+                OB_CUDA(cudaMemcpyAsync(d_mode.p, &mode, sizeof(int), cudaMemcpyHostToDevice, ctx->stream));
+                ac->allreduce(d_mode.p, 1, CommDType::I32, CommOp::MIN, ctx->stream);
+                OB_CUDA(cudaMemcpyAsync(&mode, d_mode.p, sizeof(int), cudaMemcpyDeviceToHost, ctx->stream));
+                OB_CUDA(cudaStreamSynchronize(ctx->stream));
+            }
+        }
+        const bool solve_only = mode == OB_CACHE_SOLVE_ONLY, outcome_only = mode == OB_CACHE_OUTCOME_ONLY;
         for (int v = 0; v < o->n_norm; ++v) {
             n_base += o->norm_has_base[v] ? 1 : 0;
             if (o->norm_off[v + 1] < o->norm_off[v]) fail(OB_ERR_INVALID_ARG, "norm_off not monotone");
@@ -1903,6 +1969,7 @@ ob_status ob_bootstrap_run(ob_ctx* ctx, const ob_design* d, const ob_boot_opts* 
         if (index_mode && nrep > 0 && (!o->idx_a || !o->idx_b)) fail(OB_ERR_INVALID_ARG, "index stream needs both idx_a and idx_b");
         if (o->count_bits != 0 && o->count_bits != 8 && o->count_bits != 16) fail(OB_ERR_INVALID_ARG, "count_bits must be 0, 8 or 16");
         int count_bytes = o->count_bits == 16 ? 2 : 1;
+        if (outcome_only && o->count_bits == 0) count_bytes = cache->count_bytes;   // start where the fill ended
 
         res->ms_counts = res->ms_gram = res->ms_solve = res->ms_reduce = res->ms_total = res->ms_gram_kernel = res->ms_comm = 0.0;
         res->gpu_launches = 0;
@@ -1929,8 +1996,30 @@ ob_status ob_bootstrap_run(ob_ctx* ctx, const ob_design* d, const ob_boot_opts* 
         DevBuf d_point(sizeof(double) * PE * T);
         DevBuf d_flags(sizeof(int) * 4);
 
+        // ---- cache storage: allocated by the filling call (and counted in its workspace budget) ----
+        const int nx = gram_cache_xx_cells(K), ny = gram_cache_y_cells(K, T);
+        size_t cache_new_bytes = 0;
+        if (mode == OB_CACHE_FILLED) {
+            cache_release_device(cache);
+            cache->xx_bytes = sizeof(double) * 2 * (size_t)slots * nx;
+            OB_CUDA(cudaMallocFromPoolAsync((void**)&cache->xx, cache->xx_bytes, ctx->pool_design, st));
+            cache_new_bytes += cache->xx_bytes;
+        }
+        if (mode == OB_CACHE_FILLED || outcome_only) {
+            cache->y_ok = false;
+            const size_t yb = sizeof(double) * 2 * (size_t)slots * ny;
+            if (cache->yy_bytes != yb) {          // T changed
+                if (cache->yy) cudaFreeAsync(cache->yy, st);
+                cache->yy = nullptr; cache->yy_bytes = yb;
+                OB_CUDA(cudaMallocFromPoolAsync((void**)&cache->yy, yb, ctx->pool_design, st));
+                cache_new_bytes += yb;
+            }
+        }
+
         // ---- batch the multiplicity matrix by panels under the workspace budget ----
-        const int ntiles = gram_ntiles(K, T);
+        const GramColumns gcols = solve_only ? GramColumns() : outcome_only ? gram_outcome_columns(K, T)
+                                                                              : gram_columns(K, T, d->n_cont, d->cat_levels);
+        const int ntiles = gcols.ntiles;
         const int Pld = gram_pld(K, T);
         const int64_t panels_total = (slots + BM - 1) / BM;
         const int64_t n_pad[2] = {d->g[0].n_pad, d->g[1].n_pad};
@@ -1940,21 +2029,25 @@ ob_status ob_bootstrap_run(ob_ctx* ctx, const ob_design* d, const ob_boot_opts* 
             ranks_with_rows[g] = (d->g[g].shard.segs + d->g[g].shard.leaf_span - 1) / d->g[g].shard.leaf_span;
         const int64_t local_leaves = (int64_t)(d->g[0].shard.leaf_hi - d->g[0].shard.leaf_lo) +
                                      (d->g[1].shard.leaf_hi - d->g[1].shard.leaf_lo);
-        double budget = (double)o->max_workspace_bytes;
+        // workspace of one panel: multiplicities (+ index stream), reduced Gram (+ the mode-N exchange), partial tiles, column
+        // sums; a run that only solves needs the reduced Gram alone
+        auto per_panel_bytes = [&](int cb) {
+            if (solve_only) return 2.0 * BM * Pld * 8.0;
+            return (double)(n_pad[0] + n_pad[1]) * BM * cb + (index_mode ? (double)(n_glob[0] + n_glob[1]) * BM * 4.0 : 0.0) +
+                   2.0 * BM * Pld * 8.0 * (comm ? world + 2 : 1) + (double)local_leaves * ntiles * (BM * BN * 8.0) + 2.0 * BM * 8.0;
+        };
+        double budget = (double)o->max_workspace_bytes - (double)cache_new_bytes;
         if (o->max_workspace_bytes <= 0) {
             // Steady state (the same problem again): the context's pool already holds the whole workspace -> no device
             // query at all.  cudaMemGetInfo takes the driver's global lock and stalls for milliseconds whenever another
             // thread (NVML monitoring, for one) holds it.
             const double idle = (double)pool_idle_bytes(ctx);
-            const double need_all = ((double)(n_pad[0] + n_pad[1]) * BM * count_bytes +
-                                     (index_mode ? (double)(n_glob[0] + n_glob[1]) * BM * 4.0 : 0.0) +
-                                     2.0 * BM * Pld * 8.0 * (comm ? world + 2 : 1) +
-                                     (double)local_leaves * ntiles * (BM * BN * 8.0) + 2.0 * BM * 8.0) * (double)panels_total;
+            const double need_all = per_panel_bytes(count_bytes) * (double)panels_total;
             if (idle >= 1.02 * need_all) budget = 1.01 * need_all;      // every panel in one batch, from memory the pool holds
             else {
                 size_t free_b = 0, total_b = 0;
                 OB_CUDA(cudaMemGetInfo(&free_b, &total_b));
-                budget = 0.6 * ((double)free_b + idle);
+                budget = 0.6 * ((double)free_b + idle) - (double)cache_new_bytes;
             }
         }
         DevBuf d_agree(sizeof(long long)), d_lut(2 * counts_lut_bytes());
@@ -1965,10 +2058,7 @@ ob_status ob_bootstrap_run(ob_ctx* ctx, const ob_design* d, const ob_boot_opts* 
         OB_CUDA(cudaEventCreateWithFlags(&ev_point, cudaEventDisableTiming));
         auto run_batches = [&] {
         for (int attempt = 0; attempt < 2; ++attempt) {  // second attempt only widens uint8 -> uint16 after saturation
-            const double per_panel = (double)(n_pad[0] + n_pad[1]) * BM * count_bytes +
-                                     (index_mode ? (double)(n_glob[0] + n_glob[1]) * BM * 4.0 : 0.0) +
-                                     2.0 * BM * Pld * 8.0 * (comm ? world + 2 : 1) +
-                                     (double)local_leaves * ntiles * (BM * BN * 8.0) + 2.0 * BM * 8.0;
+            const double per_panel = per_panel_bytes(count_bytes);
             int64_t ppb = (int64_t)std::floor(budget / per_panel);
             ppb = std::max<int64_t>(1, std::min<int64_t>(ppb, panels_total));
             if (comm) {   // every rank must cut the same batches: the collectives run once per batch
@@ -1984,12 +2074,19 @@ ob_status ob_bootstrap_run(ob_ctx* ctx, const ob_design* d, const ob_boot_opts* 
             const size_t gram_elems = 2 * (size_t)ppb * BM * Pld;      // [2][slots_pad][Pld]
             bool saturated = false;
             GramPlan plan; int64_t plan_panels = -1;
-            DevBuf d_partials, d_pairs, d_colmap;
-            const GramColumns gcols = gram_columns(K, T, d->n_cont, d->cat_levels);
+            DevBuf d_partials, d_pairs, d_colmap, d_cmap;
             auto allocate_workspace = [&] {
-                d_colsum.alloc(sizeof(long long) * 2 * (size_t)ppb * BM);
-                for (int g = 0; g < 2; ++g) d_C[g].alloc((size_t)ppb * n_pad[g] * BM * count_bytes);
+                if (!solve_only) {
+                    d_colsum.alloc(sizeof(long long) * 2 * (size_t)ppb * BM);
+                    for (int g = 0; g < 2; ++g) d_C[g].alloc((size_t)ppb * n_pad[g] * BM * count_bytes);
+                }
                 d_gram.alloc(sizeof(double) * gram_elems);
+                if (cache) {
+                    const std::vector<int32_t> cmap = gram_cache_map(K, T);
+                    d_cmap.alloc(sizeof(int32_t) * cmap.size());
+                    OB_CUDA(cudaMemcpyAsync(d_cmap.p, cmap.data(), sizeof(int32_t) * cmap.size(), cudaMemcpyHostToDevice, st));
+                }
+                if (solve_only) { OB_CUDA(cudaStreamSynchronize(st)); return; }
                 if (comm) { d_gram_local.alloc(sizeof(double) * gram_elems); d_gathered.alloc(sizeof(double) * gram_elems * world); }
                 plan = gram_make_plan(K, T, d->ldx, (int)std::min<int64_t>(ppb, panels_total), d->g, count_bytes, ctx->num_sms, gcols);
                 plan_panels = plan.panels;
@@ -2040,7 +2137,9 @@ ob_status ob_bootstrap_run(ob_ctx* ctx, const ob_design* d, const ob_boot_opts* 
                     ca[g].panels = (int)pn; ca[g].slots = bslots; ca[g].first_slot = first_slot; ca[g].rep0 = rep0;
                     ca[g].group = g; ca[g].seed = o->seed;
                 }
-                if (index_mode) {
+                if (solve_only) {
+                    // the cache holds every Gram cell of these slots: no multiplicities
+                } else if (index_mode) {
                     for (int g = 0; g < 2; ++g) {
                         const uint32_t* h = (g == 0 ? o->idx_a : o->idx_b);
                         const size_t nb = sizeof(uint32_t) * (size_t)std::max<int64_t>(brep, 1) * n_glob[g];
@@ -2073,7 +2172,7 @@ ob_status ob_bootstrap_run(ob_ctx* ctx, const ob_design* d, const ob_boot_opts* 
                 tr.mark("counts", st, true);
 
                 // (3) Gram / cross-product contraction
-                if (plan_panels != pn) {
+                if (!solve_only && plan_panels != pn) {
                     plan = gram_make_plan(K, T, d->ldx, (int)pn, d->g, count_bytes, ctx->num_sms, gcols);
                     plan_panels = pn;
                     d_partials.alloc(sizeof(double) * (size_t)std::max<int64_t>(plan.num_partials, 1) * BM * BN);
@@ -2094,7 +2193,11 @@ ob_status ob_bootstrap_run(ob_ctx* ctx, const ob_design* d, const ob_boot_opts* 
                     ~EventPair() { if (a) cudaEventDestroy(a); if (b) cudaEventDestroy(b); }
                 } ev;
                 ob_design* dm = const_cast<ob_design*>(d);
-                if (PendingPack* P = dm->pending) {
+                if (solve_only) {
+                    OB_CUDA(cudaEventRecord(ev.a, st));
+                    OB_CUDA(cudaMemsetAsync(d_gram.p, 0, sizeof(double) * 2 * (size_t)pn * BM * Pld, st));
+                    OB_CUDA(cudaEventRecord(ev.b, st));
+                } else if (PendingPack* P = dm->pending) {
                     // the design's upload is still in flight (ob_design_pack_async / _row_shard_async): contract the leaves
                     // whose rows the first chunk delivered, then -- once everything has arrived (row shards: once the rows
                     // owned by other ranks have been exchanged) -- the rest.  Same partial tiles, same fixed-tree sums as
@@ -2143,7 +2246,7 @@ ob_status ob_bootstrap_run(ob_ctx* ctx, const ob_design* d, const ob_boot_opts* 
                 }
                 t_gram.stop();
                 tr.mark("gram", st, true);
-                if (comm) {
+                if (comm && !solve_only) {
                     // every rank's subtree sums -> all ranks; the top of the summation tree is then evaluated in fixed
                     // order on each rank (bit-identical to the single-GPU reduction)
                     Timer t_c(st, &res->ms_comm);
@@ -2152,6 +2255,22 @@ ob_status ob_bootstrap_run(ob_ctx* ctx, const ob_design* d, const ob_boot_opts* 
                     gram_combine_launch(d_gathered.as<double>(), world, ranks_with_rows, (int64_t)pn * BM * Pld, d_gram.as<double>(), st);
                     res->gpu_launches += 1;
                     t_c.stop(); OB_CUDA(cudaStreamSynchronize(st)); t_c.collect();
+                }
+                if (cache) {
+                    // the reduced Gram of these slots is complete (the reduce / combine zeroed it first): fill the cells the
+                    // contraction skipped from the cache, keep the ones it computed
+                    Timer t_cc(st, &res->ms_gram);
+                    GramCacheCopy cc{d_gram.as<double>(), pn * BM, Pld, slot_lo, bslots, cache->xx, cache->yy, slots,
+                                     d_cmap.as<int32_t>(), nx, ny, 0, nx + ny};
+                    if (mode == OB_CACHE_FILLED) gram_cache_extract_launch(cc, st);
+                    else if (solve_only) gram_cache_assemble_launch(cc, st);
+                    else {
+                        cc.c_hi = nx; gram_cache_assemble_launch(cc, st);
+                        cc.c_lo = nx; cc.c_hi = nx + ny; gram_cache_extract_launch(cc, st);
+                        res->gpu_launches += 1;
+                    }
+                    res->gpu_launches += 1;
+                    t_cc.stop(); OB_CUDA(cudaStreamSynchronize(st)); t_cc.collect();
                 }
 
                 // (4) solves + decomposition epilogue
@@ -2217,6 +2336,17 @@ ob_status ob_bootstrap_run(ob_ctx* ctx, const ob_design* d, const ob_boot_opts* 
             if (agreed != OB_OK) fail((ob_status)agreed, std::string("another rank of the replicate-sharded run failed: ") + status_text(agreed));
         } else {
             run_batches();
+        }
+        if (cache) {
+            if (mode == OB_CACHE_FILLED) {
+                cache->design_id = d->id; cache->x_gen = d->x_gen; cache->seed = o->seed;
+                cache->reps = o->reps; cache->rep_begin = rb; cache->rep_end = re; cache->slots = slots;
+                cache->shard_reps = shard_reps ? 1 : 0; cache->rep_world = rep_world; cache->rep_rank = rep_rank;
+                cache->row_world = d->world; cache->row_rank = d->rank; cache->K = K; cache->count_bytes = count_bytes;
+                cache->xx_ok = true;
+            }
+            if (!solve_only) { cache->y_gen = d->y_gen; cache->T = T; cache->y_ok = true; }
+            cache->last_use = mode;
         }
         res->total_gap = point[5 * K];
         if (res->xa_mean) memcpy(res->xa_mean, point.data(), sizeof(double) * K);
@@ -2311,6 +2441,59 @@ ob_status ob_bootstrap_run(ob_ctx* ctx, const ob_design* d, const ob_boot_opts* 
         OB_CUDA(cudaStreamSynchronize(st));
         t_total.collect();
         tr.mark("reduce + replicate D2H", st, false);
+}
+
+ob_status ob_bootstrap_run(ob_ctx* ctx, const ob_design* d, const ob_boot_opts* o, ob_result* res) {
+    if (!ctx || !d || !o || !res) return OB_ERR_INVALID_ARG;
+    return guarded(ctx, [&] { bootstrap_body(ctx, d, o, nullptr, res); });
+}
+
+ob_status ob_gram_cache_create(ob_ctx* ctx, ob_gram_cache** out) {
+    if (!ctx || !out) return OB_ERR_INVALID_ARG;
+    auto* c = new ob_gram_cache;
+    c->owner = ctx; c->device = ctx->device;
+    {
+        std::lock_guard<std::mutex> lk(ctx->designs_mu);
+        ctx->caches.insert(c);
+    }
+    *out = c;
+    return OB_OK;
+}
+
+void ob_gram_cache_destroy(ob_gram_cache* c) {
+    if (!c) return;
+    if (ob_ctx* ctx = c->owner) {      // an orphaned cache (context already destroyed) holds no device memory any more
+        int prev = -1;
+        cudaGetDevice(&prev);
+        cudaSetDevice(c->device);
+        {
+            std::lock_guard<std::mutex> lk(ctx->designs_mu);
+            ctx->caches.erase(c);
+        }
+        cache_release_device(c);
+        if (prev >= 0 && prev != c->device) cudaSetDevice(prev);
+    }
+    delete c;
+}
+
+ob_status ob_gram_cache_last_use(const ob_gram_cache* c, int32_t* use, int64_t* bytes) {
+    if (!c) return OB_ERR_INVALID_ARG;
+    if (use) *use = c->last_use;
+    if (bytes) *bytes = (int64_t)(c->xx_bytes + c->yy_bytes);
+    return OB_OK;
+}
+
+ob_status ob_bootstrap_run_cached(ob_ctx* ctx, const ob_design* d, const ob_boot_opts* o, ob_gram_cache* cache, ob_result* res) {
+    if (!ctx || !d || !o || !cache || !res) return OB_ERR_INVALID_ARG;
+    return guarded(ctx, [&] {
+        if (cache->owner != ctx) fail(OB_ERR_INVALID_ARG, "this Gram cache belongs to another context");
+        try {
+            bootstrap_body(ctx, d, o, cache, res);
+        } catch (...) {          // whatever failed, the next call fills the cache anew
+            cache_release_device(cache);
+            cache->last_use = OB_CACHE_NONE;
+            throw;
+        }
     });
 }
 
@@ -2347,6 +2530,19 @@ int64_t ob_debug_gram_columns(int32_t K, int32_t T, int32_t n_cont, const int32_
                               uint16_t* pairs_out, int32_t* colmap_out, int64_t cap, int32_t* tiling_out) {
     if (K < 1 || T < 1 || n_cont < 0 || n_cat < 0 || (n_cat > 0 && !cat_levels) || K + T > 65535) return -1;
     const GramColumns gc = gram_columns(K, T, n_cont, std::vector<int>(cat_levels, cat_levels + n_cat));
+    const int64_t len = (int64_t)gc.colmap.size();
+    for (int64_t c = 0; c < len && c < cap; ++c) {
+        if (pairs_out) { pairs_out[2 * c] = gc.pairs[2 * (size_t)c]; pairs_out[2 * c + 1] = gc.pairs[2 * (size_t)c + 1]; }
+        if (colmap_out) colmap_out[c] = gc.colmap[(size_t)c];
+    }
+    if (tiling_out) { tiling_out[0] = gc.Pc; tiling_out[1] = gc.nfull; tiling_out[2] = gc.tail_q; }
+    return len;
+}
+
+int64_t ob_debug_gram_outcome_columns(int32_t K, int32_t T, uint16_t* pairs_out, int32_t* colmap_out, int64_t cap,
+                                      int32_t* tiling_out) {
+    if (K < 1 || T < 1 || K + T > 65535) return -1;
+    const GramColumns gc = gram_outcome_columns(K, T);
     const int64_t len = (int64_t)gc.colmap.size();
     for (int64_t c = 0; c < len && c < cap; ++c) {
         if (pairs_out) { pairs_out[2 * c] = gc.pairs[2 * (size_t)c]; pairs_out[2 * c + 1] = gc.pairs[2 * (size_t)c + 1]; }

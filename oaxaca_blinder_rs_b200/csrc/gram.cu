@@ -430,6 +430,66 @@ GramColumns gram_columns(int K, int T, int n_cont, const std::vector<int>& cat_l
     return gc;
 }
 
+// The outcome columns of gram_columns alone: (j, y_t) in the full table's order, then (y_0, y_0).  Every column's sum is
+// the same as in the full launch: its DMMA sequence and leaf tree depend on (n_g, K) only, not on the tile it sits in.
+GramColumns gram_outcome_columns(int K, int T) {
+    GramColumns gc;
+    std::vector<uint16_t> pj, pl; std::vector<int32_t> cm;
+    for (int j = 0; j < K; ++j) {
+        const int64_t base = pair_base(K, T, j);
+        for (int o = 0; o < T; ++o) { pj.push_back((uint16_t)j); pl.push_back((uint16_t)(K + o)); cm.push_back((int32_t)(base + (K - j) + o)); }
+    }
+    pj.push_back((uint16_t)K); pl.push_back((uint16_t)K); cm.push_back((int32_t)(num_pairs(K, T) - 1));
+    gc.Pc = (int)cm.size();
+    gram_col_tiling(gc.Pc, gc.nfull, gc.tail_q);
+    gc.ntiles = gc.nfull + (gc.tail_q > 0);
+    const size_t cols = (size_t)gc.ntiles * BN;
+    gc.pairs.assign(cols * 2, (uint16_t)K);
+    gc.colmap.assign(cols, -1);
+    for (size_t c = 0; c < cm.size(); ++c) { gc.pairs[2 * c] = pj[c]; gc.pairs[2 * c + 1] = pl[c]; gc.colmap[c] = cm[c]; }
+    return gc;
+}
+
+std::vector<int32_t> gram_cache_map(int K, int T) {
+    std::vector<int32_t> m;
+    m.reserve((size_t)gram_cache_xx_cells(K) + gram_cache_y_cells(K, T));
+    for (int j = 0; j < K; ++j)
+        for (int l = j; l < K; ++l) m.push_back((int32_t)(pair_base(K, T, j) + (l - j)));
+    for (int j = 0; j < K; ++j)
+        for (int o = 0; o < T; ++o) m.push_back((int32_t)(pair_base(K, T, j) + (K - j) + o));
+    m.push_back((int32_t)(num_pairs(K, T) - 1));
+    return m;
+}
+
+// cell e of the copy -> (group, batch slot, cache cell c); TO_CACHE: batch Gram -> cache, else cache -> batch Gram
+template <bool TO_CACHE>
+__device__ __forceinline__ void gram_cache_copy_cells(const GramCacheCopy& a) {
+    const long long ncell = a.c_hi - a.c_lo, per_g = a.nslots * ncell, total = 2 * per_g;
+    for (long long e = (long long)blockIdx.x * blockDim.x + threadIdx.x; e < total; e += (long long)gridDim.x * blockDim.x) {
+        const int g = e >= per_g ? 1 : 0;
+        const long long r = e - (g ? per_g : 0);
+        const long long s = r / ncell;
+        const int c = a.c_lo + (int)(r - s * ncell);
+        double* gcell = a.gram + ((size_t)g * a.slots_pad + (size_t)s) * (size_t)a.Pld + a.map[c];
+        const size_t slot = (size_t)g * a.cslots + (size_t)(a.slot_lo + s);
+        double* ccell = c < a.nx ? a.xx + slot * a.nx + c : a.yy + slot * a.ny + (c - a.nx);
+        if (TO_CACHE) *ccell = *gcell; else *gcell = *ccell;
+    }
+}
+__global__ void __launch_bounds__(256) gram_cache_extract_kernel(const GramCacheCopy a) { gram_cache_copy_cells<true>(a); }
+__global__ void __launch_bounds__(256) gram_cache_assemble_kernel(const GramCacheCopy a) { gram_cache_copy_cells<false>(a); }
+
+static void gram_cache_copy(const GramCacheCopy& a, bool to_cache, cudaStream_t st) {
+    const long long total = 2 * a.nslots * (long long)(a.c_hi - a.c_lo);
+    if (total <= 0) return;
+    const unsigned blocks = (unsigned)std::min<long long>((total + 255) / 256, 148 * 8);
+    if (to_cache) gram_cache_extract_kernel<<<blocks, 256, 0, st>>>(a);
+    else gram_cache_assemble_kernel<<<blocks, 256, 0, st>>>(a);
+    OB_CUDA(cudaGetLastError());
+}
+void gram_cache_extract_launch(const GramCacheCopy& a, cudaStream_t st) { gram_cache_copy(a, true, st); }
+void gram_cache_assemble_launch(const GramCacheCopy& a, cudaStream_t st) { gram_cache_copy(a, false, st); }
+
 GramPlan gram_make_plan(int K, int T, int ldx, int panels, const GroupData gd[2], int count_bytes, int num_sms,
                         const GramColumns& cols) {
     GramPlan pl;

@@ -380,8 +380,10 @@ void check(ob_ctx* ctx, ob_status st) {
 // prepare(), but with the O(n) work on the device (ob_ingest_begin / ob_ingest_finish).  The host only
 // dictionary-encodes the string columns (what a polars Categorical / Arrow dictionary column already is) and sorts
 // the handful of values that occur.  Fills the metadata of `p` (names, levels, normalize spec, n); returns the design.
-ob_design* OaxacaBuilder::ingest_on_device(ob_ctx* ctx, Prepared& p, bool with_weights) const {
-    std::vector<std::string> cols = {outcome_, group_};
+ob_design* OaxacaBuilder::ingest_on_device(ob_ctx* ctx, Prepared& p, bool with_weights, const std::vector<std::string>* sweep) const {
+    const std::string& outcome = sweep ? sweep->front() : outcome_;
+    std::vector<std::string> cols = {outcome, group_};
+    if (sweep) cols.insert(cols.end(), sweep->begin() + 1, sweep->end());
     cols.insert(cols.end(), predictors_.begin(), predictors_.end());
     cols.insert(cols.end(), categorical_.begin(), categorical_.end());
     if (has_weights_) cols.push_back(weights_col_);
@@ -411,7 +413,7 @@ ob_design* OaxacaBuilder::ingest_on_device(ob_ctx* ctx, Prepared& p, bool with_w
     };
     std::vector<Dict> cat_dicts;
     for (const auto& cat : categorical_) { const Column* c = dataframe_.find(cat); require_str(c); cat_dicts.push_back(encode(c)); }
-    const Column* yc = dataframe_.find(outcome_);
+    const Column* yc = dataframe_.find(outcome);
     require_f64(yc);
     std::vector<ob_raw_f64> cont;
     for (const auto& pr : predictors_) { const Column* c = dataframe_.find(pr); require_f64(c); cont.push_back(raw_f64(c)); }
@@ -428,6 +430,8 @@ ob_design* OaxacaBuilder::ingest_on_device(ob_ctx* ctx, Prepared& p, bool with_w
     }
     if (has_selection_) filter_only.push_back(dataframe_.find(selection_outcome_));
     for (const auto& sp : selection_predictors_) filter_only.push_back(dataframe_.find(sp));
+    if (sweep)           // the other outcomes of the sweep: one cleaned frame for all of them
+        for (size_t k = 1; k < sweep->size(); ++k) { const Column* c = dataframe_.find((*sweep)[k]); require_f64(c); filter_only.push_back(c); }
     std::vector<uint8_t> merged_valid;
     for (const Column* c : filter_only) {
         if (c->valid.empty()) continue;
@@ -494,17 +498,24 @@ ob_design* OaxacaBuilder::ingest_on_device(ob_ctx* ctx, Prepared& p, bool with_w
     return des;
 }
 
-OaxacaResults OaxacaBuilder::run() const { return run_impl(false, 0.0); }
+OaxacaResults OaxacaBuilder::run() const { return run_impl(false, 0.0).front(); }
+
+std::vector<OaxacaResults> OaxacaBuilder::run_outcomes(const std::vector<std::string>& outcomes) const {
+    if (outcomes.empty()) throw OaxacaError(OB_ERR_INVALID_ARG, "run_outcomes needs at least one outcome column");
+    if (has_selection_) throw OaxacaError(OB_ERR_UNSUPPORTED, "run_outcomes with heckman_selection is not supported");
+    if (idx_a_ || idx_b_) throw OaxacaError(OB_ERR_UNSUPPORTED, "run_outcomes needs the native resampling stream (no index_stream)");
+    return run_impl(false, 0.0, &outcomes);
+}
 
 OaxacaResults OaxacaBuilder::decompose_quantile(double quantile) const {
     // builder.rs:711-757: RIF per group on the cleaned frame, then a fresh builder with the same predictors /
     // categoricals / reps / reference / normalize / weights (Heckman settings are NOT forwarded) -> run()
     OaxacaBuilder b = *this;
     b.has_selection_ = false; b.selection_outcome_.clear(); b.selection_predictors_.clear();
-    return b.run_impl(true, quantile);
+    return b.run_impl(true, quantile).front();
 }
 
-OaxacaResults OaxacaBuilder::run_impl(bool rif, double tau) const {
+std::vector<OaxacaResults> OaxacaBuilder::run_impl(bool rif, double tau, const std::vector<std::string>* sweep) const {
     Prepared p;
     CtxGuard g;
     ob_status st = ob_ctx_create(device_, &g.ctx);
@@ -513,7 +524,7 @@ OaxacaResults OaxacaBuilder::run_impl(bool rif, double tau) const {
     // combination rather than guess what beta* = Weighted should weigh with
     if (has_selection_ && has_weights_)
         throw OaxacaError(OB_ERR_UNSUPPORTED, "heckman_selection together with weights is not supported on the B200 path");
-    g.des = ingest_on_device(g.ctx, p, has_weights_);
+    g.des = ingest_on_device(g.ctx, p, has_weights_, sweep);
     if (rif) check(g.ctx, ob_design_apply_rif(g.ctx, g.des, tau));
     int K1 = 0;
     if (has_selection_) {
@@ -535,55 +546,65 @@ OaxacaResults OaxacaBuilder::run_impl(bool rif, double tau) const {
     const int S = has_selection_ ? ob_num_stats_heckman(K, K1) : ob_num_stats(K, n_norm, p.norm_has_base.data());
     const int D = has_selection_ ? Kc : (S - 5) / 2;
 
-    ob_boot_opts o{};
-    switch (reference_coeffs_) {
-    case ReferenceCoefficients::GroupA: o.ref_kind = OB_REF_GROUP_A; break;
-    case ReferenceCoefficients::GroupB: o.ref_kind = OB_REF_GROUP_B; break;
-    case ReferenceCoefficients::Pooled: case ReferenceCoefficients::Neumark: o.ref_kind = OB_REF_POOLED; break;
-    default: o.ref_kind = OB_REF_WEIGHTED; break;
-    }
-    o.n_norm = n_norm; o.norm_m = p.norm_m.data(); o.norm_off = p.norm_off.data();
-    o.norm_idx = p.norm_idx.data(); o.norm_has_base = p.norm_has_base.data();
-    o.reps = (int64_t)bootstrap_reps_; o.seed = seed_;
-    o.idx_a = idx_a_; o.idx_b = idx_b_;
+    struct CacheGuard { ob_gram_cache* c = nullptr; ~CacheGuard() { ob_gram_cache_destroy(c); } } cache;
+    if (sweep && sweep->size() > 1) check(g.ctx, ob_gram_cache_create(g.ctx, &cache.c));
+    std::vector<OaxacaResults> all;
+    for (size_t k = 0; k < (sweep ? sweep->size() : 1); ++k) {
+        if (k > 0) {     // the next outcome into the packed rows; X, weights and the group split stay in HBM
+            const Column* c = dataframe_.find((*sweep)[k]);
+            check(g.ctx, ob_design_update_outcome(g.ctx, g.des, c->f64.data(), (int64_t)dataframe_.height()));
+        }
+        ob_boot_opts o{};
+        switch (reference_coeffs_) {
+        case ReferenceCoefficients::GroupA: o.ref_kind = OB_REF_GROUP_A; break;
+        case ReferenceCoefficients::GroupB: o.ref_kind = OB_REF_GROUP_B; break;
+        case ReferenceCoefficients::Pooled: case ReferenceCoefficients::Neumark: o.ref_kind = OB_REF_POOLED; break;
+        default: o.ref_kind = OB_REF_WEIGHTED; break;
+        }
+        o.n_norm = n_norm; o.norm_m = p.norm_m.data(); o.norm_off = p.norm_off.data();
+        o.norm_idx = p.norm_idx.data(); o.norm_has_base = p.norm_has_base.data();
+        o.reps = (int64_t)bootstrap_reps_; o.seed = seed_;
+        o.idx_a = idx_a_; o.idx_b = idx_b_;
 
-    OaxacaResults R;
-    std::vector<double> point(S), se(S), pv(S), lo(S), hi(S), t(S);
-    R.xa_mean.resize(Kc); R.xb_mean.resize(Kc); R.beta_star.resize(Kc); R.residuals.resize((size_t)nb);
-    ob_result r{};
-    r.point_stats = point.data(); r.xa_mean = R.xa_mean.data(); r.xb_mean = R.xb_mean.data(); r.beta_star = R.beta_star.data();
-    r.residuals_b = R.residuals.data();
-    r.std_err = se.data(); r.p_value = pv.data(); r.ci_lower = lo.data(); r.ci_upper = hi.data(); r.t_stat = t.data();
-    check(g.ctx, ob_bootstrap_run(g.ctx, g.des, &o, &r));
+        OaxacaResults R;
+        std::vector<double> point(S), se(S), pv(S), lo(S), hi(S), t(S);
+        R.xa_mean.resize(Kc); R.xb_mean.resize(Kc); R.beta_star.resize(Kc); R.residuals.resize((size_t)nb);
+        ob_result r{};
+        r.point_stats = point.data(); r.xa_mean = R.xa_mean.data(); r.xb_mean = R.xb_mean.data(); r.beta_star = R.beta_star.data();
+        r.residuals_b = R.residuals.data();
+        r.std_err = se.data(); r.p_value = pv.data(); r.ci_lower = lo.data(); r.ci_upper = hi.data(); r.t_stat = t.data();
+        check(g.ctx, cache.c ? ob_bootstrap_run_cached(g.ctx, g.des, &o, cache.c, &r) : ob_bootstrap_run(g.ctx, g.des, &o, &r));
 
-    R.bootstrap_reps = (int64_t)bootstrap_reps_;
-    R.successful_bootstraps = r.n_ok;
-    if (r.n_ok < (int64_t)bootstrap_reps_)   // builder.rs:841-847
-        std::cerr << "Warning: " << (bootstrap_reps_ - r.n_ok) << " out of " << bootstrap_reps_
-                  << " bootstrap replications failed and were discarded. The analysis is based on " << r.n_ok
-                  << " successful replications." << std::endl;
-    auto comp = [&](const std::string& name, int j) {
-        return ComponentResult{name, point[j], se[j], t[j], pv[j], lo[j], hi[j]};
-    };
-    R.total_gap = r.total_gap;
-    R.two_fold.aggregate = {comp("explained", 0), comp("unexplained", 1)};                            // :867-884
-    R.three_fold.aggregate = {comp("endowments", 2), comp("coefficients", 3), comp("interaction", 4)}; // :885-910
-    std::vector<std::string> rows = p.names;
-    if (has_selection_) rows.push_back("IMR");                                                        // estimation.rs:153-154
-    else rows.insert(rows.end(), p.base_names.begin(), p.base_names.end());                           // :661-669
-    for (int j = 0; j < D; ++j) {
-        R.two_fold.detailed_explained.push_back(comp(rows[j], 5 + j));
-        R.two_fold.detailed_unexplained.push_back(comp(rows[j], 5 + D + j));
+        R.bootstrap_reps = (int64_t)bootstrap_reps_;
+        R.successful_bootstraps = r.n_ok;
+        if (r.n_ok < (int64_t)bootstrap_reps_)   // builder.rs:841-847
+            std::cerr << "Warning: " << (bootstrap_reps_ - r.n_ok) << " out of " << bootstrap_reps_
+                      << " bootstrap replications failed and were discarded. The analysis is based on " << r.n_ok
+                      << " successful replications." << std::endl;
+        auto comp = [&](const std::string& name, int j) {
+            return ComponentResult{name, point[j], se[j], t[j], pv[j], lo[j], hi[j]};
+        };
+        R.total_gap = r.total_gap;
+        R.two_fold.aggregate = {comp("explained", 0), comp("unexplained", 1)};                            // :867-884
+        R.three_fold.aggregate = {comp("endowments", 2), comp("coefficients", 3), comp("interaction", 4)}; // :885-910
+        std::vector<std::string> rows = p.names;
+        if (has_selection_) rows.push_back("IMR");                                                        // estimation.rs:153-154
+        else rows.insert(rows.end(), p.base_names.begin(), p.base_names.end());                           // :661-669
+        for (int j = 0; j < D; ++j) {
+            R.two_fold.detailed_explained.push_back(comp(rows[j], 5 + j));
+            R.two_fold.detailed_unexplained.push_back(comp(rows[j], 5 + D + j));
+        }
+        if (has_selection_) {                                                                             // builder.rs:507-534, :925-930
+            R.two_fold.detailed_selection.push_back(comp("__ob_intercept__", 5 + 2 * D));
+            for (size_t j = 0; j < selection_predictors_.size(); ++j)
+                R.two_fold.detailed_selection.push_back(comp(selection_predictors_[j], 5 + 2 * D + 1 + (int)j));
+        }
+        R.n_a = (size_t)na; R.n_b = (size_t)nb;
+        R.predictor_names = has_selection_ ? rows : p.names;
+        R.ms_total = r.ms_total; R.ms_gram = r.ms_gram;
+        all.push_back(std::move(R));
     }
-    if (has_selection_) {                                                                             // builder.rs:507-534, :925-930
-        R.two_fold.detailed_selection.push_back(comp("__ob_intercept__", 5 + 2 * D));
-        for (size_t j = 0; j < selection_predictors_.size(); ++j)
-            R.two_fold.detailed_selection.push_back(comp(selection_predictors_[j], 5 + 2 * D + 1 + (int)j));
-    }
-    R.n_a = (size_t)na; R.n_b = (size_t)nb;
-    R.predictor_names = has_selection_ ? rows : p.names;
-    R.ms_total = r.ms_total; R.ms_gram = r.ms_gram;
-    return R;
+    return all;
 }
 
 DataMatrices OaxacaBuilder::get_data_matrices() const {   // builder.rs:252-291

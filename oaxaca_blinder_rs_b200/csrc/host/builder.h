@@ -108,6 +108,9 @@ public:
     OaxacaBuilder& index_stream(const uint32_t* idx_a, const uint32_t* idx_b) { idx_a_ = idx_a; idx_b_ = idx_b; return *this; }
 
     OaxacaResults run() const;                              // builder.rs:787-951
+    // run() once per listed outcome column on one ingest: rows are cleaned over all of them, the first run fills a Gram
+    // cache and the others only contract their outcome columns (ob_bootstrap_run_cached)
+    std::vector<OaxacaResults> run_outcomes(const std::vector<std::string>& outcomes) const;
     OaxacaResults decompose_quantile(double quantile) const; // builder.rs:711-757
     DataMatrices get_data_matrices() const;                 // builder.rs:252-291
     std::string describe() const;                           // host-only JSON view of the prepared frame (tests)
@@ -116,8 +119,9 @@ private:
     struct Prepared;
     Prepared prepare() const;                                    // host-only restatement (describe(), CPU tests)
     void fill_norm_spec(Prepared& p) const;
-    ob_design* ingest_on_device(ob_ctx* ctx, Prepared& meta, bool with_weights) const;   // production path
-    OaxacaResults run_impl(bool rif, double tau) const;
+    // production path; sweep (run_outcomes): the outcome columns, sweep[0] packed in place of outcome_
+    ob_design* ingest_on_device(ob_ctx* ctx, Prepared& meta, bool with_weights, const std::vector<std::string>* sweep = nullptr) const;
+    std::vector<OaxacaResults> run_impl(bool rif, double tau, const std::vector<std::string>* sweep = nullptr) const;
 
     DataFrame dataframe_;
     std::string outcome_, group_, reference_group_;

@@ -123,6 +123,19 @@ ob_status ob_builder_run(ob_builder* b, ob_results** out) {
     *out = nullptr;
     return guarded(b, [&] { auto r = std::make_unique<ob_results>(); r->r = b->b->run(); *out = r.release(); });
 }
+ob_status ob_builder_run_outcomes(ob_builder* b, const char* const* names, int32_t n, ob_results** outs) {
+    if (!outs || n < 0 || (n > 0 && !names)) return OB_ERR_INVALID_ARG;
+    for (int32_t k = 0; k < n; ++k) outs[k] = nullptr;
+    return guarded(b, [&] {
+        std::vector<std::string> cols;
+        for (int32_t k = 0; k < n; ++k) {
+            if (!names[k]) throw ob::OaxacaError(OB_ERR_INVALID_ARG, "null outcome column name");
+            cols.emplace_back(names[k]);
+        }
+        std::vector<ob::OaxacaResults> rs = b->b->run_outcomes(cols);
+        for (int32_t k = 0; k < n; ++k) { auto r = std::make_unique<ob_results>(); r->r = std::move(rs[(size_t)k]); outs[k] = r.release(); }
+    });
+}
 ob_status ob_builder_decompose_quantile(ob_builder* b, double quantile, ob_results** out) {
     if (!out) return OB_ERR_INVALID_ARG;
     *out = nullptr;

@@ -138,6 +138,28 @@ struct GramColumns {
 // cat_levels: level counts (incl. the base level) of the design's categorical predictors, in column order, or empty
 // when unknown (ob_design_from_dense): then nothing is dropped.
 GramColumns gram_columns(int K, int T, int n_cont, const std::vector<int>& cat_levels);
+// the outcome columns of gram_columns alone (the K T cells of X'Wy and (y_0, y_0)), same order, same colmap targets:
+// the narrow contraction of a cached run whose X'WX is known (ob_bootstrap_run_cached)
+GramColumns gram_outcome_columns(int K, int T);
+
+// ---- per-replicate Gram cache (ob_gram_cache): compact layouts that do not depend on T ----
+// xx [2][slots][K(K+1)/2]: the X'WX upper triangle, row-major; yy [2][slots][K T + 1]: the X'Wy cells (j, y_t) j-major, then
+// (y_0, y_0).  gram_cache_map(K, T)[c] = position in a reduced-Gram row [Pld] of xx cell c (c < K(K+1)/2), else of yy cell
+// c - K(K+1)/2.
+inline int gram_cache_xx_cells(int K) { return K * (K + 1) / 2; }
+inline int gram_cache_y_cells(int K, int T) { return K * T + 1; }
+std::vector<int32_t> gram_cache_map(int K, int T);
+struct GramCacheCopy {
+    double* gram; int64_t slots_pad; int Pld;  // the batch's reduced Gram [2][slots_pad][Pld]
+    int64_t slot_lo, nslots;                   // its slots are the run's slots [slot_lo, slot_lo + nslots)
+    double* xx; double* yy; int64_t cslots;    // the cache, [2][cslots][nx] and [2][cslots][ny]
+    const int32_t* map; int nx, ny;            // device gram_cache_map, nx = K(K+1)/2, ny = K T + 1
+    int c_lo, c_hi;                            // cells [c_lo, c_hi) of the map are copied
+};
+// batch Gram -> cache (after gram_reduce_launch / gram_combine_launch)
+void gram_cache_extract_launch(const GramCacheCopy& a, cudaStream_t st);
+// cache -> batch Gram; after gram_reduce_launch / gram_combine_launch, which zero the whole buffer first
+void gram_cache_assemble_launch(const GramCacheCopy& a, cudaStream_t st);
 struct GramPlan {
     int K, T, ldx, panels, ntiles;
     int nfull, tail_q, Pld;       // column tiling of the computed columns and the row stride of the reduced Gram (gram_pld)
