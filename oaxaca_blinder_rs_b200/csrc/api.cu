@@ -10,10 +10,13 @@
 #include <cmath>
 #include <cstdio>
 #include <cstring>
+#include <exception>
 #include <memory>
 #include <atomic>
 #include <mutex>
+#include <optional>
 #include <set>
+#include <type_traits>
 
 using namespace ob;
 
@@ -356,6 +359,176 @@ const char* status_text(int s) {
     case OB_ERR_INSUFFICIENT_DATA: return "Insufficient data: Insufficient data for OLS calculation: n_obs must be strictly greater than k";
     default: return "error";
     }
+}
+
+// ---- the replicate-batch skeleton shared by the bootstrap drivers (bootstrap_body, heckman_run, mm_run) ----
+
+// The replicate range of a call, from the fields ob_boot_opts and ob_mm_opts share: global replicate ids [rb, re), whether
+// the library shards the work over the context's communicator (mode R), and the multiplicity width to start with.
+// OLS and Heckman then narrow [rb, re) to the rank's share; Machado-Mata shards its regressions instead.
+struct RepRange {
+    bool shard_reps; int64_t rb, re, nrep;
+    bool index_mode; int count_bytes;
+};
+
+template <typename Opts>
+RepRange replicate_range(const ob_ctx* ctx, const Opts* o) {
+    if (o->reps < 0) fail(OB_ERR_INVALID_ARG, "negative reps");
+    RepRange r;
+    r.shard_reps = o->shard_replicates != 0 && ctx->comm && ctx->comm->world > 1;
+    if (r.shard_reps && (o->rep_begin != 0 || o->rep_end != 0 || o->skip_reduce))
+        fail(OB_ERR_INVALID_ARG, "shard_replicates computes the shard itself: rep_begin / rep_end / skip_reduce must be 0");
+    r.rb = o->rep_begin; r.re = o->rep_end > 0 ? o->rep_end : o->reps;
+    if (r.rb < 0 || r.re < r.rb || r.re > o->reps) fail(OB_ERR_INVALID_ARG, "bad replicate shard");
+    r.nrep = r.re - r.rb;
+    r.index_mode = o->idx_a != nullptr || o->idx_b != nullptr;
+    if (r.index_mode && r.nrep > 0 && (!o->idx_a || !o->idx_b)) fail(OB_ERR_INVALID_ARG, "index stream needs both idx_a and idx_b");
+    if (o->count_bits != 0 && o->count_bits != 8 && o->count_bits != 16) fail(OB_ERR_INVALID_ARG, "count_bits must be 0, 8 or 16");
+    r.count_bytes = o->count_bits == 16 ? 2 : 1;
+    return r;
+}
+
+// One batch of the panel loop: panels [p0, p0 + pn) of the multiplicity matrix hold slots [slot_lo, slot_hi) of the call's
+// 1 + nrep (slot 0 of the first batch is the point estimate)
+struct Batch {
+    int64_t pn, slot_lo, slot_hi, bslots;
+    int first_slot;
+    int64_t brep;                 // replicates in this batch
+    int64_t rep0;                 // global replicate id of the batch's slot 0
+    Batch(int64_t p0, int64_t ppb, int64_t panels_total, int64_t slots, int64_t rb)
+        : pn(std::min(ppb, panels_total - p0)), slot_lo(p0 * BM), slot_hi(std::min(slots, (p0 + pn) * BM)),
+          bslots(slot_hi - slot_lo), first_slot(p0 == 0 ? 1 : 0), brep(bslots - first_slot), rep0(rb + slot_lo - 1) {}
+    // GramArgs::tail_mi: valid slots of the batch's last panel -> 8-slot groups, rounded up to a multiple of 4
+    int tail_mi() const {
+        const int64_t last = bslots - (pn - 1) * BM;
+        return (int)std::min<int64_t>(16, ((last + 7) / 8 + 3) / 4 * 4);
+    }
+};
+
+// The batch's multiplicity columns of both groups (resample.cu), from the caller's index stream or the native Philox
+// stream.  The native fix-up tops every replicate up to exactly n_global draws, so it needs the column sums over all row
+// shards: row_comm is the mode-N communicator (null otherwise; ms_comm then goes unused).  On a design that is not row
+// sharded, shard.n_global == n and shard.row_begin == 0: alloc_group sets row_shard(n, 0, 1), and ob_design_set_row_shard
+// with world 1 accepts only n_global == n.  colsum holds 2 x ppb * BM sums.  Returns the number of kernels launched.
+template <typename Opts>
+int generate_counts(const ob_design* d, const Opts* o, const Batch& b, int count_bytes, int64_t ppb, DevBuf (&C)[2],
+                    DevBuf (&idx)[2], DevBuf& colsum, DevBuf& lut, int* flags, Comm* row_comm, double* ms_comm, cudaStream_t st) {
+    CountsArgs ca[2];
+    for (int g = 0; g < 2; ++g) {
+        const GroupData& G = d->g[g];
+        ca[g].C = C[g].p; ca[g].count_bytes = count_bytes; ca[g].n = G.n; ca[g].n_pad = G.n_pad;
+        ca[g].n_global = G.shard.n_global; ca[g].row_begin = G.shard.row_begin;
+        ca[g].panels = (int)b.pn; ca[g].slots = b.bslots; ca[g].first_slot = b.first_slot; ca[g].rep0 = b.rep0;
+        ca[g].group = g; ca[g].seed = o->seed;
+    }
+    int launches = 0;
+    if (o->idx_a || o->idx_b) {
+        for (int g = 0; g < 2; ++g) {
+            const uint32_t* h = g == 0 ? o->idx_a : o->idx_b;
+            const int64_t n_glob = ca[g].n_global;
+            const size_t nb = sizeof(uint32_t) * (size_t)std::max<int64_t>(b.brep, 1) * n_glob;
+            if (idx[g].bytes < nb) idx[g].alloc(nb);
+            if (b.brep > 0)
+                OB_CUDA(cudaMemcpyAsync(idx[g].p, h + (size_t)(b.rep0 + b.first_slot) * n_glob,
+                                        sizeof(uint32_t) * (size_t)b.brep * n_glob, cudaMemcpyHostToDevice, st));
+            counts_from_indices(ca[g], idx[g].as<uint32_t>(), flags, st);
+            launches += 1 + (b.brep > 0 ? (int)((b.brep + 32767) / 32768) : 0);
+        }
+        return launches;
+    }
+    long long* sums[2] = {colsum.as<long long>(), colsum.as<long long>() + (size_t)ppb * BM};
+    OB_CUDA(cudaMemsetAsync(colsum.p, 0, colsum.bytes, st));
+    for (int g = 0; g < 2; ++g) {
+        counts_philox_body_launch(ca[g], sums[g], lut.as<unsigned char>() + (size_t)g * counts_lut_bytes(), st);
+        launches += 2;
+    }
+    if (row_comm) {
+        Timer t_c(st, ms_comm);
+        row_comm->allreduce(colsum.p, 2 * (size_t)ppb * BM, CommDType::I64, CommOp::SUM, st);
+        t_c.stop(); OB_CUDA(cudaStreamSynchronize(st)); t_c.collect();
+    }
+    for (int g = 0; g < 2; ++g) {
+        counts_philox_fixup_launch(ca[g], sums[g], flags, st);
+        launches += b.brep > 0 ? 1 : 0;
+    }
+    return launches;
+}
+
+// A batch's deferred error flags (multiplicity kernels): a bad index or a Poisson overshoot fails the call.  A saturated
+// count returns true when the run may widen to 16-bit counts and redo, and fails when it may not.
+bool check_batch_flags(const int flags[4], int count_bytes, int count_bits) {
+    if (flags[2]) fail(OB_ERR_INVALID_ARG, "resample index out of range");
+    if (flags[0]) fail(OB_ERR_CUDA, "Poisson body overshot n (probability < 1e-15 per replicate); rerun with another seed");
+    if (flags[1] && (count_bytes == 2 || count_bits == 8)) fail(OB_ERR_UNSUPPORTED, "row multiplicity overflows the count width");
+    return flags[1] != 0;
+}
+
+// A host value through an all-reduce over comm (int: I32, long long: I64); every rank returns the same result.
+template <typename T>
+T allreduce_scalar(Comm* comm, T v, CommOp op, cudaStream_t st) {
+    static_assert(std::is_same<T, int>::value || std::is_same<T, long long>::value, "I32 or I64");
+    DevBuf d(sizeof v);
+    OB_CUDA(cudaMemcpyAsync(d.p, &v, sizeof v, cudaMemcpyHostToDevice, st));
+    comm->allreduce(d.p, 1, std::is_same<T, int>::value ? CommDType::I32 : CommDType::I64, op, st);
+    OB_CUDA(cudaMemcpyAsync(&v, d.p, sizeof v, cudaMemcpyDeviceToHost, st));
+    OB_CUDA(cudaStreamSynchronize(st));
+    return v;
+}
+
+// Runs body.  With a communicator all ranks leave together: a rank that failed (a bad index in its share, device memory it
+// could not get) must not leave its peers waiting in their next collective.  The ranks agree on the highest status; a
+// rank that failed raises its own error, the others peer_msg with the agreed status.
+template <typename F>
+void agree_on_status(Comm* comm, cudaStream_t st, F&& body, const char* peer_msg) {
+    if (!comm) { body(); return; }
+    int rc = OB_OK;
+    std::exception_ptr own;
+    try { body(); }
+    catch (const StatusError& e) { rc = e.code; own = std::current_exception(); }
+    catch (const CudaError& e) {
+        cudaGetLastError();
+        if (e.code != cudaErrorMemoryAllocation) throw;
+        rc = OB_ERR_CUDA; own = std::current_exception();
+    }
+    const int agreed = allreduce_scalar(comm, rc, CommOp::MAX, st);
+    if (own) std::rethrow_exception(own);
+    if (agreed != OB_OK) fail((ob_status)agreed, std::string(peer_msg) + ": " + status_text(agreed));
+}
+
+// All-gather of per-rank rows in shard order: rank r contributes rows [b, e) of ob_replicate_shard(total, world, r) from
+// `mine`, `unit` elements each; every rank receives all `total` rows in `all` (grown as needed), which is returned.
+template <typename T>
+T* allgather_shards(Comm* comm, int64_t total, size_t unit, const T* mine, DevBuf& all, cudaStream_t st) {
+    const size_t row = sizeof(T) * unit, need = row * (size_t)std::max<int64_t>(total, 1);
+    if (all.bytes < need) all.alloc(need);
+    std::vector<size_t> off(comm->world), sz(comm->world);
+    for (int r = 0; r < comm->world; ++r) {
+        int64_t b = 0, e = 0;
+        ob_replicate_shard(total, comm->world, r, &b, &e);
+        off[r] = (size_t)b * row; sz[r] = (size_t)(e - b) * row;
+    }
+    comm->allgatherv(mine, all.p, off.data(), sz.data(), st);
+    return all.as<T>();
+}
+
+// (5) The replicate rows reduced to standard errors, p-values, percentile CIs and t statistics (reduce_stats.cu), each
+// [S] result downloaded to dst[k] unless that is null.  ms (may be null) accumulates the reduction's device time.
+void reduce_to_host(cudaStream_t st, const double* stats_rows, const int* status_rows, int64_t reps, int S,
+                    const double* point, double* const dst[5], int64_t* n_ok, double* ms) {
+    DevBuf d_out(sizeof(double) * 5 * (size_t)S), d_nok(sizeof(long long)), d_rs(reduce_stats_scratch_bytes(reps, S));
+    std::optional<Timer> t_red;
+    if (ms) t_red.emplace(st, ms);
+    reduce_stats_launch(stats_rows, status_rows, reps, S, point, d_out.as<double>(), d_nok.as<long long>(), st, d_rs.as<double>());
+    if (t_red) t_red->stop();
+    std::vector<double> out5(5 * (size_t)S);
+    long long nok = 0;
+    OB_CUDA(cudaMemcpyAsync(out5.data(), d_out.p, d_out.bytes, cudaMemcpyDeviceToHost, st));
+    OB_CUDA(cudaMemcpyAsync(&nok, d_nok.p, sizeof nok, cudaMemcpyDeviceToHost, st));
+    OB_CUDA(cudaStreamSynchronize(st));
+    if (t_red) t_red->collect();
+    if (n_ok) *n_ok = nok;
+    for (int k = 0; k < 5; ++k)
+        if (dst[k]) memcpy(dst[k], out5.data() + (size_t)k * S, sizeof(double) * S);
 }
 
 }  // namespace
@@ -1372,26 +1545,18 @@ void heckman_run(ob_ctx* ctx, const ob_design* d, const ob_boot_opts* o, ob_resu
         fail(OB_ERR_UNSUPPORTED, "Pooled / Neumark reference coefficients with Heckman selection: the reference's pooled regression has K "
                                  "coefficients, the Heckman fits K + 1 (builder.rs:548-589 vs estimation.rs:139-141)");
     if (d->T != 1) fail(OB_ERR_UNSUPPORTED, "Heckman selection on a multi-outcome design");
-    if (o->reps < 0) fail(OB_ERR_INVALID_ARG, "negative reps");
+    if (d->world > 1) fail(OB_ERR_UNSUPPORTED, "Heckman selection on a row-sharded design");
+    RepRange rr = replicate_range(ctx, o);
     // mode R inside the library, as for the OLS path: this rank's contiguous share of the global replicate ids
-    const bool shard_reps = o->shard_replicates != 0 && ctx->comm && ctx->comm->world > 1;
-    if (shard_reps && (o->rep_begin != 0 || o->rep_end != 0 || o->skip_reduce))
-        fail(OB_ERR_INVALID_ARG, "shard_replicates computes the shard itself: rep_begin / rep_end / skip_reduce must be 0");
-    int64_t rb = o->rep_begin, re = o->rep_end > 0 ? o->rep_end : o->reps;
-    if (shard_reps) ob_replicate_shard(o->reps, ctx->comm->world, ctx->comm->rank, &rb, &re);
-    if (rb < 0 || re < rb || re > o->reps) fail(OB_ERR_INVALID_ARG, "bad replicate shard");
-    const int64_t nrep = re - rb;
+    if (rr.shard_reps) { ob_replicate_shard(o->reps, ctx->comm->world, ctx->comm->rank, &rr.rb, &rr.re); rr.nrep = rr.re - rr.rb; }
     if (d->g[0].n == 0 || d->g[1].n == 0) fail(OB_ERR_INVALID_GROUP, "Invalid group variable: One group has no data");
-    const bool index_mode = o->idx_a != nullptr || o->idx_b != nullptr;
-    if (index_mode && nrep > 0 && (!o->idx_a || !o->idx_b)) fail(OB_ERR_INVALID_ARG, "index stream needs both idx_a and idx_b");
-    if (o->count_bits != 0 && o->count_bits != 8 && o->count_bits != 16) fail(OB_ERR_INVALID_ARG, "count_bits must be 0, 8 or 16");
-    int count_bytes = o->count_bits == 16 ? 2 : 1;
+    int count_bytes = rr.count_bytes;
     const int S = ob_num_stats_heckman(K, K1);
 
     res->ms_counts = res->ms_gram = res->ms_solve = res->ms_reduce = res->ms_total = res->ms_gram_kernel = res->ms_comm = 0.0;
     res->gpu_launches = 0; res->n_ok = 0;
     Timer t_total(st, &res->ms_total);
-    const int64_t slots = 1 + nrep, panels_total = (slots + BM - 1) / BM;
+    const int64_t slots = 1 + rr.nrep, panels_total = (slots + BM - 1) / BM;
     const bool want_beta = res->rep_beta_a || res->rep_beta_b || res->beta_a || res->beta_b;
     DevBuf d_stats(sizeof(double) * (size_t)slots * S), d_status(sizeof(int) * (size_t)slots);
     DevBuf d_ba(want_beta ? sizeof(double) * (size_t)slots * Ka : 0), d_bb(want_beta ? sizeof(double) * (size_t)slots * Ka : 0);
@@ -1410,7 +1575,7 @@ void heckman_run(ob_ctx* ctx, const ob_design* d, const ob_boot_opts* o, ob_resu
         OB_CUDA(cudaMemGetInfo(&free_b, &total_b));
         const double budget = o->max_workspace_bytes > 0 ? (double)o->max_workspace_bytes : 0.6 * ((double)free_b + (double)pool_idle_bytes(ctx));
         const double per_panel = (double)(n_pad[0] + n_pad[1]) * BM * (count_bytes + 8.0) +        // counts + L = c * IMR
-                                 (index_mode ? (double)(n_g[0] + n_g[1]) * BM * 4.0 : 0.0) + 2.0 * BM * Pld * 8.0 +
+                                 (rr.index_mode ? (double)(n_g[0] + n_g[1]) * BM * 4.0 : 0.0) + 2.0 * BM * Pld * 8.0 +
                                  (double)leaves * ntiles * (BM * BN * 8.0) +
                                  (double)(nch[0] + nch[1]) * BM * 8.0 * std::max(std::max(nacc_p, nacc_t), K);
         int64_t ppb = std::max<int64_t>(1, std::min<int64_t>((int64_t)std::floor(budget / per_panel), panels_total));
@@ -1436,36 +1601,12 @@ void heckman_run(ob_ctx* ctx, const ob_design* d, const ob_boot_opts* o, ob_resu
         GramPlan plan; int64_t plan_panels = -1;
         bool saturated = false;
         for (int64_t p0 = 0; p0 < panels_total && !saturated; p0 += ppb) {
-            const int64_t pn = std::min(ppb, panels_total - p0);
-            const int64_t slot_lo = p0 * BM, slot_hi = std::min(slots, (p0 + pn) * BM), bslots = slot_hi - slot_lo;
-            const int first_slot = p0 == 0 ? 1 : 0;
-            const int64_t brep = bslots - first_slot, rep0 = rb + slot_lo - 1, slots_pad = pn * BM;
+            const Batch b(p0, ppb, panels_total, slots, rr.rb);
+            const int64_t pn = b.pn, bslots = b.bslots, slots_pad = pn * BM;
             OB_CUDA(cudaMemsetAsync(d_flags.p, 0, sizeof(int) * 4, st));
             // (2) replicate generation: the same multiplicity matrix as the OLS path
             Timer t_counts(st, &res->ms_counts);
-            CountsArgs ca[2];
-            for (int g = 0; g < 2; ++g) {
-                ca[g].C = d_C[g].p; ca[g].count_bytes = count_bytes; ca[g].n = n_g[g]; ca[g].n_pad = n_pad[g];
-                ca[g].n_global = n_g[g]; ca[g].row_begin = 0; ca[g].panels = (int)pn; ca[g].slots = bslots;
-                ca[g].first_slot = first_slot; ca[g].rep0 = rep0; ca[g].group = g; ca[g].seed = o->seed;
-            }
-            if (index_mode) {
-                for (int g = 0; g < 2; ++g) {
-                    const uint32_t* h = g == 0 ? o->idx_a : o->idx_b;
-                    const size_t nb = sizeof(uint32_t) * (size_t)std::max<int64_t>(brep, 1) * n_g[g];
-                    if (d_idx[g].bytes < nb) d_idx[g].alloc(nb);
-                    if (brep > 0) OB_CUDA(cudaMemcpyAsync(d_idx[g].p, h + (size_t)(rep0 + first_slot) * n_g[g], sizeof(uint32_t) * (size_t)brep * n_g[g], cudaMemcpyHostToDevice, st));
-                    counts_from_indices(ca[g], d_idx[g].as<uint32_t>(), d_flags.as<int>(), st);
-                    res->gpu_launches += 2;
-                }
-            } else {
-                OB_CUDA(cudaMemsetAsync(d_colsum.p, 0, d_colsum.bytes, st));
-                for (int g = 0; g < 2; ++g) {
-                    counts_philox_body_launch(ca[g], d_colsum.as<long long>() + (size_t)g * ppb * BM, d_lut.as<unsigned char>() + (size_t)g * counts_lut_bytes(), st);
-                    counts_philox_fixup_launch(ca[g], d_colsum.as<long long>() + (size_t)g * ppb * BM, d_flags.as<int>(), st);
-                    res->gpu_launches += 3;
-                }
-            }
+            res->gpu_launches += generate_counts(d, o, b, count_bytes, ppb, d_C, d_idx, d_colsum, d_lut, d_flags.as<int>(), nullptr, nullptr, st);
             t_counts.stop();
 
             // (3a) probit of every slot, both groups: Fisher scoring until every slot has converged (<= 100 steps)
@@ -1507,7 +1648,7 @@ void heckman_run(ob_ctx* ctx, const ob_design* d, const ob_boot_opts* o, ob_resu
             GramArgs ga;
             for (int g = 0; g < 2; ++g) { ga.X[g] = d->g[g].hk_Xm; ga.C[g] = d_C[g].p; }
             ga.count_bytes = count_bytes; ga.partials = d_partials.as<double>(); ga.d_pairs = d_pairs.as<uint16_t>(); ga.d_colmap = d_colmap.as<int32_t>(); ga.gram = d_gram.as<double>();
-            { const int64_t last = bslots - (pn - 1) * BM; ga.tail_mi = (int)std::min<int64_t>(16, ((last + 7) / 8 + 3) / 4 * 4); }
+            ga.tail_mi = b.tail_mi();
             gram_launch(plan, ga, st);
             res->gpu_launches += 2;
             t_gram.stop();
@@ -1518,9 +1659,9 @@ void heckman_run(ob_ctx* ctx, const ob_design* d, const ob_boot_opts* o, ob_resu
             sa.gram = d_gram.as<double>(); sa.slots_pad = slots_pad; sa.Pld = Pld; sa.slots = bslots; sa.K = K; sa.K1 = K1; sa.ref_kind = o->ref_kind;
             for (int g = 0; g < 2; ++g) { sa.terms[g] = d_terms[g].as<double>(); sa.xterm[g] = d_xterm[g].as<double>(); sa.gamma[g] = d_gamma[g].as<double>(); sa.pstatus[g] = d_pst[g].as<int>(); }
             sa.na = (double)n_g[0]; sa.nb = (double)n_g[1]; sa.S = S;
-            sa.stats = d_stats.as<double>() + (size_t)slot_lo * S; sa.status = d_status.as<int>() + slot_lo;
-            sa.beta_a = want_beta ? d_ba.as<double>() + (size_t)slot_lo * Ka : nullptr;
-            sa.beta_b = want_beta ? d_bb.as<double>() + (size_t)slot_lo * Ka : nullptr;
+            sa.stats = d_stats.as<double>() + (size_t)b.slot_lo * S; sa.status = d_status.as<int>() + b.slot_lo;
+            sa.beta_a = want_beta ? d_ba.as<double>() + (size_t)b.slot_lo * Ka : nullptr;
+            sa.beta_b = want_beta ? d_bb.as<double>() + (size_t)b.slot_lo * Ka : nullptr;
             sa.point_extra = p0 == 0 ? d_point.as<double>() : nullptr;
             hk_solve_launch(sa, st);
             res->gpu_launches += 1;
@@ -1529,12 +1670,7 @@ void heckman_run(ob_ctx* ctx, const ob_design* d, const ob_boot_opts* o, ob_resu
             OB_CUDA(cudaMemcpyAsync(flags, d_flags.p, sizeof flags, cudaMemcpyDeviceToHost, st));
             OB_CUDA(cudaStreamSynchronize(st));
             t_counts.collect(); t_solve.collect(); t_gram.collect(); t_solve2.collect();
-            if (flags[2]) fail(OB_ERR_INVALID_ARG, "resample index out of range");
-            if (flags[0]) fail(OB_ERR_CUDA, "Poisson body overshot n (probability < 1e-15 per replicate); rerun with another seed");
-            if (flags[1]) {
-                if (count_bytes == 2 || o->count_bits == 8) fail(OB_ERR_UNSUPPORTED, "row multiplicity overflows the count width");
-                saturated = true;
-            }
+            saturated = check_batch_flags(flags, count_bytes, o->count_bits);
         }
         if (!saturated) break;
         count_bytes = 2;
@@ -1547,20 +1683,7 @@ void heckman_run(ob_ctx* ctx, const ob_design* d, const ob_boot_opts* o, ob_resu
     if (point_status != OB_OK)
         fail((ob_status)point_status, point_status == OB_ERR_INVALID_GROUP ? "Invalid group variable: No observed outcomes in group" : status_text(point_status));
     };   // run_batches
-    if (shard_reps) {      // all ranks leave together (see ob_bootstrap_run)
-        int rc = OB_OK; std::string msg;
-        try { run_batches(); } catch (const StatusError& e) { rc = e.code; msg = e.msg; }
-        DevBuf d_rc(sizeof(int));
-        int agreed = rc;
-        OB_CUDA(cudaMemcpyAsync(d_rc.p, &agreed, sizeof(int), cudaMemcpyHostToDevice, st));
-        ctx->comm->allreduce(d_rc.p, 1, CommDType::I32, CommOp::MAX, st);
-        OB_CUDA(cudaMemcpyAsync(&agreed, d_rc.p, sizeof(int), cudaMemcpyDeviceToHost, st));
-        OB_CUDA(cudaStreamSynchronize(st));
-        if (rc != OB_OK) fail((ob_status)rc, msg);
-        if (agreed != OB_OK) fail((ob_status)agreed, std::string("another rank of the replicate-sharded run failed: ") + status_text(agreed));
-    } else {
-        run_batches();
-    }
+    agree_on_status(rr.shard_reps ? ctx->comm.get() : nullptr, st, run_batches, "another rank of the replicate-sharded run failed");
     res->total_gap = point[3 * Ka + 2 * K1];
     if (res->xa_mean) memcpy(res->xa_mean, point.data(), sizeof(double) * Ka);
     if (res->xb_mean) memcpy(res->xb_mean, point.data() + Ka, sizeof(double) * Ka);
@@ -1572,50 +1695,25 @@ void heckman_run(ob_ctx* ctx, const ob_design* d, const ob_boot_opts* o, ob_resu
     if (res->point_stats) OB_CUDA(cudaMemcpyAsync(res->point_stats, d_stats.p, sizeof(double) * S, cudaMemcpyDeviceToHost, st));
     if (res->beta_a) OB_CUDA(cudaMemcpyAsync(res->beta_a, d_ba.p, sizeof(double) * Ka, cudaMemcpyDeviceToHost, st));
     if (res->beta_b) OB_CUDA(cudaMemcpyAsync(res->beta_b, d_bb.p, sizeof(double) * Ka, cudaMemcpyDeviceToHost, st));
-    const int64_t reps_all = shard_reps ? o->reps : nrep;
+    const int64_t reps_all = rr.shard_reps ? o->reps : rr.nrep;
     DevBuf d_gstats, d_gstatus, d_gba, d_gbb;
     const double* stats_rows = d_stats.as<double>() + S;
     const int* status_rows = d_status.as<int>() + 1;
     const double* ba_rows = want_beta ? d_ba.as<double>() + Ka : nullptr;
     const double* bb_rows = want_beta ? d_bb.as<double>() + Ka : nullptr;
-    if (shard_reps) {      // replicate rows of all ranks, device to device, into global replicate order
+    if (rr.shard_reps) {      // replicate rows of all ranks, device to device, into global replicate order
         Timer t_c(st, &res->ms_comm);
         Comm* cm = ctx->comm.get();
-        const int w = cm->world;
-        std::vector<size_t> off(w), sz(w);
-        auto gather_rows = [&](const void* mine, DevBuf& all, size_t row_bytes) {
-            all.alloc(row_bytes * (size_t)std::max<int64_t>(reps_all, 1));
-            for (int r = 0; r < w; ++r) {
-                int64_t b = 0, e = 0;
-                ob_replicate_shard(o->reps, w, r, &b, &e);
-                off[r] = (size_t)b * row_bytes; sz[r] = (size_t)(e - b) * row_bytes;
-            }
-            cm->allgatherv(mine, all.p, off.data(), sz.data(), st);
-        };
-        gather_rows(stats_rows, d_gstats, sizeof(double) * (size_t)S);
-        gather_rows(status_rows, d_gstatus, sizeof(int));
-        stats_rows = d_gstats.as<double>(); status_rows = d_gstatus.as<int>();
-        if (res->rep_beta_a) { gather_rows(ba_rows, d_gba, sizeof(double) * (size_t)Ka); ba_rows = d_gba.as<double>(); }
-        if (res->rep_beta_b) { gather_rows(bb_rows, d_gbb, sizeof(double) * (size_t)Ka); bb_rows = d_gbb.as<double>(); }
+        stats_rows = allgather_shards(cm, o->reps, S, stats_rows, d_gstats, st);
+        status_rows = allgather_shards(cm, o->reps, 1, status_rows, d_gstatus, st);
+        if (res->rep_beta_a) ba_rows = allgather_shards(cm, o->reps, Ka, ba_rows, d_gba, st);
+        if (res->rep_beta_b) bb_rows = allgather_shards(cm, o->reps, Ka, bb_rows, d_gbb, st);
         t_c.stop(); OB_CUDA(cudaStreamSynchronize(st)); t_c.collect();
     }
     if (!o->skip_reduce) {
-        DevBuf d_out(sizeof(double) * 5 * (size_t)S), d_nok(sizeof(long long)), d_rs(reduce_stats_scratch_bytes(reps_all, S));
-        Timer t_red(st, &res->ms_reduce);
-        reduce_stats_launch(stats_rows, status_rows, reps_all, S, d_stats.as<double>(), d_out.as<double>(),
-                            d_nok.as<long long>(), st, d_rs.as<double>());
-        res->gpu_launches += 1;
-        t_red.stop();
-        std::vector<double> out5(5 * (size_t)S);
-        long long nok = 0;
-        OB_CUDA(cudaMemcpyAsync(out5.data(), d_out.p, d_out.bytes, cudaMemcpyDeviceToHost, st));
-        OB_CUDA(cudaMemcpyAsync(&nok, d_nok.p, sizeof nok, cudaMemcpyDeviceToHost, st));
-        OB_CUDA(cudaStreamSynchronize(st));
-        t_red.collect();
-        res->n_ok = nok;
         double* dst[5] = {res->std_err, res->p_value, res->ci_lower, res->ci_upper, res->t_stat};
-        for (int k = 0; k < 5; ++k)
-            if (dst[k]) memcpy(dst[k], out5.data() + (size_t)k * S, sizeof(double) * S);
+        reduce_to_host(st, stats_rows, status_rows, reps_all, S, d_stats.as<double>(), dst, &res->n_ok, &res->ms_reduce);
+        res->gpu_launches += 1;
     }
     if (reps_all > 0) {
         if (res->rep_stats) OB_CUDA(cudaMemcpyAsync(res->rep_stats, stats_rows, sizeof(double) * (size_t)reps_all * S, cudaMemcpyDeviceToHost, st));
@@ -1635,39 +1733,30 @@ void mm_run(ob_ctx* ctx, const ob_design* d, const ob_mm_opts* o, ob_mm_result* 
     const int K = d->K, sims = o->simulations, nq = o->n_quantiles, S = 3 * nq;
     if (sims < 1 || sims > MM_MAX_SIMS) fail(OB_ERR_INVALID_ARG, "simulations must be in [1, 4096]");
     if (nq < 1 || nq > 1024 || !o->quantiles) fail(OB_ERR_INVALID_ARG, "n_quantiles must be in [1, 1024]");
-    if (o->reps < 0) fail(OB_ERR_INVALID_ARG, "negative reps");
     if (K > MM_MAX_COLS) fail(OB_ERR_UNSUPPORTED, "Machado-Mata: more than 47 design columns");
     if (d->weighted) fail(OB_ERR_UNSUPPORTED, "Machado-Mata on a weighted design (QuantileDecompositionBuilder has no weights)");
     if (d->T != 1 || d->g[0].y_raw || d->g[1].y_raw) fail(OB_ERR_UNSUPPORTED, "Machado-Mata needs the raw outcome (the design carries RIF outcomes)");
     if (d->world > 1) fail(OB_ERR_UNSUPPORTED, "Machado-Mata on a row-sharded design");
     if (d->g[0].n < 2 || d->g[1].n < 2) fail(OB_ERR_INVALID_GROUP, "Invalid group variable: One group has insufficient data");   // :210-214
-    const bool shard_reps = o->shard_replicates != 0 && ctx->comm && ctx->comm->world > 1;
-    if (shard_reps && (o->rep_begin != 0 || o->rep_end != 0 || o->skip_reduce))
-        fail(OB_ERR_INVALID_ARG, "shard_replicates computes the shard itself: rep_begin / rep_end / skip_reduce must be 0");
     // Mode R inside the library shards the REGRESSIONS, not the passes: every rank builds the multiplicity columns and the
     // streams of all passes (cheap), solves a contiguous balanced share of each batch's (pass, simulation, group) problems,
     // the coefficients are all-gathered device to device, and effects + reduction run on every rank.  With the builder's
     // default of 20 passes a pass-level split over 8 GPUs would leave ranks with 4 or 3 passes (the point pass included)
     // against 2.6 on average; the problem-level split is even to one regression.
-    int64_t rb = o->rep_begin, re = o->rep_end > 0 ? o->rep_end : o->reps;
-    if (rb < 0 || re < rb || re > o->reps) fail(OB_ERR_INVALID_ARG, "bad replicate shard");
-    const int64_t nrep = re - rb;
-    const bool index_mode = o->idx_a != nullptr || o->idx_b != nullptr;
-    if (index_mode && nrep > 0 && (!o->idx_a || !o->idx_b)) fail(OB_ERR_INVALID_ARG, "index stream needs both idx_a and idx_b");
+    const RepRange rr = replicate_range(ctx, o);
     const bool draws_given = o->draw_a != nullptr || o->draw_b != nullptr;
     if (draws_given && (!o->draw_a || !o->draw_b)) fail(OB_ERR_INVALID_ARG, "simulated-row stream needs both draw_a and draw_b");
-    if (draws_given && nrep > 0 && !index_mode)
+    if (draws_given && rr.nrep > 0 && !rr.index_mode)
         fail(OB_ERR_INVALID_ARG, "draw_a / draw_b are positions in the resampled frames: they need the explicit resample stream idx_a / idx_b");
-    if (o->count_bits != 0 && o->count_bits != 8 && o->count_bits != 16) fail(OB_ERR_INVALID_ARG, "count_bits must be 0, 8 or 16");
     for (int q = 0; q < nq; ++q)
         if (!(o->quantiles[q] >= 0.0 && o->quantiles[q] <= 1.0)) fail(OB_ERR_INVALID_ARG, "target quantiles must lie in [0, 1]");
-    int count_bytes = o->count_bits == 16 ? 2 : 1;
+    int count_bytes = rr.count_bytes;
 
     res->ms_counts = res->ms_qr = res->ms_effects = res->ms_reduce = res->ms_total = 0.0;
     res->gpu_launches = 0; res->n_ok = 0;
     res->qr_total = res->qr_vertex = res->qr_approx = res->qr_failed = res->qr_iterations = 0;
     Timer t_total(st, &res->ms_total);
-    const int64_t slots = 1 + nrep, panels_total = (slots + BM - 1) / BM;
+    const int64_t slots = 1 + rr.nrep, panels_total = (slots + BM - 1) / BM;
     const int64_t n_pad[2] = {d->g[0].n_pad, d->g[1].n_pad}, n_g[2] = {d->g[0].n, d->g[1].n};
     DevBuf d_stats(sizeof(double) * (size_t)slots * S), d_status(sizeof(int) * (size_t)slots);
     DevBuf d_q(sizeof(double) * (size_t)nq), d_flags(sizeof(int) * 4), d_lut(2 * counts_lut_bytes()), d_counter(sizeof(int));
@@ -1687,7 +1776,7 @@ void mm_run(ob_ctx* ctx, const ob_design* d, const ob_mm_opts* o, ob_mm_result* 
         const double slab = 8.0 * mm_state_vectors() * (double)stride;
         int grid = ctx->num_sms * mm_blocks_per_sm(K, std::max(n_g[0], n_g[1]));
         grid = (int)std::max<int64_t>(1, std::min<int64_t>(grid, (int64_t)std::floor(0.5 * budget / slab)));
-        const double per_panel = (double)(n_pad[0] + n_pad[1]) * BM * count_bytes + (index_mode ? (double)(n_g[0] + n_g[1]) * BM * 4.0 : 0.0) +
+        const double per_panel = (double)(n_pad[0] + n_pad[1]) * BM * count_bytes + (rr.index_mode ? (double)(n_g[0] + n_g[1]) * BM * 4.0 : 0.0) +
                                  (double)BM * sims * (2.0 * K * 8.0 + 2.0 * 4.0 + 8.0 + 8.0);
         int64_t ppb = std::max<int64_t>(1, std::min<int64_t>((int64_t)std::floor((budget - grid * slab) / per_panel), panels_total));
         DevBuf d_C[2], d_idx[2], d_colsum(sizeof(long long) * 2 * (size_t)ppb * BM);
@@ -1695,40 +1784,16 @@ void mm_run(ob_ctx* ctx, const ob_design* d, const ob_mm_opts* o, ob_mm_result* 
         const size_t bs_max = (size_t)std::min<int64_t>(ppb * BM, slots);
         DevBuf d_state(sizeof(double) * (size_t)mm_state_vectors() * (size_t)stride * (size_t)grid);
         DevBuf d_betas(sizeof(double) * 2 * bs_max * sims * K), d_info(sizeof(int) * 2 * bs_max * sims);
-        DevBuf d_betas_all(shard_reps ? d_betas.bytes : 0), d_info_all(shard_reps ? d_info.bytes : 0);
+        DevBuf d_betas_all, d_info_all;      // mode R: every rank's share of them (allgather_shards)
         DevBuf d_taus(sizeof(double) * bs_max * sims), d_rows_a(sizeof(uint32_t) * bs_max * sims), d_rows_b(sizeof(uint32_t) * bs_max * sims);
         bool saturated = false;
         for (int64_t p0 = 0; p0 < panels_total && !saturated; p0 += ppb) {
-            const int64_t pn = std::min(ppb, panels_total - p0);
-            const int64_t slot_lo = p0 * BM, slot_hi = std::min(slots, (p0 + pn) * BM), bslots = slot_hi - slot_lo;
-            const int first_slot = p0 == 0 ? 1 : 0;
-            const int64_t brep = bslots - first_slot, rep0 = rb + slot_lo - 1;
+            const Batch b(p0, ppb, panels_total, slots, rr.rb);
+            const int64_t bslots = b.bslots;
             OB_CUDA(cudaMemsetAsync(d_flags.p, 0, sizeof(int) * 4, st));
             // (1) the passes' multiplicity columns: the same replicate generation as ob_bootstrap_run
             Timer t_counts(st, &res->ms_counts);
-            CountsArgs ca[2];
-            for (int g = 0; g < 2; ++g) {
-                ca[g].C = d_C[g].p; ca[g].count_bytes = count_bytes; ca[g].n = n_g[g]; ca[g].n_pad = n_pad[g];
-                ca[g].n_global = n_g[g]; ca[g].row_begin = 0; ca[g].panels = (int)pn; ca[g].slots = bslots;
-                ca[g].first_slot = first_slot; ca[g].rep0 = rep0; ca[g].group = g; ca[g].seed = o->seed;
-            }
-            if (index_mode) {
-                for (int g = 0; g < 2; ++g) {
-                    const uint32_t* h = g == 0 ? o->idx_a : o->idx_b;
-                    const size_t nb = sizeof(uint32_t) * (size_t)std::max<int64_t>(brep, 1) * n_g[g];
-                    if (d_idx[g].bytes < nb) d_idx[g].alloc(nb);
-                    if (brep > 0) OB_CUDA(cudaMemcpyAsync(d_idx[g].p, h + (size_t)(rep0 + first_slot) * n_g[g], sizeof(uint32_t) * (size_t)brep * n_g[g], cudaMemcpyHostToDevice, st));
-                    counts_from_indices(ca[g], d_idx[g].as<uint32_t>(), d_flags.as<int>(), st);
-                    res->gpu_launches += 2;
-                }
-            } else {
-                OB_CUDA(cudaMemsetAsync(d_colsum.p, 0, d_colsum.bytes, st));
-                for (int g = 0; g < 2; ++g) {
-                    counts_philox_body_launch(ca[g], d_colsum.as<long long>() + (size_t)g * ppb * BM, d_lut.as<unsigned char>() + (size_t)g * counts_lut_bytes(), st);
-                    counts_philox_fixup_launch(ca[g], d_colsum.as<long long>() + (size_t)g * ppb * BM, d_flags.as<int>(), st);
-                    res->gpu_launches += 3;
-                }
-            }
+            res->gpu_launches += generate_counts(d, o, b, count_bytes, ppb, d_C, d_idx, d_colsum, d_lut, d_flags.as<int>(), nullptr, nullptr, st);
             t_counts.stop();
             // (2) random quantiles and simulated rows of the batch's passes
             MmArgs ma;
@@ -1738,15 +1803,15 @@ void mm_run(ob_ctx* ctx, const ob_design* d, const ob_mm_opts* o, ob_mm_result* 
             ma.betas = d_betas.as<double>(); ma.info = d_info.as<int>(); ma.counter = d_counter.as<int>();
             // global pass ids: 0 = point estimates (slot 0 of the first batch), r + 1 = replicate r.  With a replicate shard
             // the batch's slots 1.. are replicates rb.., so consecutive only from slot 1 on: the point slot is special-cased
-            const int64_t gpass0 = rep0 + 1;          // pass id slot 0 of this batch WOULD have as a replicate slot
+            const int64_t gpass0 = b.rep0 + 1;        // pass id slot 0 of this batch WOULD have as a replicate slot
             if (!o->taus || !draws_given) {
-                mm_streams_launch(ma, gpass0, first_slot, o->seed, d_taus.as<double>(), d_rows_a.as<uint32_t>(), d_rows_b.as<uint32_t>(), st);
+                mm_streams_launch(ma, gpass0, b.first_slot, o->seed, d_taus.as<double>(), d_rows_a.as<uint32_t>(), d_rows_b.as<uint32_t>(), st);
                 res->gpu_launches += 1;
             }
             if (o->taus) {      // explicit quantiles: rows of the [(reps + 1) x sims] table, row 0 = point pass, row r + 1 = replicate r
                 h_taus.resize((size_t)bslots * sims);
                 for (int64_t s_ = 0; s_ < bslots; ++s_) {
-                    const int64_t pass = (p0 == 0 && s_ == 0) ? 0 : rep0 + s_ + 1;
+                    const int64_t pass = (p0 == 0 && s_ == 0) ? 0 : b.rep0 + s_ + 1;
                     memcpy(h_taus.data() + (size_t)s_ * sims, o->taus + (size_t)pass * sims, sizeof(double) * (size_t)sims);
                 }
                 OB_CUDA(cudaMemcpyAsync(d_taus.p, h_taus.data(), sizeof(double) * h_taus.size(), cudaMemcpyHostToDevice, st));
@@ -1757,11 +1822,12 @@ void mm_run(ob_ctx* ctx, const ob_design* d, const ob_mm_opts* o, ob_mm_result* 
                     const uint32_t* ix = g == 0 ? o->idx_a : o->idx_b;
                     h_rows[g].resize((size_t)bslots * sims);
                     for (int64_t s_ = 0; s_ < bslots; ++s_) {
-                        const int64_t pass = (p0 == 0 && s_ == 0) ? 0 : rep0 + s_ + 1;
+                        const int64_t pass = (p0 == 0 && s_ == 0) ? 0 : b.rep0 + s_ + 1;
                         for (int i = 0; i < sims; ++i) {
                             const uint32_t pos = dr[(size_t)pass * sims + i];
                             if ((int64_t)pos >= n_g[g]) fail(OB_ERR_INVALID_ARG, "simulated-row position out of range");
                             h_rows[g][(size_t)s_ * sims + i] = pass == 0 ? pos : ix[(size_t)(pass - 1) * n_g[g] + pos];
+                            if ((int64_t)h_rows[g][(size_t)s_ * sims + i] >= n_g[g]) fail(OB_ERR_INVALID_ARG, "resample index out of range");
                         }
                     }
                     OB_CUDA(cudaMemcpyAsync((g == 0 ? d_rows_a : d_rows_b).p, h_rows[g].data(), sizeof(uint32_t) * h_rows[g].size(), cudaMemcpyHostToDevice, st));
@@ -1772,32 +1838,21 @@ void mm_run(ob_ctx* ctx, const ob_design* d, const ob_mm_opts* o, ob_mm_result* 
             OB_CUDA(cudaMemsetAsync(d_counter.p, 0, sizeof(int), st));
             const int64_t nprob = 2 * bslots * sims;
             ma.p_begin = 0; ma.p_end = nprob;
-            if (shard_reps) ob_replicate_shard(nprob, ctx->comm->world, ctx->comm->rank, &ma.p_begin, &ma.p_end);
+            if (rr.shard_reps) ob_replicate_shard(nprob, ctx->comm->world, ctx->comm->rank, &ma.p_begin, &ma.p_end);
             if (ma.p_end > ma.p_begin) {
                 mm_qr_launch(ma, (int)std::min<int64_t>(grid, ma.p_end - ma.p_begin), st);
                 res->gpu_launches += 1;
             }
             t_qr.stop();
-            if (shard_reps) {      // every rank's coefficients and status words, device to device, in problem order
+            if (rr.shard_reps) {      // every rank's coefficients and status words, device to device, in problem order
                 Comm* cm = ctx->comm.get();
-                const int w = cm->world;
-                std::vector<size_t> off(w), sz(w);
-                auto gather = [&](const DevBuf& mine, DevBuf& all, size_t unit) {
-                    for (int r = 0; r < w; ++r) {
-                        int64_t b = 0, e = 0;
-                        ob_replicate_shard(nprob, w, r, &b, &e);
-                        off[r] = (size_t)b * unit; sz[r] = (size_t)(e - b) * unit;
-                    }
-                    cm->allgatherv(static_cast<const char*>(mine.p) + off[cm->rank], all.p, off.data(), sz.data(), st);
-                };
-                gather(d_betas, d_betas_all, sizeof(double) * (size_t)K);
-                gather(d_info, d_info_all, sizeof(int));
-                ma.betas = d_betas_all.as<double>(); ma.info = d_info_all.as<int>();
+                ma.betas = allgather_shards(cm, nprob, (size_t)K, d_betas.as<double>() + (size_t)ma.p_begin * K, d_betas_all, st);
+                ma.info = allgather_shards(cm, nprob, 1, d_info.as<int>() + ma.p_begin, d_info_all, st);
             }
             // (4) simulation, empirical quantiles, effects
             Timer t_eff(st, &res->ms_effects);
-            mm_effects_launch(ma, d_rows_a.as<uint32_t>(), d_rows_b.as<uint32_t>(), nq, d_q.as<double>(), d_stats.as<double>() + (size_t)slot_lo * S,
-                              d_status.as<int>() + slot_lo, nullptr, st);
+            mm_effects_launch(ma, d_rows_a.as<uint32_t>(), d_rows_b.as<uint32_t>(), nq, d_q.as<double>(), d_stats.as<double>() + (size_t)b.slot_lo * S,
+                              d_status.as<int>() + b.slot_lo, nullptr, st);
             res->gpu_launches += 1;
             t_eff.stop();
             int flags[4];
@@ -1810,13 +1865,8 @@ void mm_run(ob_ctx* ctx, const ob_design* d, const ob_mm_opts* o, ob_mm_result* 
             }
             OB_CUDA(cudaStreamSynchronize(st));
             t_counts.collect(); t_qr.collect(); t_eff.collect();
-            if (flags[2]) fail(OB_ERR_INVALID_ARG, "resample index out of range");
-            if (flags[0]) fail(OB_ERR_CUDA, "Poisson body overshot n (probability < 1e-15 per replicate); rerun with another seed");
-            if (flags[1]) {
-                if (count_bytes == 2 || o->count_bits == 8) fail(OB_ERR_UNSUPPORTED, "row multiplicity overflows the count width");
-                saturated = true;
-                break;
-            }
+            saturated = check_batch_flags(flags, count_bytes, o->count_bits);
+            if (saturated) break;
             if (p0 == 0 && (res->point_betas_a || res->point_betas_b))
                 for (int s_ = 0; s_ < sims; ++s_) {
                     if (res->point_betas_a) memcpy(res->point_betas_a + (size_t)s_ * K, h_pbetas.data() + ((size_t)2 * s_ + 0) * K, sizeof(double) * (size_t)K);
@@ -1845,41 +1895,15 @@ void mm_run(ob_ctx* ctx, const ob_design* d, const ob_mm_opts* o, ob_mm_result* 
     if (point_status != OB_OK)
         fail(OB_ERR_NALGEBRA, "Nalgebra error: Failed to estimate a sufficient number of quantile regressions.");      // :238-242
     };   // run_batches
-    if (shard_reps) {      // all ranks leave together (see ob_bootstrap_run)
-        int rc = OB_OK; std::string msg;
-        try { run_batches(); } catch (const StatusError& e) { rc = e.code; msg = e.msg; }
-        DevBuf d_rc(sizeof(int));
-        int agreed = rc;
-        OB_CUDA(cudaMemcpyAsync(d_rc.p, &agreed, sizeof(int), cudaMemcpyHostToDevice, st));
-        ctx->comm->allreduce(d_rc.p, 1, CommDType::I32, CommOp::MAX, st);
-        OB_CUDA(cudaMemcpyAsync(&agreed, d_rc.p, sizeof(int), cudaMemcpyDeviceToHost, st));
-        OB_CUDA(cudaStreamSynchronize(st));
-        if (rc != OB_OK) fail((ob_status)rc, msg);
-        if (agreed != OB_OK) fail((ob_status)agreed, std::string("another rank of the replicate-sharded run failed: ") + status_text(agreed));
-    } else {
-        run_batches();
-    }
+    agree_on_status(rr.shard_reps ? ctx->comm.get() : nullptr, st, run_batches, "another rank of the replicate-sharded run failed");
     if (res->point_stats) OB_CUDA(cudaMemcpyAsync(res->point_stats, d_stats.p, sizeof(double) * S, cudaMemcpyDeviceToHost, st));
-    const int64_t reps_all = nrep;         // (mode R: every rank has computed the effects of all passes)
+    const int64_t reps_all = rr.nrep;      // (mode R: every rank has computed the effects of all passes)
     const double* stats_rows = d_stats.as<double>() + S;
     const int* status_rows = d_status.as<int>() + 1;
     if (!o->skip_reduce) {
-        DevBuf d_out(sizeof(double) * 5 * (size_t)S), d_nok(sizeof(long long)), d_rs(reduce_stats_scratch_bytes(reps_all, S));
-        Timer t_red(st, &res->ms_reduce);
-        reduce_stats_launch(stats_rows, status_rows, reps_all, S, d_stats.as<double>(), d_out.as<double>(),
-                            d_nok.as<long long>(), st, d_rs.as<double>());
-        res->gpu_launches += 1;
-        t_red.stop();
-        std::vector<double> out5(5 * (size_t)S);
-        long long nok = 0;
-        OB_CUDA(cudaMemcpyAsync(out5.data(), d_out.p, d_out.bytes, cudaMemcpyDeviceToHost, st));
-        OB_CUDA(cudaMemcpyAsync(&nok, d_nok.p, sizeof nok, cudaMemcpyDeviceToHost, st));
-        OB_CUDA(cudaStreamSynchronize(st));
-        t_red.collect();
-        res->n_ok = nok;
         double* dst[5] = {res->std_err, res->p_value, res->ci_lower, res->ci_upper, res->t_stat};
-        for (int k = 0; k < 5; ++k)
-            if (dst[k]) memcpy(dst[k], out5.data() + (size_t)k * S, sizeof(double) * S);
+        reduce_to_host(st, stats_rows, status_rows, reps_all, S, d_stats.as<double>(), dst, &res->n_ok, &res->ms_reduce);
+        res->gpu_launches += 1;
     }
     if (reps_all > 0) {
         if (res->rep_stats) OB_CUDA(cudaMemcpyAsync(res->rep_stats, stats_rows, sizeof(double) * (size_t)reps_all * S, cudaMemcpyDeviceToHost, st));
@@ -1917,16 +1941,11 @@ static void bootstrap_body(ob_ctx* ctx, const ob_design* d, const ob_boot_opts* 
         cudaStream_t st = ctx->stream;
         const int K = d->K, T = d->T;
         if (o->ref_kind < 0 || o->ref_kind > 3) fail(OB_ERR_INVALID_ARG, "ref_kind out of range");
-        if (o->reps < 0 || o->n_norm < 0) fail(OB_ERR_INVALID_ARG, "negative reps / n_norm");
-        // mode R inside the library: this rank's contiguous share of the global replicate ids
-        const bool shard_reps = o->shard_replicates != 0 && ctx->comm && ctx->comm->world > 1;
+        if (o->n_norm < 0) fail(OB_ERR_INVALID_ARG, "negative n_norm");
+        RepRange rr = replicate_range(ctx, o);
         if (o->shard_replicates && d->world > 1) fail(OB_ERR_INVALID_ARG, "shard_replicates on a row-sharded design (its communicator shards rows)");
-        if (shard_reps && (o->rep_begin != 0 || o->rep_end != 0 || o->skip_reduce))
-            fail(OB_ERR_INVALID_ARG, "shard_replicates computes the shard itself: rep_begin / rep_end / skip_reduce must be 0");
-        int64_t rb = o->rep_begin, re = o->rep_end > 0 ? o->rep_end : o->reps;
-        if (shard_reps) ob_replicate_shard(o->reps, ctx->comm->world, ctx->comm->rank, &rb, &re);
-        if (rb < 0 || re < rb || re > o->reps) fail(OB_ERR_INVALID_ARG, "bad replicate shard");
-        const int64_t nrep = re - rb;
+        // mode R inside the library: this rank's contiguous share of the global replicate ids
+        if (rr.shard_reps) { ob_replicate_shard(o->reps, ctx->comm->world, ctx->comm->rank, &rr.rb, &rr.re); rr.nrep = rr.re - rr.rb; }
         // builder.rs:431-435 (either group empty)
         if (d->g[0].shard.n_global == 0 || d->g[1].shard.n_global == 0) fail(OB_ERR_INVALID_GROUP, "Invalid group variable: One group has no data");
         // mode N: this design is one row shard; the context must carry the matching communicator
@@ -1937,23 +1956,17 @@ static void bootstrap_body(ob_ctx* ctx, const ob_design* d, const ob_boot_opts* 
         int n_base = 0, n_idx = 0;
         // ---- Gram cache: what of this run the cache already holds ----
         int mode = OB_CACHE_NONE;
-        const int rep_world = shard_reps ? ctx->comm->world : 1, rep_rank = shard_reps ? ctx->comm->rank : 0;
+        const int rep_world = rr.shard_reps ? ctx->comm->world : 1, rep_rank = rr.shard_reps ? ctx->comm->rank : 0;
         if (cache) {
             const bool xx_hit = cache->xx_ok && cache->design_id == d->id && cache->x_gen == d->x_gen && cache->seed == o->seed &&
-                                cache->reps == o->reps && cache->rep_begin == rb && cache->rep_end == re &&
-                                cache->shard_reps == (shard_reps ? 1 : 0) && cache->rep_world == rep_world && cache->rep_rank == rep_rank &&
+                                cache->reps == o->reps && cache->rep_begin == rr.rb && cache->rep_end == rr.re &&
+                                cache->shard_reps == (rr.shard_reps ? 1 : 0) && cache->rep_world == rep_world && cache->rep_rank == rep_rank &&
                                 cache->row_world == d->world && cache->row_rank == d->rank && cache->K == d->K &&
                                 !(o->count_bits == 8 && cache->count_bytes == 2);   // that run saturates 8-bit counts: let it fail
             mode = !xx_hit ? OB_CACHE_FILLED : (cache->y_ok && cache->y_gen == d->y_gen && cache->T == d->T) ? OB_CACHE_SOLVE_ONLY
                                                                                                            : OB_CACHE_OUTCOME_ONLY;
             // sharded runs: every rank must run the same collectives -- all take the least reuse any rank can do
-            if (Comm* ac = shard_reps ? ctx->comm.get() : comm) {
-                DevBuf d_mode(sizeof(int));
-                OB_CUDA(cudaMemcpyAsync(d_mode.p, &mode, sizeof(int), cudaMemcpyHostToDevice, ctx->stream));
-                ac->allreduce(d_mode.p, 1, CommDType::I32, CommOp::MIN, ctx->stream);
-                OB_CUDA(cudaMemcpyAsync(&mode, d_mode.p, sizeof(int), cudaMemcpyDeviceToHost, ctx->stream));
-                OB_CUDA(cudaStreamSynchronize(ctx->stream));
-            }
+            if (Comm* ac = rr.shard_reps ? ctx->comm.get() : comm) mode = allreduce_scalar(ac, mode, CommOp::MIN, st);
         }
         const bool solve_only = mode == OB_CACHE_SOLVE_ONLY, outcome_only = mode == OB_CACHE_OUTCOME_ONLY;
         for (int v = 0; v < o->n_norm; ++v) {
@@ -1965,10 +1978,7 @@ static void bootstrap_body(ob_ctx* ctx, const ob_design* d, const ob_boot_opts* 
             if (o->norm_idx[t] < 0 || o->norm_idx[t] >= K) fail(OB_ERR_INVALID_ARG, "norm_idx outside the design");
         const int D = K + n_base, S = 5 + 2 * D;
         const int SE = T * S, KE = T * K;     // per slot: T outcomes (a quantile sweep) x S statistics / K coefficients
-        const bool index_mode = o->idx_a != nullptr || o->idx_b != nullptr;
-        if (index_mode && nrep > 0 && (!o->idx_a || !o->idx_b)) fail(OB_ERR_INVALID_ARG, "index stream needs both idx_a and idx_b");
-        if (o->count_bits != 0 && o->count_bits != 8 && o->count_bits != 16) fail(OB_ERR_INVALID_ARG, "count_bits must be 0, 8 or 16");
-        int count_bytes = o->count_bits == 16 ? 2 : 1;
+        int count_bytes = rr.count_bytes;
         if (outcome_only && o->count_bits == 0) count_bytes = cache->count_bytes;   // start where the fill ended
 
         res->ms_counts = res->ms_gram = res->ms_solve = res->ms_reduce = res->ms_total = res->ms_gram_kernel = res->ms_comm = 0.0;
@@ -1988,7 +1998,7 @@ static void bootstrap_body(ob_ctx* ctx, const ob_design* d, const ob_boot_opts* 
         }
 
         // ---- outputs over all slots of this shard (slot 0 = point estimate) ----
-        const int64_t slots = 1 + nrep;
+        const int64_t slots = 1 + rr.nrep;
         const bool want_beta = res->rep_beta_a || res->rep_beta_b || res->beta_a || res->beta_b;
         DevBuf d_stats(sizeof(double) * (size_t)slots * SE), d_status(sizeof(int) * (size_t)slots);
         DevBuf d_ba(want_beta ? sizeof(double) * (size_t)slots * KE : 0), d_bb(want_beta ? sizeof(double) * (size_t)slots * KE : 0);
@@ -2033,7 +2043,7 @@ static void bootstrap_body(ob_ctx* ctx, const ob_design* d, const ob_boot_opts* 
         // sums; a run that only solves needs the reduced Gram alone
         auto per_panel_bytes = [&](int cb) {
             if (solve_only) return 2.0 * BM * Pld * 8.0;
-            return (double)(n_pad[0] + n_pad[1]) * BM * cb + (index_mode ? (double)(n_glob[0] + n_glob[1]) * BM * 4.0 : 0.0) +
+            return (double)(n_pad[0] + n_pad[1]) * BM * cb + (rr.index_mode ? (double)(n_glob[0] + n_glob[1]) * BM * 4.0 : 0.0) +
                    2.0 * BM * Pld * 8.0 * (comm ? world + 2 : 1) + (double)local_leaves * ntiles * (BM * BN * 8.0) + 2.0 * BM * 8.0;
         };
         double budget = (double)o->max_workspace_bytes - (double)cache_new_bytes;
@@ -2050,7 +2060,7 @@ static void bootstrap_body(ob_ctx* ctx, const ob_design* d, const ob_boot_opts* 
                 budget = 0.6 * ((double)free_b + idle) - (double)cache_new_bytes;
             }
         }
-        DevBuf d_agree(sizeof(long long)), d_lut(2 * counts_lut_bytes());
+        DevBuf d_lut(2 * counts_lut_bytes());
 
         std::vector<double> point(PE * T);
         cudaEvent_t ev_point = nullptr;          // recorded on st once the point estimate's coefficients are on the device
@@ -2061,14 +2071,8 @@ static void bootstrap_body(ob_ctx* ctx, const ob_design* d, const ob_boot_opts* 
             const double per_panel = per_panel_bytes(count_bytes);
             int64_t ppb = (int64_t)std::floor(budget / per_panel);
             ppb = std::max<int64_t>(1, std::min<int64_t>(ppb, panels_total));
-            if (comm) {   // every rank must cut the same batches: the collectives run once per batch
-                long long v = ppb;
-                OB_CUDA(cudaMemcpyAsync(d_agree.p, &v, sizeof v, cudaMemcpyHostToDevice, st));
-                comm->allreduce(d_agree.p, 1, CommDType::I64, CommOp::MIN, st);
-                OB_CUDA(cudaMemcpyAsync(&v, d_agree.p, sizeof v, cudaMemcpyDeviceToHost, st));
-                OB_CUDA(cudaStreamSynchronize(st));
-                ppb = v;
-            }
+            // every rank must cut the same batches: the collectives run once per batch
+            if (comm) ppb = allreduce_scalar(comm, (long long)ppb, CommOp::MIN, st);
             tr.mark("setup", st, true);
             DevBuf d_C[2], d_idx[2], d_colsum, d_gram, d_gram_local, d_gathered;
             const size_t gram_elems = 2 * (size_t)ppb * BM * Pld;      // [2][slots_pad][Pld]
@@ -2097,77 +2101,21 @@ static void bootstrap_body(ob_ctx* ctx, const ob_design* d, const ob_boot_opts* 
                 OB_CUDA(cudaMemcpyAsync(d_colmap.p, gcols.colmap.data(), sizeof(int32_t) * gcols.colmap.size(), cudaMemcpyHostToDevice, st));
                 OB_CUDA(cudaStreamSynchronize(st));
             };
-            if (!comm) allocate_workspace();
-            else {
-                // row shards: a rank whose workspace cannot be had (its GPU is shared, say) must not leave its peers waiting
-                // in the first collective of the batch loop -- all ranks agree on the outcome of the allocation phase
-                int rc = OB_OK; std::string msg;
-                try { allocate_workspace(); }
-                catch (const StatusError& e) { rc = e.code; msg = e.msg; }
-                catch (const CudaError& e) {
-                    cudaGetLastError();
-                    if (e.code != cudaErrorMemoryAllocation) throw;
-                    rc = OB_ERR_CUDA; msg = "workspace allocation failed on this rank (out of device memory)";
-                }
-                int agreed = rc;
-                OB_CUDA(cudaMemcpyAsync(d_agree.p, &agreed, sizeof(int), cudaMemcpyHostToDevice, st));
-                comm->allreduce(d_agree.p, 1, CommDType::I32, CommOp::MAX, st);
-                OB_CUDA(cudaMemcpyAsync(&agreed, d_agree.p, sizeof(int), cudaMemcpyDeviceToHost, st));
-                OB_CUDA(cudaStreamSynchronize(st));
-                if (rc != OB_OK) fail((ob_status)rc, msg);
-                if (agreed != OB_OK) fail((ob_status)agreed, "another rank of the row-sharded run could not allocate its workspace");
-            }
+            // row shards: a rank whose workspace cannot be had (its GPU is shared, say) must not leave its peers waiting in the
+            // first collective of the batch loop -- all ranks agree on the outcome of the allocation phase
+            agree_on_status(comm, st, allocate_workspace, "another rank of the row-sharded run could not allocate its workspace");
 
             tr.mark("workspace + pair table", st, true);
             for (int64_t p0 = 0; p0 < panels_total && !saturated; p0 += ppb) {
-                const int64_t pn = std::min(ppb, panels_total - p0);
-                const int64_t slot_lo = p0 * BM, slot_hi = std::min(slots, (p0 + pn) * BM);
-                const int64_t bslots = slot_hi - slot_lo;
-                const int first_slot = (p0 == 0) ? 1 : 0;
-                const int64_t brep = bslots - first_slot;                 // replicates in this batch
-                const int64_t rep0 = rb + slot_lo - 1;                    // global replicate id of local slot 0
+                const Batch b(p0, ppb, panels_total, slots, rr.rb);
+                const int64_t pn = b.pn, bslots = b.bslots;
                 OB_CUDA(cudaMemsetAsync(d_flags.p, 0, sizeof(int) * 4, st));
 
-                // (2) replicate generation
+                // (2) replicate generation (none when the cache holds every Gram cell of these slots)
                 Timer t_counts(st, &res->ms_counts);
-                CountsArgs ca[2];
-                for (int g = 0; g < 2; ++g) {
-                    ca[g].C = d_C[g].p; ca[g].count_bytes = count_bytes; ca[g].n = d->g[g].n; ca[g].n_pad = n_pad[g];
-                    ca[g].n_global = n_glob[g]; ca[g].row_begin = d->g[g].shard.row_begin;
-                    ca[g].panels = (int)pn; ca[g].slots = bslots; ca[g].first_slot = first_slot; ca[g].rep0 = rep0;
-                    ca[g].group = g; ca[g].seed = o->seed;
-                }
-                if (solve_only) {
-                    // the cache holds every Gram cell of these slots: no multiplicities
-                } else if (index_mode) {
-                    for (int g = 0; g < 2; ++g) {
-                        const uint32_t* h = (g == 0 ? o->idx_a : o->idx_b);
-                        const size_t nb = sizeof(uint32_t) * (size_t)std::max<int64_t>(brep, 1) * n_glob[g];
-                        if (d_idx[g].bytes < nb) d_idx[g].alloc(nb);
-                        if (brep > 0)
-                            OB_CUDA(cudaMemcpyAsync(d_idx[g].p, h + (size_t)(rep0 + first_slot) * n_glob[g],
-                                                    sizeof(uint32_t) * (size_t)brep * n_glob[g], cudaMemcpyHostToDevice, st));
-                        counts_from_indices(ca[g], d_idx[g].as<uint32_t>(), d_flags.as<int>(), st);
-                        res->gpu_launches += 1 + (brep > 0 ? (int)((brep + 32767) / 32768) : 0);
-                    }
-                } else {
-                    OB_CUDA(cudaMemsetAsync(d_colsum.p, 0, d_colsum.bytes, st));
-                    for (int g = 0; g < 2; ++g) {
-                        counts_philox_body_launch(ca[g], d_colsum.as<long long>() + (size_t)g * ppb * BM,
-                                                  d_lut.as<unsigned char>() + (size_t)g * counts_lut_bytes(), st);
-                        res->gpu_launches += 2;
-                    }
-                    // the fix-up tops every replicate up to exactly n_g draws: it needs the column sums over ALL row shards
-                    if (comm) {
-                        Timer t_c(st, &res->ms_comm);
-                        comm->allreduce(d_colsum.p, 2 * (size_t)ppb * BM, CommDType::I64, CommOp::SUM, st);
-                        t_c.stop(); OB_CUDA(cudaStreamSynchronize(st)); t_c.collect();
-                    }
-                    for (int g = 0; g < 2; ++g) {
-                        counts_philox_fixup_launch(ca[g], d_colsum.as<long long>() + (size_t)g * ppb * BM, d_flags.as<int>(), st);
-                        res->gpu_launches += brep > 0 ? 1 : 0;
-                    }
-                }
+                if (!solve_only)
+                    res->gpu_launches += generate_counts(d, o, b, count_bytes, ppb, d_C, d_idx, d_colsum, d_lut, d_flags.as<int>(), comm,
+                                                         &res->ms_comm, st);
                 t_counts.stop();
                 tr.mark("counts", st, true);
 
@@ -2183,10 +2131,7 @@ static void bootstrap_body(ob_ctx* ctx, const ob_design* d, const ob_boot_opts* 
                 ga.count_bytes = count_bytes; ga.partials = d_partials.as<double>();
                 ga.d_pairs = d_pairs.as<uint16_t>(); ga.d_colmap = d_colmap.as<int32_t>();
                 ga.gram = comm ? d_gram_local.as<double>() : d_gram.as<double>();
-                {   // valid slots of this batch's last panel -> 8-slot groups, rounded up to a multiple of 4
-                    const int64_t last = bslots - (pn - 1) * BM;
-                    ga.tail_mi = (int)std::min<int64_t>(16, ((last + 7) / 8 + 3) / 4 * 4);
-                }
+                ga.tail_mi = b.tail_mi();
                 struct EventPair {   // RAII: an error thrown further down must not leak the events
                     cudaEvent_t a = nullptr, b = nullptr;
                     EventPair() { OB_CUDA(cudaEventCreate(&a)); OB_CUDA(cudaEventCreate(&b)); }
@@ -2260,7 +2205,7 @@ static void bootstrap_body(ob_ctx* ctx, const ob_design* d, const ob_boot_opts* 
                     // the reduced Gram of these slots is complete (the reduce / combine zeroed it first): fill the cells the
                     // contraction skipped from the cache, keep the ones it computed
                     Timer t_cc(st, &res->ms_gram);
-                    GramCacheCopy cc{d_gram.as<double>(), pn * BM, Pld, slot_lo, bslots, cache->xx, cache->yy, slots,
+                    GramCacheCopy cc{d_gram.as<double>(), pn * BM, Pld, b.slot_lo, bslots, cache->xx, cache->yy, slots,
                                      d_cmap.as<int32_t>(), nx, ny, 0, nx + ny};
                     if (mode == OB_CACHE_FILLED) gram_cache_extract_launch(cc, st);
                     else if (solve_only) gram_cache_assemble_launch(cc, st);
@@ -2282,10 +2227,10 @@ static void bootstrap_body(ob_ctx* ctx, const ob_design* d, const ob_boot_opts* 
                 sa.d_norm_idx = d_nidx.as<int>(); sa.d_norm_has_base = d_nhb.as<int>();
                 sa.n_base = n_base; sa.S = S; sa.weighted = d->weighted ? 1 : 0;
                 sa.na = (double)n_glob[0]; sa.nb = (double)n_glob[1];
-                sa.stats = d_stats.as<double>() + (size_t)slot_lo * SE;
-                sa.status = d_status.as<int>() + slot_lo;
-                sa.beta_a = want_beta ? d_ba.as<double>() + (size_t)slot_lo * KE : nullptr;
-                sa.beta_b = want_beta ? d_bb.as<double>() + (size_t)slot_lo * KE : nullptr;
+                sa.stats = d_stats.as<double>() + (size_t)b.slot_lo * SE;
+                sa.status = d_status.as<int>() + b.slot_lo;
+                sa.beta_a = want_beta ? d_ba.as<double>() + (size_t)b.slot_lo * KE : nullptr;
+                sa.beta_b = want_beta ? d_bb.as<double>() + (size_t)b.slot_lo * KE : nullptr;
                 sa.point_extra = (p0 == 0) ? d_point.as<double>() : nullptr;
                 DevBuf d_solve_scratch(solve_scratch_bytes(K, o->ref_kind == OB_REF_POOLED, o->n_norm, T, bslots));   // wide designs only
                 sa.scratch = d_solve_scratch.as<double>();
@@ -2300,12 +2245,7 @@ static void bootstrap_body(ob_ctx* ctx, const ob_design* d, const ob_boot_opts* 
                 tr.mark("solve + flags", st, false);
                 t_counts.collect(); t_gram.collect(); t_solve.collect();
                 { float ms = 0; cudaEventElapsedTime(&ms, ev.a, ev.b); res->ms_gram_kernel += ms; }
-                if (flags[2]) fail(OB_ERR_INVALID_ARG, "resample index out of range");
-                if (flags[0]) fail(OB_ERR_CUDA, "Poisson body overshot n (probability < 1e-15 per replicate); rerun with another seed");
-                if (flags[1]) {
-                    if (count_bytes == 2 || o->count_bits == 8) fail(OB_ERR_UNSUPPORTED, "row multiplicity overflows the count width");
-                    saturated = true;
-                }
+                saturated = check_batch_flags(flags, count_bytes, o->count_bits);
             }
             if (!saturated) break;
             count_bytes = 2;  // widen and redo
@@ -2321,27 +2261,13 @@ static void bootstrap_body(ob_ctx* ctx, const ob_design* d, const ob_boot_opts* 
         if (point_status != OB_OK) fail((ob_status)point_status, status_text(point_status));
         };   // run_batches
 
-        if (shard_reps) {
-            // all ranks leave together: a rank that failed (rank-local workspace shortage, bad index, ...) must not leave
-            // its peers waiting inside the gather
-            int rc = OB_OK; std::string msg;
-            try { run_batches(); } catch (const StatusError& e) { rc = e.code; msg = e.msg; }
-            DevBuf d_rc(sizeof(int));
-            int agreed = rc;
-            OB_CUDA(cudaMemcpyAsync(d_rc.p, &agreed, sizeof(int), cudaMemcpyHostToDevice, st));
-            ctx->comm->allreduce(d_rc.p, 1, CommDType::I32, CommOp::MAX, st);
-            OB_CUDA(cudaMemcpyAsync(&agreed, d_rc.p, sizeof(int), cudaMemcpyDeviceToHost, st));
-            OB_CUDA(cudaStreamSynchronize(st));
-            if (rc != OB_OK) fail((ob_status)rc, msg);
-            if (agreed != OB_OK) fail((ob_status)agreed, std::string("another rank of the replicate-sharded run failed: ") + status_text(agreed));
-        } else {
-            run_batches();
-        }
+        // mode R: a rank that failed must not leave its peers waiting inside the gather
+        agree_on_status(rr.shard_reps ? ctx->comm.get() : nullptr, st, run_batches, "another rank of the replicate-sharded run failed");
         if (cache) {
             if (mode == OB_CACHE_FILLED) {
                 cache->design_id = d->id; cache->x_gen = d->x_gen; cache->seed = o->seed;
-                cache->reps = o->reps; cache->rep_begin = rb; cache->rep_end = re; cache->slots = slots;
-                cache->shard_reps = shard_reps ? 1 : 0; cache->rep_world = rep_world; cache->rep_rank = rep_rank;
+                cache->reps = o->reps; cache->rep_begin = rr.rb; cache->rep_end = rr.re; cache->slots = slots;
+                cache->shard_reps = rr.shard_reps ? 1 : 0; cache->rep_world = rep_world; cache->rep_rank = rep_rank;
                 cache->row_world = d->world; cache->row_rank = d->rank; cache->K = K; cache->count_bytes = count_bytes;
                 cache->xx_ok = true;
             }
@@ -2378,31 +2304,19 @@ static void bootstrap_body(ob_ctx* ctx, const ob_design* d, const ob_boot_opts* 
         tr.mark("point + residuals queued", st, false);
 
         // ---- mode R: replicate rows of all ranks, device to device, into global replicate order ----
-        const int64_t reps_all = shard_reps ? o->reps : nrep;
+        const int64_t reps_all = rr.shard_reps ? o->reps : rr.nrep;
         DevBuf d_gstats, d_gstatus, d_gba, d_gbb;
         const double* stats_rows = d_stats.as<double>() + SE;     // [reps_all][T][S]
         const int* status_rows = d_status.as<int>() + 1;
         const double* ba_rows = want_beta ? d_ba.as<double>() + KE : nullptr;
         const double* bb_rows = want_beta ? d_bb.as<double>() + KE : nullptr;
-        if (shard_reps) {
+        if (rr.shard_reps) {
             Timer t_c(st, &res->ms_comm);
             Comm* cm = ctx->comm.get();
-            const int w = cm->world;
-            std::vector<size_t> off(w), sz(w);
-            auto gather_rows = [&](const void* mine, DevBuf& all, size_t row_bytes) {
-                all.alloc(row_bytes * (size_t)std::max<int64_t>(reps_all, 1));
-                for (int r = 0; r < w; ++r) {
-                    int64_t b = 0, e = 0;
-                    ob_replicate_shard(o->reps, w, r, &b, &e);
-                    off[r] = (size_t)b * row_bytes; sz[r] = (size_t)(e - b) * row_bytes;
-                }
-                cm->allgatherv(mine, all.p, off.data(), sz.data(), st);
-            };
-            gather_rows(stats_rows, d_gstats, sizeof(double) * (size_t)SE);
-            gather_rows(status_rows, d_gstatus, sizeof(int));
-            stats_rows = d_gstats.as<double>(); status_rows = d_gstatus.as<int>();
-            if (res->rep_beta_a) { gather_rows(ba_rows, d_gba, sizeof(double) * (size_t)KE); ba_rows = d_gba.as<double>(); }
-            if (res->rep_beta_b) { gather_rows(bb_rows, d_gbb, sizeof(double) * (size_t)KE); bb_rows = d_gbb.as<double>(); }
+            stats_rows = allgather_shards(cm, o->reps, SE, stats_rows, d_gstats, st);
+            status_rows = allgather_shards(cm, o->reps, 1, status_rows, d_gstatus, st);
+            if (res->rep_beta_a) ba_rows = allgather_shards(cm, o->reps, KE, ba_rows, d_gba, st);
+            if (res->rep_beta_b) bb_rows = allgather_shards(cm, o->reps, KE, bb_rows, d_gbb, st);
             t_c.stop(); OB_CUDA(cudaStreamSynchronize(st)); t_c.collect();
             tr.mark("replicate all-gather", st, false);
         }
@@ -2410,22 +2324,9 @@ static void bootstrap_body(ob_ctx* ctx, const ob_design* d, const ob_boot_opts* 
         // ---- (5) reduction to standard errors / p-values / percentile CIs ----
         if (!o->skip_reduce) {
             // the T x S statistics of a slot reduce independently: one launch over T*S columns; outputs are [T][S]
-            DevBuf d_out(sizeof(double) * 5 * (size_t)SE), d_nok(sizeof(long long)), d_rs(reduce_stats_scratch_bytes(reps_all, SE));
-            Timer t_red(st, &res->ms_reduce);
-            reduce_stats_launch(stats_rows, status_rows, reps_all, SE, d_stats.as<double>(),
-                                d_out.as<double>(), d_nok.as<long long>(), st, d_rs.as<double>());
-            res->gpu_launches += 1;
-            t_red.stop();
-            std::vector<double> out5(5 * (size_t)SE);
-            long long nok = 0;
-            OB_CUDA(cudaMemcpyAsync(out5.data(), d_out.p, d_out.bytes, cudaMemcpyDeviceToHost, st));
-            OB_CUDA(cudaMemcpyAsync(&nok, d_nok.p, sizeof nok, cudaMemcpyDeviceToHost, st));
-            OB_CUDA(cudaStreamSynchronize(st));
-            t_red.collect();
-            res->n_ok = nok;
             double* dst[5] = {res->std_err, res->p_value, res->ci_lower, res->ci_upper, res->t_stat};
-            for (int k = 0; k < 5; ++k)
-                if (dst[k]) memcpy(dst[k], out5.data() + (size_t)k * SE, sizeof(double) * SE);
+            reduce_to_host(st, stats_rows, status_rows, reps_all, SE, d_stats.as<double>(), dst, &res->n_ok, &res->ms_reduce);
+            res->gpu_launches += 1;
         }
         if (reps_all > 0) {
             if (res->rep_stats) OB_CUDA(cudaMemcpyAsync(res->rep_stats, stats_rows, sizeof(double) * (size_t)reps_all * SE, cudaMemcpyDeviceToHost, st));
@@ -2504,24 +2405,14 @@ ob_status ob_reduce_stats(ob_ctx* ctx, const double* rep_stats, const int32_t* r
     return guarded(ctx, [&] {
         cudaStream_t st = ctx->stream;
         DevBuf d_stats(sizeof(double) * (size_t)std::max<int64_t>(reps, 1) * S), d_status(sizeof(int) * (size_t)std::max<int64_t>(reps, 1));
-        DevBuf d_point(sizeof(double) * S), d_out(sizeof(double) * 5 * (size_t)S), d_nok(sizeof(long long));
-        DevBuf d_rs(reduce_stats_scratch_bytes(reps, S));
+        DevBuf d_point(sizeof(double) * S);
         if (reps) {
             OB_CUDA(cudaMemcpyAsync(d_stats.p, rep_stats, sizeof(double) * (size_t)reps * S, cudaMemcpyHostToDevice, st));
             OB_CUDA(cudaMemcpyAsync(d_status.p, rep_status, sizeof(int) * (size_t)reps, cudaMemcpyHostToDevice, st));
         }
         OB_CUDA(cudaMemcpyAsync(d_point.p, point_stats, sizeof(double) * S, cudaMemcpyHostToDevice, st));
-        reduce_stats_launch(d_stats.as<double>(), d_status.as<int>(), reps, S, d_point.as<double>(), d_out.as<double>(),
-                            d_nok.as<long long>(), st, d_rs.as<double>());
-        std::vector<double> out5(5 * (size_t)S);
-        long long nok = 0;
-        OB_CUDA(cudaMemcpyAsync(out5.data(), d_out.p, d_out.bytes, cudaMemcpyDeviceToHost, st));
-        OB_CUDA(cudaMemcpyAsync(&nok, d_nok.p, sizeof nok, cudaMemcpyDeviceToHost, st));
-        OB_CUDA(cudaStreamSynchronize(st));
-        if (n_ok) *n_ok = nok;
         double* dst[5] = {std_err, p_value, ci_lower, ci_upper, t_stat};
-        for (int k = 0; k < 5; ++k)
-            if (dst[k]) memcpy(dst[k], out5.data() + (size_t)k * S, sizeof(double) * S);
+        reduce_to_host(st, d_stats.as<double>(), d_status.as<int>(), reps, S, d_point.as<double>(), dst, n_ok, nullptr);
     });
 }
 
