@@ -197,6 +197,33 @@ ob_status ob_design_attach_selection(ob_ctx* ctx, ob_design* d, const ob_selecti
 ob_status ob_design_selection_cols(const ob_design* d, int32_t* k1_out);     /* 0 = no selection equation attached */
 int32_t ob_num_stats_heckman(int32_t K, int32_t K1);
 
+/* ---- cluster bootstrap: resample whole clusters instead of rows ---------------------------------------------------
+ * Rows nested in clusters (employees in firms, people in panels, households in PSUs) are not independent draws; under
+ * intra-cluster correlation the row bootstrap understates every SE, p-value and CI width.  A clustered design resamples
+ * UNITS with replacement, and a drawn unit brings all its rows; replicate b is the reference's run_single_pass
+ * (builder.rs:420-699) on the frame made of the drawn units' rows, so group sizes vary by replicate:
+ *   OB_CLUSTER_BY_GROUP  a unit is a (cluster, group) pair; each replicate draws M_A units from group A's and M_B from group
+ *                        B's, independently (M_g = clusters with at least one row in group g).  With singleton clusters
+ *                        this is the row bootstrap; coded in frame order, the native stream gives its counts bit for bit.
+ *   OB_CLUSTER_JOINT     one stratum: a unit is a cluster with a row in group A or B, each replicate draws M of them and a
+ *                        drawn unit contributes its rows of both groups.  A group can come out empty or too small; such a
+ *                        replicate fails (OB_ERR_INVALID_GROUP / OB_ERR_INSUFFICIENT_DATA) and is dropped like any failed
+ *                        replicate.
+ * Units are numbered by ascending cluster code; an explicit index stream (ob_boot_opts.idx_a / idx_b) draws unit positions:
+ * BY_GROUP idx_a [reps x M_A], idx_b [reps x M_B]; JOINT idx_a [reps x M] with idx_b = NULL.  The native stream is keyed
+ * like the row stream by (seed; unit, stream tag, global replicate id), tag = the group under BY_GROUP and 2 under JOINT,
+ * so results do not depend on batching or replicate sharding.  The point estimate and RIF outcomes use the full sample.
+ * codes_frame [n_frame]: one code in [0, n_codes) per row of the frame the design was packed from (rows the cleaning
+ * dropped are never read; a kept row's code out of range is OB_ERR_INVALID_ARG).  strata NONE detaches (codes may be NULL)
+ * and the design resamples rows again.  Attaching or detaching invalidates a Gram cache's X'WX (the next cached run fills).
+ * Refused (OB_ERR_UNSUPPORTED): row-sharded designs (mode N), designs with a selection equation (either order), and
+ * ob_mm_run on a clustered design.  ob_debug_counts returns the expanded row counts of the native stream. */
+typedef enum { OB_CLUSTER_NONE = 0, OB_CLUSTER_BY_GROUP = 1, OB_CLUSTER_JOINT = 2 } ob_cluster_strata;
+ob_status ob_design_attach_clusters(ob_ctx* ctx, ob_design* d, const int32_t* codes_frame, int64_t n_frame,
+                                    int32_t n_codes, int32_t strata);
+/* strata and unit counts of a design (NONE, 0, 0 when unclustered; JOINT: units_a == units_b == M) */
+ob_status ob_design_clusters(const ob_design* d, int32_t* strata, int64_t* units_a, int64_t* units_b);
+
 /* ---- (2)-(5) bootstrap ---------------------------------------------------------------------*/
 typedef struct ob_boot_opts {
     int32_t ref_kind;                /* ob_ref_kind; builder default is GROUP_A (builder.rs:123) */

@@ -47,6 +47,11 @@ ob_status ob_builder_heckman_selection(ob_builder* b, const char* outcome, const
 ob_status ob_builder_seed(ob_builder* b, uint64_t seed);
 ob_status ob_builder_device(ob_builder* b, int32_t device);
 ob_status ob_builder_index_stream(ob_builder* b, const uint32_t* idx_a, const uint32_t* idx_b);
+/* cluster bootstrap (ob_design_attach_clusters): resample whole clusters of `column` (string or numeric labels, coded in
+ * their sorted order; the column joins the null filter) with ob_cluster_strata `strata`; OB_CLUSTER_NONE resamples rows
+ * again.  run, run_outcomes and decompose_quantile honour it; an index stream then draws units (joint: idx_b = NULL).
+ * The results gain a summary line and a "clusters" JSON key {strata, units_a, units_b}. */
+ob_status ob_builder_cluster(ob_builder* b, const char* column, int32_t strata);
 
 ob_status ob_builder_run(ob_builder* b, ob_results** out);
 /* run() once per outcome column names[n] (f64 columns) on ONE ingest: rows are cleaned over every listed column (plus the

@@ -31,7 +31,7 @@ SYMBOLS = ["ob_abi_version", "ob_device_count", "ob_ctx_create", "ob_ctx_destroy
            "ob_design_redistribute_rows", "ob_design_row_shard", "ob_design_apply_rif_multi", "ob_design_num_outcomes",
            "ob_design_pack_row_shard_async", "ob_design_attach_selection", "ob_design_selection_cols", "ob_num_stats_heckman",
            "ob_mm_run", "ob_debug_gram_columns", "ob_gram_cache_create", "ob_gram_cache_destroy", "ob_gram_cache_last_use",
-           "ob_bootstrap_run_cached", "ob_debug_gram_outcome_columns"]
+           "ob_bootstrap_run_cached", "ob_debug_gram_outcome_columns", "ob_design_attach_clusters", "ob_design_clusters"]
 
 
 class FrameView(C.Structure):
@@ -172,6 +172,8 @@ def lib() -> C.CDLL:
         L.ob_design_num_outcomes.argtypes = [C.c_void_p, _IP]
         L.ob_design_attach_selection.argtypes = [C.c_void_p, C.c_void_p, C.POINTER(SelectionView), C.c_int64]
         L.ob_design_selection_cols.argtypes = [C.c_void_p, _IP]
+        L.ob_design_attach_clusters.argtypes = [C.c_void_p, C.c_void_p, _IP, C.c_int64, C.c_int32, C.c_int32]
+        L.ob_design_clusters.argtypes = [C.c_void_p, _IP, C.POINTER(C.c_int64), C.POINTER(C.c_int64)]
         L.ob_num_stats_heckman.argtypes = [C.c_int32, C.c_int32]
         L.ob_num_stats_heckman.restype = C.c_int32
         L.ob_design_row_shard.argtypes = [C.c_void_p, C.POINTER(C.c_int64), C.POINTER(C.c_int64), _IP, _IP]

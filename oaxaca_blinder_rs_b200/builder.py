@@ -56,6 +56,7 @@ def _blib():
         L.ob_builder_bootstrap_reps.argtypes = [vp, i64]
         L.ob_builder_reference_coefficients.argtypes = [vp, i32]
         L.ob_builder_heckman_selection.argtypes = [vp, cp, C.POINTER(cp), i32]
+        L.ob_builder_cluster.argtypes = [vp, cp, i32]
         L.ob_builder_seed.argtypes = [vp, C.c_uint64]
         L.ob_builder_device.argtypes = [vp, i32]
         L.ob_builder_index_stream.argtypes = [vp, N._U32P, N._U32P]
@@ -96,7 +97,7 @@ BUILDER_SYMBOLS = ["ob_frame_new", "ob_frame_free", "ob_frame_add_f64", "ob_fram
                    "ob_builder_new", "ob_builder_from_formula", "ob_builder_free", "ob_builder_predictors",
                    "ob_builder_categorical_predictors", "ob_builder_normalize", "ob_builder_weights",
                    "ob_builder_bootstrap_reps", "ob_builder_reference_coefficients", "ob_builder_heckman_selection",
-                   "ob_builder_seed", "ob_builder_device", "ob_builder_index_stream", "ob_builder_run", "ob_builder_run_outcomes",
+                   "ob_builder_cluster", "ob_builder_seed", "ob_builder_device", "ob_builder_index_stream", "ob_builder_run", "ob_builder_run_outcomes",
                    "ob_builder_decompose_quantile", "ob_builder_get_data_matrices", "ob_builder_describe", "ob_builder_last_error", "ob_builder_last_status",
                    "ob_results_free", "ob_results_json", "ob_results_summary", "ob_results_markdown",
                    "ob_results_residuals",
@@ -214,6 +215,7 @@ class OaxacaResults:
         self.bootstrap_reps, self.successful_bootstraps = d["bootstrap_reps"], d["successful_bootstraps"]
         self.predictor_names = d["predictor_names"]
         self.timings_ms = dict(total=d["ms_total"], gram=d["ms_gram"])
+        self.clusters = d.get("clusters")        # dict(strata, units_a, units_b) on a cluster bootstrap, else None
         n = L.ob_results_residuals(handle, None)
         self.residuals = np.empty(n)
         L.ob_results_residuals(handle, self.residuals.ctypes.data_as(N._DP))
@@ -297,15 +299,28 @@ class OaxacaBuilder:
     def seed(self, seed: int):
         return self._check(_blib().ob_builder_seed(self._h, int(seed)))
 
+    def cluster(self, column: Optional[str], strata: Optional[str] = "group"):
+        """Cluster bootstrap: resample whole clusters of `column` (string or numeric labels) instead of rows.  strata
+        "group": a unit is a (cluster, group) pair and each group resamples its own units; "joint": one stratum, a drawn
+        cluster brings its rows of both groups; None: resample rows again.  The column joins the null filter."""
+        from .core import CLUSTER_NONE, CLUSTER_STRATA
+        if strata is None or column is None:
+            return self._check(_blib().ob_builder_cluster(self._h, None, CLUSTER_NONE))
+        if strata not in CLUSTER_STRATA:
+            raise ValueError(f"strata must be 'group', 'joint' or None, not {strata!r}")
+        return self._check(_blib().ob_builder_cluster(self._h, column.encode(), CLUSTER_STRATA[strata]))
+
     def device(self, device: int):
         return self._check(_blib().ob_builder_device(self._h, int(device)))
 
     def index_stream(self, idx_a, idx_b):
-        """Test-only explicit resample index stream [reps x n_a], [reps x n_b] (row positions within each group)."""
+        """Test-only explicit resample index stream [reps x n_a], [reps x n_b] (row positions within each group).  Under
+        cluster(): unit positions, [reps x units_a], [reps x units_b], or idx_a [reps x M] and idx_b=None for joint strata."""
         ia = np.ascontiguousarray(idx_a, dtype=np.uint32)
-        ib = np.ascontiguousarray(idx_b, dtype=np.uint32)
+        ib = None if idx_b is None else np.ascontiguousarray(idx_b, dtype=np.uint32)
         self._keep = [ia, ib]
-        return self._check(_blib().ob_builder_index_stream(self._h, ia.ctypes.data_as(N._U32P), ib.ctypes.data_as(N._U32P)))
+        return self._check(_blib().ob_builder_index_stream(self._h, ia.ctypes.data_as(N._U32P),
+                                                           None if ib is None else ib.ctypes.data_as(N._U32P)))
 
     def run(self) -> OaxacaResults:                                  # builder.rs:787
         out = C.c_void_p()

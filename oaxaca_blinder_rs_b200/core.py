@@ -117,6 +117,8 @@ def row_shard_plan(n_group: int, world: int, rank: int):
 
 
 CACHE_NONE, CACHE_FILLED, CACHE_OUTCOME_ONLY, CACHE_SOLVE_ONLY = 0, 1, 2, 3
+CLUSTER_NONE, CLUSTER_BY_GROUP, CLUSTER_JOINT = 0, 1, 2
+CLUSTER_STRATA = {"group": CLUSTER_BY_GROUP, "joint": CLUSTER_JOINT}
 CACHE_USE_NAMES = {CACHE_NONE: "none", CACHE_FILLED: "filled", CACHE_OUTCOME_ONLY: "outcome_only", CACHE_SOLVE_ONLY: "solve_only"}
 
 
@@ -297,6 +299,32 @@ class Design:
         arr = (N._DP * max(len(preds), 1))(*[_dp(p) for p in preds])
         sv.pred, sv.outcome = arr, _dp(s)
         self.ctx.check(N.lib().ob_design_attach_selection(self.ctx._h, self._h, C.byref(sv), s.shape[0]))
+
+    def attach_clusters(self, codes, n_codes: Optional[int] = None, strata: Optional[str] = "group"):
+        """ob_design_attach_clusters: resample whole clusters instead of rows.  codes: one integer code in [0, n_codes) per
+        row of the frame this design was packed from (n_codes defaults to max + 1); strata "group" (a unit is a (cluster,
+        group) pair, each group resamples its own units), "joint" (one stratum: a drawn cluster brings its rows of both
+        groups) or None (detach: rows are resampled again).  Units are numbered by ascending code; an explicit index stream
+        passed to bootstrap() then draws units (see `clusters`)."""
+        if strata is None:
+            self.ctx.check(N.lib().ob_design_attach_clusters(self.ctx._h, self._h, None, 0, 0, CLUSTER_NONE))
+            return
+        if strata not in CLUSTER_STRATA:
+            raise ValueError(f"strata must be 'group', 'joint' or None, not {strata!r}")
+        c = np.ascontiguousarray(codes, dtype=np.int32)
+        if n_codes is None:
+            n_codes = int(c.max()) + 1 if c.size else 1
+        self.ctx.check(N.lib().ob_design_attach_clusters(self.ctx._h, self._h, _ip(c), c.shape[0], int(n_codes),
+                                                         CLUSTER_STRATA[strata]))
+
+    @property
+    def clusters(self) -> Optional[dict]:
+        """None when rows are resampled, else dict(strata="group" | "joint", units_a=M_A, units_b=M_B) (joint: both = M)."""
+        st, ua, ub = C.c_int32(), C.c_int64(), C.c_int64()
+        N.lib().ob_design_clusters(self._h, C.byref(st), C.byref(ua), C.byref(ub))
+        if st.value == CLUSTER_NONE:
+            return None
+        return dict(strata="joint" if st.value == CLUSTER_JOINT else "group", units_a=ua.value, units_b=ub.value)
 
     @property
     def selection_cols(self) -> int:
@@ -483,6 +511,8 @@ def bootstrap(design: Design, reps: int, ref_kind: int = REF_GROUP_A, norm: Sequ
               want_rep: bool = False, want_residuals: bool = True, residuals_out: Optional[np.ndarray] = None,
               shard_replicates: bool = False, cache: Optional[GramCache] = None) -> dict:
     """ob_bootstrap_run (ob_bootstrap_run_cached with a GramCache: same results, and `cache_use` in the dict).  Returns point estimates, per-statistic SE/p/CI/t and (optionally) replicate detail.
+    On a clustered design (Design.attach_clusters) idx_a / idx_b draw units: [reps x units_a] / [reps x units_b], or
+    idx_a [reps x M] with idx_b=None under joint strata.
     residuals_out: optional preallocated float64 [n_b] buffer for OaxacaResults.residuals (reusing one across calls
     avoids first-touch page faults on a fresh 8 n_b byte array during the device-to-host copy; a page-locked one --
     pinned_empty() -- takes the DMA directly).
@@ -505,10 +535,18 @@ def bootstrap(design: Design, reps: int, ref_kind: int = REF_GROUP_A, norm: Sequ
     hb = np.array([int(v.has_base) for v in norm] + [0], dtype=np.int32)
     o.norm_m, o.norm_off, o.norm_idx, o.norm_has_base = _ip(m), _ip(off), _ip(idx), _ip(hb)
     o.reps, o.seed = reps, seed
-    if idx_a is not None:
+    cl = design.clusters
+    if idx_a is not None and cl is not None and cl["strata"] == "joint":
+        # one unit stream over both groups
+        assert idx_b is None, "a joint cluster design takes one unit stream (idx_b=None)"
+        idx_a = np.ascontiguousarray(idx_a, dtype=np.uint32)
+        assert idx_a.shape == (reps, cl["units_a"])
+        o.idx_a = idx_a.ctypes.data_as(N._U32P)
+    elif idx_a is not None:
         idx_a = np.ascontiguousarray(idx_a, dtype=np.uint32)
         idx_b = np.ascontiguousarray(idx_b, dtype=np.uint32)
-        assert idx_a.shape == (reps, design.n_a_global) and idx_b.shape == (reps, design.n_b_global)
+        n_a, n_b = (cl["units_a"], cl["units_b"]) if cl is not None else (design.n_a_global, design.n_b_global)
+        assert idx_a.shape == (reps, n_a) and idx_b.shape == (reps, n_b)
         o.idx_a, o.idx_b = idx_a.ctypes.data_as(N._U32P), idx_b.ctypes.data_as(N._U32P)
     o.rep_begin, o.rep_end = rep_begin, rep_end
     o.skip_reduce, o.count_bits, o.max_workspace_bytes = int(skip_reduce), count_bits, max_workspace_bytes

@@ -70,6 +70,10 @@ struct ob_design {
     int world = 1, rank = 0;         // row sharding (mode N): this design holds rank's rows of a world-way split
     double ms_h2d = 0.0, ms_pack = 0.0;   // device time of the column upload and of the pack kernels (ob_design_pack)
     GroupData g[2];
+    // clusters (ob_design_attach_clusters): ob_cluster_strata and the resampling units of each stratum (JOINT: both = M);
+    // the unit of every packed row is GroupData::uid
+    int cl_strata = OB_CLUSTER_NONE;
+    int64_t cl_units[2] = {0, 0};
     // identity for ob_gram_cache keys: a process-wide unique id (addresses are reused after destroy), the generation of
     // the design columns / weights / rows / row-shard marking, and the generation of the outcome columns
     uint64_t id = 0, x_gen = 0, y_gen = 0;
@@ -83,6 +87,7 @@ struct ob_gram_cache {
     int last_use = OB_CACHE_NONE;
     double* xx = nullptr; size_t xx_bytes = 0;   // [2][slots][K(K+1)/2]
     double* yy = nullptr; size_t yy_bytes = 0;   // [2][slots][K T + 1]
+    long long* rows = nullptr; size_t rows_bytes = 0;   // clustered designs: [2][slots] group row counts (a SOLVE_ONLY run draws none)
     // key of xx (valid while xx_ok): what decides the resamples and the design's X'WX
     bool xx_ok = false;
     uint64_t design_id = 0, x_gen = 0, seed = 0;
@@ -264,7 +269,8 @@ void design_release_device(ob_design* d) {
         if (g.hk_Z) cudaFreeAsync(g.hk_Z, st);
         if (g.hk_sel) cudaFreeAsync(g.hk_sel, st);
         if (g.hk_Xm) cudaFreeAsync(g.hk_Xm, st);
-        g.X = g.w = g.Xs = g.y_raw = g.hk_Z = g.hk_Xm = nullptr; g.src = nullptr; g.hk_sel = nullptr;
+        if (g.uid) cudaFreeAsync(g.uid, st);
+        g.X = g.w = g.Xs = g.y_raw = g.hk_Z = g.hk_Xm = nullptr; g.src = g.uid = nullptr; g.hk_sel = nullptr;
     }
 }
 
@@ -274,8 +280,9 @@ void cache_release_device(ob_gram_cache* c) {
         cudaStream_t st = c->owner->stream;
         if (c->xx) cudaFreeAsync(c->xx, st);
         if (c->yy) cudaFreeAsync(c->yy, st);
+        if (c->rows) cudaFreeAsync(c->rows, st);
     }
-    c->xx = c->yy = nullptr; c->xx_bytes = c->yy_bytes = 0;
+    c->xx = c->yy = nullptr; c->rows = nullptr; c->xx_bytes = c->yy_bytes = c->rows_bytes = 0;
     c->xx_ok = c->y_ok = false;
 }
 
@@ -371,8 +378,10 @@ struct RepRange {
     bool index_mode; int count_bytes;
 };
 
+// On a clustered design an explicit index stream draws units: BY_GROUP idx_a [reps x M_A] and idx_b [reps x M_B], JOINT
+// idx_a [reps x M] alone.
 template <typename Opts>
-RepRange replicate_range(const ob_ctx* ctx, const Opts* o) {
+RepRange replicate_range(const ob_ctx* ctx, const ob_design* d, const Opts* o) {
     if (o->reps < 0) fail(OB_ERR_INVALID_ARG, "negative reps");
     RepRange r;
     r.shard_reps = o->shard_replicates != 0 && ctx->comm && ctx->comm->world > 1;
@@ -382,7 +391,9 @@ RepRange replicate_range(const ob_ctx* ctx, const Opts* o) {
     if (r.rb < 0 || r.re < r.rb || r.re > o->reps) fail(OB_ERR_INVALID_ARG, "bad replicate shard");
     r.nrep = r.re - r.rb;
     r.index_mode = o->idx_a != nullptr || o->idx_b != nullptr;
-    if (r.index_mode && r.nrep > 0 && (!o->idx_a || !o->idx_b)) fail(OB_ERR_INVALID_ARG, "index stream needs both idx_a and idx_b");
+    if (d->cl_strata == OB_CLUSTER_JOINT) {
+        if (o->idx_b) fail(OB_ERR_INVALID_ARG, "a JOINT cluster design takes one unit stream: idx_a [reps x M] and idx_b = NULL");
+    } else if (r.index_mode && r.nrep > 0 && (!o->idx_a || !o->idx_b)) fail(OB_ERR_INVALID_ARG, "index stream needs both idx_a and idx_b");
     if (o->count_bits != 0 && o->count_bits != 8 && o->count_bits != 16) fail(OB_ERR_INVALID_ARG, "count_bits must be 0, 8 or 16");
     r.count_bytes = o->count_bits == 16 ? 2 : 1;
     return r;
@@ -410,20 +421,47 @@ struct Batch {
 // shards: row_comm is the mode-N communicator (null otherwise; ms_comm then goes unused).  On a design that is not row
 // sharded, shard.n_global == n and shard.row_begin == 0: alloc_group sets row_shard(n, 0, 1), and ob_design_set_row_shard
 // with world 1 accepts only n_global == n.  colsum holds 2 x ppb * BM sums.  Returns the number of kernels launched.
+// A clustered design (cw non-null) draws the same streams over its units into cw->U (unit_mats matrices: one per group, or
+// one for both under JOINT, keyed with stream tag 2), then expands them to the row matrices C and sums the per-slot row
+// counts into cw->rows [2][b.pn * BM].
+struct ClusterWork {
+    DevBuf U[2];                  // [ppb][pad_rows(M)][BM]
+    long long* rows = nullptr;    // [2][ppb * BM]
+};
+int unit_mats(const ob_design* d) { return d->cl_strata == OB_CLUSTER_JOINT ? 1 : 2; }
+
 template <typename Opts>
 int generate_counts(const ob_design* d, const Opts* o, const Batch& b, int count_bytes, int64_t ppb, DevBuf (&C)[2],
-                    DevBuf (&idx)[2], DevBuf& colsum, DevBuf& lut, int* flags, Comm* row_comm, double* ms_comm, cudaStream_t st) {
+                    DevBuf (&idx)[2], DevBuf& colsum, DevBuf& lut, int* flags, Comm* row_comm, double* ms_comm, cudaStream_t st,
+                    ClusterWork* cw = nullptr) {
     CountsArgs ca[2];
-    for (int g = 0; g < 2; ++g) {
+    const int mats = cw ? unit_mats(d) : 2;
+    for (int g = 0; g < mats; ++g) {
         const GroupData& G = d->g[g];
         ca[g].C = C[g].p; ca[g].count_bytes = count_bytes; ca[g].n = G.n; ca[g].n_pad = G.n_pad;
         ca[g].n_global = G.shard.n_global; ca[g].row_begin = G.shard.row_begin;
         ca[g].panels = (int)b.pn; ca[g].slots = b.bslots; ca[g].first_slot = b.first_slot; ca[g].rep0 = b.rep0;
         ca[g].group = g; ca[g].seed = o->seed;
+        if (cw) {                 // units take the place of rows: M of them, in ascending cluster code
+            const int64_t M = d->cl_units[g];
+            ca[g].C = cw->U[g].p; ca[g].n = ca[g].n_global = M; ca[g].n_pad = pad_rows(M); ca[g].row_begin = 0;
+            ca[g].group = mats == 1 ? 2 : g;
+        }
     }
     int launches = 0;
-    if (o->idx_a || o->idx_b) {
+    auto expand = [&] {
+        if (!cw) return;
+        OB_CUDA(cudaMemsetAsync(cw->rows, 0, sizeof(long long) * 2 * (size_t)b.pn * BM, st));
         for (int g = 0; g < 2; ++g) {
+            const int m = mats == 1 ? 0 : g;
+            ExpandArgs ea{C[g].p, cw->U[m].p, d->g[g].uid, count_bytes, d->g[g].n, d->g[g].n_pad, pad_rows(d->cl_units[m]),
+                          (int)b.pn, b.bslots, cw->rows + (size_t)g * b.pn * BM};
+            counts_expand_launch(ea, st);
+            launches += 1;
+        }
+    };
+    if (o->idx_a || o->idx_b) {
+        for (int g = 0; g < mats; ++g) {
             const uint32_t* h = g == 0 ? o->idx_a : o->idx_b;
             const int64_t n_glob = ca[g].n_global;
             const size_t nb = sizeof(uint32_t) * (size_t)std::max<int64_t>(b.brep, 1) * n_glob;
@@ -434,11 +472,12 @@ int generate_counts(const ob_design* d, const Opts* o, const Batch& b, int count
             counts_from_indices(ca[g], idx[g].as<uint32_t>(), flags, st);
             launches += 1 + (b.brep > 0 ? (int)((b.brep + 32767) / 32768) : 0);
         }
+        expand();
         return launches;
     }
     long long* sums[2] = {colsum.as<long long>(), colsum.as<long long>() + (size_t)ppb * BM};
     OB_CUDA(cudaMemsetAsync(colsum.p, 0, colsum.bytes, st));
-    for (int g = 0; g < 2; ++g) {
+    for (int g = 0; g < mats; ++g) {
         counts_philox_body_launch(ca[g], sums[g], lut.as<unsigned char>() + (size_t)g * counts_lut_bytes(), st);
         launches += 2;
     }
@@ -447,10 +486,11 @@ int generate_counts(const ob_design* d, const Opts* o, const Batch& b, int count
         row_comm->allreduce(colsum.p, 2 * (size_t)ppb * BM, CommDType::I64, CommOp::SUM, st);
         t_c.stop(); OB_CUDA(cudaStreamSynchronize(st)); t_c.collect();
     }
-    for (int g = 0; g < 2; ++g) {
+    for (int g = 0; g < mats; ++g) {
         counts_philox_fixup_launch(ca[g], sums[g], flags, st);
         launches += b.brep > 0 ? 1 : 0;
     }
+    expand();
     return launches;
 }
 
@@ -1494,6 +1534,8 @@ ob_status ob_design_attach_selection(ob_ctx* ctx, ob_design* d, const ob_selecti
         if (!sv->outcome || (sv->n_pred && !sv->pred)) fail(OB_ERR_INVALID_ARG, "null selection column");
         if (n_frame != d->n_frame) fail(OB_ERR_INVALID_ARG, "selection columns differ in length from the frame the design was packed from");
         if (d->world > 1) fail(OB_ERR_UNSUPPORTED, "Heckman selection on a row-sharded design");
+        if (d->cl_strata != OB_CLUSTER_NONE)
+            fail(OB_ERR_UNSUPPORTED, "Heckman selection on a clustered design: its estimator assumes constant group sizes (detach the clusters)");
         if (d->weighted) fail(OB_ERR_UNSUPPORTED, "Heckman selection with sample weights (the reference's estimator ignores them, estimation.rs:132-133)");
         if (!d->g[0].src || !d->g[1].src) fail(OB_ERR_UNSUPPORTED, "this design carries no frame-row map");
         cudaStream_t st = ctx->stream;
@@ -1532,6 +1574,84 @@ ob_status ob_design_attach_selection(ob_ctx* ctx, ob_design* d, const ob_selecti
     });
 }
 
+// Cluster labels (cluster.cu): the codes of the kept rows are gathered through each group's frame-row map, checked on the
+// device, and the codes present in a stratum numbered in ascending order (the units).  The design is changed only once
+// everything has succeeded.
+ob_status ob_design_attach_clusters(ob_ctx* ctx, ob_design* d, const int32_t* codes_frame, int64_t n_frame, int32_t n_codes,
+                                    int32_t strata) {
+    if (!ctx || !d) return OB_ERR_INVALID_ARG;
+    return guarded(ctx, [&] {
+        design_ready(d);
+        cudaStream_t st = ctx->stream;
+        if (strata != OB_CLUSTER_NONE && strata != OB_CLUSTER_BY_GROUP && strata != OB_CLUSTER_JOINT)
+            fail(OB_ERR_INVALID_ARG, "strata must be OB_CLUSTER_NONE, OB_CLUSTER_BY_GROUP or OB_CLUSTER_JOINT");
+        auto install = [&](uint32_t* const uid[2], int st_new, const int64_t units[2]) {
+            for (int g = 0; g < 2; ++g) {
+                if (d->g[g].uid) cudaFreeAsync(d->g[g].uid, st);
+                d->g[g].uid = uid[g];
+                d->cl_units[g] = units[g];
+            }
+            d->cl_strata = st_new;
+            ++d->x_gen;              // the resamples change: a Gram cache refills
+        };
+        if (strata == OB_CLUSTER_NONE) {
+            uint32_t* none[2] = {nullptr, nullptr};
+            const int64_t zero[2] = {0, 0};
+            install(none, OB_CLUSTER_NONE, zero);
+            return;
+        }
+        if (n_frame != d->n_frame) fail(OB_ERR_INVALID_ARG, "cluster codes differ in length from the frame the design was packed from");
+        if (!codes_frame && n_frame > 0) fail(OB_ERR_INVALID_ARG, "null cluster codes");
+        if (n_codes < 1) fail(OB_ERR_INVALID_ARG, "n_codes must be at least 1");
+        if (d->world > 1) fail(OB_ERR_UNSUPPORTED, "clusters on a row-sharded design (mode N): a unit's rows may sit on several ranks");
+        if (d->K1 > 0)
+            fail(OB_ERR_UNSUPPORTED, "clusters on a design with a selection equation: the Heckman estimator assumes constant group sizes");
+        if (!d->g[0].src || !d->g[1].src) fail(OB_ERR_UNSUPPORTED, "this design carries no frame-row map");
+        g_alloc_pack = true;
+        struct Uids {               // the new maps, released unless installed
+            uint32_t* p[2] = {nullptr, nullptr}; cudaStream_t st;
+            ~Uids() { for (auto q : p) if (q) cudaFreeAsync(q, st); }
+        } nu{{nullptr, nullptr}, st};
+        for (int g = 0; g < 2; ++g)
+            OB_CUDA(cudaMallocFromPoolAsync((void**)&nu.p[g], sizeof(uint32_t) * (size_t)std::max<int64_t>(d->g[g].n, 1), ctx->pool_design, st));
+        const int nstrata = strata == OB_CLUSTER_JOINT ? 1 : 2;
+        DevBuf d_codes(sizeof(int32_t) * (size_t)std::max<int64_t>(n_frame, 1)), d_flags(sizeof(int) * 4);
+        DevBuf d_present((size_t)nstrata * n_codes), d_unit(sizeof(uint32_t) * (size_t)nstrata * n_codes), d_units(sizeof(long long) * 2);
+        if (n_frame) OB_CUDA(cudaMemcpyAsync(d_codes.p, codes_frame, sizeof(int32_t) * (size_t)n_frame, cudaMemcpyHostToDevice, st));
+        OB_CUDA(cudaMemsetAsync(d_flags.p, 0, d_flags.bytes, st));
+        OB_CUDA(cudaMemsetAsync(d_present.p, 0, d_present.bytes, st));
+        OB_CUDA(cudaMemsetAsync(d_units.p, 0, d_units.bytes, st));
+        for (int g = 0; g < 2; ++g) {
+            const int m = nstrata == 1 ? 0 : g;
+            cluster_gather_launch(d_codes.as<int32_t>(), d->g[g].src, d->g[g].n, n_codes, nu.p[g],
+                                  d_present.as<uint8_t>() + (size_t)m * n_codes, d_flags.as<int>(), st);
+        }
+        for (int m = 0; m < nstrata; ++m)
+            cluster_scan_launch(d_present.as<uint8_t>() + (size_t)m * n_codes, n_codes, d_unit.as<uint32_t>() + (size_t)m * n_codes,
+                                d_units.as<long long>() + m, st);
+        for (int g = 0; g < 2; ++g)
+            cluster_remap_launch(nu.p[g], d->g[g].n, d_unit.as<uint32_t>() + (size_t)(nstrata == 1 ? 0 : g) * n_codes, st);
+        int flags[4];
+        long long units[2];
+        OB_CUDA(cudaMemcpyAsync(flags, d_flags.p, sizeof flags, cudaMemcpyDeviceToHost, st));
+        OB_CUDA(cudaMemcpyAsync(units, d_units.p, sizeof units, cudaMemcpyDeviceToHost, st));
+        OB_CUDA(cudaStreamSynchronize(st));
+        if (flags[0]) fail(OB_ERR_INVALID_ARG, "cluster code outside [0, n_codes) on a row the design holds");
+        if (nstrata == 1) units[1] = units[0];
+        const int64_t u[2] = {units[0], units[1]};
+        install(nu.p, strata, u);
+        nu.p[0] = nu.p[1] = nullptr;
+    });
+}
+
+ob_status ob_design_clusters(const ob_design* d, int32_t* strata, int64_t* units_a, int64_t* units_b) {
+    if (!d) return OB_ERR_INVALID_ARG;
+    if (strata) *strata = d->cl_strata;
+    if (units_a) *units_a = d->cl_units[0];
+    if (units_b) *units_b = d->cl_units[1];
+    return OB_OK;
+}
+
 }  // extern "C"
 
 namespace {
@@ -1546,7 +1666,7 @@ void heckman_run(ob_ctx* ctx, const ob_design* d, const ob_boot_opts* o, ob_resu
                                  "coefficients, the Heckman fits K + 1 (builder.rs:548-589 vs estimation.rs:139-141)");
     if (d->T != 1) fail(OB_ERR_UNSUPPORTED, "Heckman selection on a multi-outcome design");
     if (d->world > 1) fail(OB_ERR_UNSUPPORTED, "Heckman selection on a row-sharded design");
-    RepRange rr = replicate_range(ctx, o);
+    RepRange rr = replicate_range(ctx, d, o);
     // mode R inside the library, as for the OLS path: this rank's contiguous share of the global replicate ids
     if (rr.shard_reps) { ob_replicate_shard(o->reps, ctx->comm->world, ctx->comm->rank, &rr.rb, &rr.re); rr.nrep = rr.re - rr.rb; }
     if (d->g[0].n == 0 || d->g[1].n == 0) fail(OB_ERR_INVALID_GROUP, "Invalid group variable: One group has no data");
@@ -1743,7 +1863,7 @@ void mm_run(ob_ctx* ctx, const ob_design* d, const ob_mm_opts* o, ob_mm_result* 
     // the coefficients are all-gathered device to device, and effects + reduction run on every rank.  With the builder's
     // default of 20 passes a pass-level split over 8 GPUs would leave ranks with 4 or 3 passes (the point pass included)
     // against 2.6 on average; the problem-level split is even to one regression.
-    const RepRange rr = replicate_range(ctx, o);
+    const RepRange rr = replicate_range(ctx, d, o);
     const bool draws_given = o->draw_a != nullptr || o->draw_b != nullptr;
     if (draws_given && (!o->draw_a || !o->draw_b)) fail(OB_ERR_INVALID_ARG, "simulated-row stream needs both draw_a and draw_b");
     if (draws_given && rr.nrep > 0 && !rr.index_mode)
@@ -1922,6 +2042,8 @@ ob_status ob_mm_run(ob_ctx* ctx, const ob_design* d, const ob_mm_opts* o, ob_mm_
     if (!ctx || !d || !o || !res) return OB_ERR_INVALID_ARG;
     return guarded(ctx, [&] {
         design_ready(d);
+        if (d->cl_strata != OB_CLUSTER_NONE)
+            fail(OB_ERR_UNSUPPORTED, "Machado-Mata on a clustered design: its row draws assume constant group sizes (detach the clusters)");
         mm_run(ctx, d, o, res);
     });
 }
@@ -1940,9 +2062,12 @@ static void bootstrap_body(ob_ctx* ctx, const ob_design* d, const ob_boot_opts* 
         }
         cudaStream_t st = ctx->stream;
         const int K = d->K, T = d->T;
+        const bool clustered = d->cl_strata != OB_CLUSTER_NONE;
+        if (clustered && d->world > 1)
+            fail(OB_ERR_UNSUPPORTED, "clusters on a row-sharded design (mode N): a unit's rows may sit on several ranks");
         if (o->ref_kind < 0 || o->ref_kind > 3) fail(OB_ERR_INVALID_ARG, "ref_kind out of range");
         if (o->n_norm < 0) fail(OB_ERR_INVALID_ARG, "negative n_norm");
-        RepRange rr = replicate_range(ctx, o);
+        RepRange rr = replicate_range(ctx, d, o);
         if (o->shard_replicates && d->world > 1) fail(OB_ERR_INVALID_ARG, "shard_replicates on a row-sharded design (its communicator shards rows)");
         // mode R inside the library: this rank's contiguous share of the global replicate ids
         if (rr.shard_reps) { ob_replicate_shard(o->reps, ctx->comm->world, ctx->comm->rank, &rr.rb, &rr.re); rr.nrep = rr.re - rr.rb; }
@@ -2014,6 +2139,11 @@ static void bootstrap_body(ob_ctx* ctx, const ob_design* d, const ob_boot_opts* 
             cache->xx_bytes = sizeof(double) * 2 * (size_t)slots * nx;
             OB_CUDA(cudaMallocFromPoolAsync((void**)&cache->xx, cache->xx_bytes, ctx->pool_design, st));
             cache_new_bytes += cache->xx_bytes;
+            if (clustered) {
+                cache->rows_bytes = sizeof(long long) * 2 * (size_t)slots;
+                OB_CUDA(cudaMallocFromPoolAsync((void**)&cache->rows, cache->rows_bytes, ctx->pool_design, st));
+                cache_new_bytes += cache->rows_bytes;
+            }
         }
         if (mode == OB_CACHE_FILLED || outcome_only) {
             cache->y_ok = false;
@@ -2034,6 +2164,11 @@ static void bootstrap_body(ob_ctx* ctx, const ob_design* d, const ob_boot_opts* 
         const int64_t panels_total = (slots + BM - 1) / BM;
         const int64_t n_pad[2] = {d->g[0].n_pad, d->g[1].n_pad};
         const int64_t n_glob[2] = {d->g[0].shard.n_global, d->g[1].shard.n_global};
+        // clustered: the unit matrices (padded like row matrices) and the lengths of an explicit stream, which draws units
+        const int mats = clustered ? unit_mats(d) : 0;
+        int64_t u_pad_all = 0;
+        for (int m = 0; m < mats; ++m) u_pad_all += pad_rows(d->cl_units[m]);
+        const int64_t idx_len = clustered ? d->cl_units[0] + (mats == 2 ? d->cl_units[1] : 0) : n_glob[0] + n_glob[1];
         int ranks_with_rows[2];
         for (int g = 0; g < 2; ++g)
             ranks_with_rows[g] = (d->g[g].shard.segs + d->g[g].shard.leaf_span - 1) / d->g[g].shard.leaf_span;
@@ -2041,10 +2176,12 @@ static void bootstrap_body(ob_ctx* ctx, const ob_design* d, const ob_boot_opts* 
                                      (d->g[1].shard.leaf_hi - d->g[1].shard.leaf_lo);
         // workspace of one panel: multiplicities (+ index stream), reduced Gram (+ the mode-N exchange), partial tiles, column
         // sums; a run that only solves needs the reduced Gram alone
+        // (clustered: + the unit matrices and the per-slot row counts)
         auto per_panel_bytes = [&](int cb) {
-            if (solve_only) return 2.0 * BM * Pld * 8.0;
-            return (double)(n_pad[0] + n_pad[1]) * BM * cb + (rr.index_mode ? (double)(n_glob[0] + n_glob[1]) * BM * 4.0 : 0.0) +
-                   2.0 * BM * Pld * 8.0 * (comm ? world + 2 : 1) + (double)local_leaves * ntiles * (BM * BN * 8.0) + 2.0 * BM * 8.0;
+            const double cl = clustered ? (solve_only ? 0.0 : (double)u_pad_all * BM * cb) + 2.0 * BM * 8.0 : 0.0;
+            if (solve_only) return 2.0 * BM * Pld * 8.0 + cl;
+            return (double)(n_pad[0] + n_pad[1]) * BM * cb + (rr.index_mode ? (double)idx_len * BM * 4.0 : 0.0) +
+                   2.0 * BM * Pld * 8.0 * (comm ? world + 2 : 1) + (double)local_leaves * ntiles * (BM * BN * 8.0) + 2.0 * BM * 8.0 + cl;
         };
         double budget = (double)o->max_workspace_bytes - (double)cache_new_bytes;
         if (o->max_workspace_bytes <= 0) {
@@ -2074,7 +2211,8 @@ static void bootstrap_body(ob_ctx* ctx, const ob_design* d, const ob_boot_opts* 
             // every rank must cut the same batches: the collectives run once per batch
             if (comm) ppb = allreduce_scalar(comm, (long long)ppb, CommOp::MIN, st);
             tr.mark("setup", st, true);
-            DevBuf d_C[2], d_idx[2], d_colsum, d_gram, d_gram_local, d_gathered;
+            DevBuf d_C[2], d_idx[2], d_colsum, d_gram, d_gram_local, d_gathered, d_rows;
+            ClusterWork cw;
             const size_t gram_elems = 2 * (size_t)ppb * BM * Pld;      // [2][slots_pad][Pld]
             bool saturated = false;
             GramPlan plan; int64_t plan_panels = -1;
@@ -2083,7 +2221,9 @@ static void bootstrap_body(ob_ctx* ctx, const ob_design* d, const ob_boot_opts* 
                 if (!solve_only) {
                     d_colsum.alloc(sizeof(long long) * 2 * (size_t)ppb * BM);
                     for (int g = 0; g < 2; ++g) d_C[g].alloc((size_t)ppb * n_pad[g] * BM * count_bytes);
+                    for (int m = 0; m < mats; ++m) cw.U[m].alloc((size_t)ppb * pad_rows(d->cl_units[m]) * BM * count_bytes);
                 }
+                if (clustered) { d_rows.alloc(sizeof(long long) * 2 * (size_t)ppb * BM); cw.rows = d_rows.as<long long>(); }
                 d_gram.alloc(sizeof(double) * gram_elems);
                 if (cache) {
                     const std::vector<int32_t> cmap = gram_cache_map(K, T);
@@ -2115,7 +2255,7 @@ static void bootstrap_body(ob_ctx* ctx, const ob_design* d, const ob_boot_opts* 
                 Timer t_counts(st, &res->ms_counts);
                 if (!solve_only)
                     res->gpu_launches += generate_counts(d, o, b, count_bytes, ppb, d_C, d_idx, d_colsum, d_lut, d_flags.as<int>(), comm,
-                                                         &res->ms_comm, st);
+                                                         &res->ms_comm, st, clustered ? &cw : nullptr);
                 t_counts.stop();
                 tr.mark("counts", st, true);
 
@@ -2207,6 +2347,13 @@ static void bootstrap_body(ob_ctx* ctx, const ob_design* d, const ob_boot_opts* 
                     Timer t_cc(st, &res->ms_gram);
                     GramCacheCopy cc{d_gram.as<double>(), pn * BM, Pld, b.slot_lo, bslots, cache->xx, cache->yy, slots,
                                      d_cmap.as<int32_t>(), nx, ny, 0, nx + ny};
+                    // clustered: the per-slot row counts travel with the cells (a SOLVE_ONLY run draws no multiplicities)
+                    for (int g = 0; clustered && g < 2 && (mode == OB_CACHE_FILLED || solve_only); ++g) {
+                        long long* batch_rows = d_rows.as<long long>() + (size_t)g * pn * BM;
+                        long long* kept = cache->rows + (size_t)g * slots + b.slot_lo;
+                        OB_CUDA(cudaMemcpyAsync(solve_only ? batch_rows : kept, solve_only ? kept : batch_rows, sizeof(long long) * (size_t)bslots,
+                                                cudaMemcpyDeviceToDevice, st));
+                    }
                     if (mode == OB_CACHE_FILLED) gram_cache_extract_launch(cc, st);
                     else if (solve_only) gram_cache_assemble_launch(cc, st);
                     else {
@@ -2227,6 +2374,7 @@ static void bootstrap_body(ob_ctx* ctx, const ob_design* d, const ob_boot_opts* 
                 sa.d_norm_idx = d_nidx.as<int>(); sa.d_norm_has_base = d_nhb.as<int>();
                 sa.n_base = n_base; sa.S = S; sa.weighted = d->weighted ? 1 : 0;
                 sa.na = (double)n_glob[0]; sa.nb = (double)n_glob[1];
+                sa.rows = clustered ? d_rows.as<long long>() : nullptr;     // [2][pn * BM]
                 sa.stats = d_stats.as<double>() + (size_t)b.slot_lo * SE;
                 sa.status = d_status.as<int>() + b.slot_lo;
                 sa.beta_a = want_beta ? d_ba.as<double>() + (size_t)b.slot_lo * KE : nullptr;
@@ -2380,7 +2528,7 @@ void ob_gram_cache_destroy(ob_gram_cache* c) {
 ob_status ob_gram_cache_last_use(const ob_gram_cache* c, int32_t* use, int64_t* bytes) {
     if (!c) return OB_ERR_INVALID_ARG;
     if (use) *use = c->last_use;
-    if (bytes) *bytes = (int64_t)(c->xx_bytes + c->yy_bytes);
+    if (bytes) *bytes = (int64_t)(c->xx_bytes + c->yy_bytes + c->rows_bytes);
     return OB_OK;
 }
 
@@ -2473,9 +2621,23 @@ ob_status ob_debug_counts(ob_ctx* ctx, const ob_design* d, uint64_t seed, int64_
         ca.first_slot = 1; ca.rep0 = rep - 1; ca.group = group; ca.seed = seed;
         ca.n_global = G.shard.n_global; ca.row_begin = G.shard.row_begin;
         if (d->world > 1) fail(OB_ERR_UNSUPPORTED, "ob_debug_counts on a row-sharded design");
+        DevBuf d_U, d_rows;
+        const int m = d->cl_strata == OB_CLUSTER_JOINT ? 0 : group;
+        if (d->cl_strata != OB_CLUSTER_NONE) {      // the unit counts of the replicate, expanded to the group's rows below
+            const int64_t M = d->cl_units[m];
+            d_U.alloc((size_t)pad_rows(M) * BM * 2);
+            d_rows.alloc(sizeof(long long) * 2 * BM);
+            ca.C = d_U.p; ca.n = ca.n_global = M; ca.n_pad = pad_rows(M); ca.row_begin = 0;
+            ca.group = d->cl_strata == OB_CLUSTER_JOINT ? 2 : group;
+        }
         OB_CUDA(cudaMemsetAsync(d_colsum.p, 0, d_colsum.bytes, st));
         counts_philox_body_launch(ca, d_colsum.as<long long>(), d_lut.as<unsigned char>(), st);
         counts_philox_fixup_launch(ca, d_colsum.as<long long>(), d_flags.as<int>(), st);
+        if (d->cl_strata != OB_CLUSTER_NONE) {
+            OB_CUDA(cudaMemsetAsync(d_rows.p, 0, d_rows.bytes, st));
+            ExpandArgs ea{d_C.p, d_U.p, G.uid, 2, G.n, G.n_pad, ca.n_pad, 1, 2, d_rows.as<long long>()};
+            counts_expand_launch(ea, st);
+        }
         // slot 1 column of the single panel
         OB_CUDA(cudaMemcpy2DAsync(counts_out, sizeof(uint16_t), d_C.as<uint16_t>() + 1, sizeof(uint16_t) * BM,
                                   sizeof(uint16_t), (size_t)G.n, cudaMemcpyDeviceToHost, st));

@@ -285,6 +285,7 @@ OaxacaBuilder::Prepared OaxacaBuilder::prepare() const {
     if (has_weights_) cols.push_back(weights_col_);
     if (has_selection_) cols.push_back(selection_outcome_);
     cols.insert(cols.end(), selection_predictors_.begin(), selection_predictors_.end());
+    if (cluster_strata_ != OB_CLUSTER_NONE) cols.push_back(cluster_col_);
     std::vector<const Column*> used;
     for (const auto& c : cols) {
         const Column* col = dataframe_.find(c);
@@ -389,6 +390,7 @@ ob_design* OaxacaBuilder::ingest_on_device(ob_ctx* ctx, Prepared& p, bool with_w
     if (has_weights_) cols.push_back(weights_col_);
     if (has_selection_) cols.push_back(selection_outcome_);
     cols.insert(cols.end(), selection_predictors_.begin(), selection_predictors_.end());
+    if (cluster_strata_ != OB_CLUSTER_NONE) cols.push_back(cluster_col_);
     for (const auto& c : cols)
         if (!dataframe_.find(c)) throw OaxacaError(OB_ERR_COLUMN_NOT_FOUND, OaxacaError::display(OB_ERR_COLUMN_NOT_FOUND, c));
     const int64_t n = (int64_t)dataframe_.height();
@@ -430,6 +432,7 @@ ob_design* OaxacaBuilder::ingest_on_device(ob_ctx* ctx, Prepared& p, bool with_w
     }
     if (has_selection_) filter_only.push_back(dataframe_.find(selection_outcome_));
     for (const auto& sp : selection_predictors_) filter_only.push_back(dataframe_.find(sp));
+    if (cluster_strata_ != OB_CLUSTER_NONE) filter_only.push_back(dataframe_.find(cluster_col_));
     if (sweep)           // the other outcomes of the sweep: one cleaned frame for all of them
         for (size_t k = 1; k < sweep->size(); ++k) { const Column* c = dataframe_.find((*sweep)[k]); require_f64(c); filter_only.push_back(c); }
     std::vector<uint8_t> merged_valid;
@@ -538,6 +541,37 @@ std::vector<OaxacaResults> OaxacaBuilder::run_impl(bool rif, double tau, const s
         check(g.ctx, ob_design_attach_selection(g.ctx, g.des, &sv, (int64_t)dataframe_.height()));
         K1 = 1 + (int)preds.size();
     }
+    if (cluster_strata_ != OB_CLUSTER_NONE) {
+        // cluster codes in the sorted order of the labels, one per frame row (the design's frame-row map picks the kept
+        // rows; null rows were dropped by the filter and get any code)
+        const Column* c = dataframe_.find(cluster_col_);
+        const size_t n = dataframe_.height();
+        std::vector<int32_t> codes(n, 0);
+        size_t levels = 0;
+        if (c->is_str) {
+            std::set<std::string> uniq;
+            for (size_t i = 0; i < n; ++i) if (c->is_valid(i)) uniq.insert(c->str[i]);
+            const std::vector<std::string> sorted(uniq.begin(), uniq.end());
+            for (size_t i = 0; i < n; ++i)
+                if (c->is_valid(i)) codes[i] = (int32_t)(std::lower_bound(sorted.begin(), sorted.end(), c->str[i]) - sorted.begin());
+            levels = sorted.size();
+        } else {
+            std::vector<double> sorted;
+            for (size_t i = 0; i < n; ++i) if (c->is_valid(i) && c->f64[i] == c->f64[i]) sorted.push_back(c->f64[i]);
+            std::sort(sorted.begin(), sorted.end());
+            sorted.erase(std::unique(sorted.begin(), sorted.end()), sorted.end());
+            for (size_t i = 0; i < n; ++i) {
+                if (!c->is_valid(i)) continue;
+                const double v = c->f64[i];      // a NaN label is a cluster of its own, after every number
+                codes[i] = v == v ? (int32_t)(std::lower_bound(sorted.begin(), sorted.end(), v) - sorted.begin()) : (int32_t)sorted.size();
+            }
+            levels = sorted.size() + 1;
+        }
+        if (levels >= (size_t)INT32_MAX) throw OaxacaError(OB_ERR_UNSUPPORTED, "more than 2^31 - 1 cluster labels");
+        check(g.ctx, ob_design_attach_clusters(g.ctx, g.des, codes.data(), (int64_t)n, (int32_t)std::max<size_t>(levels, 1), cluster_strata_));
+    }
+    int32_t cl_strata = OB_CLUSTER_NONE; int64_t cl_ua = 0, cl_ub = 0;
+    ob_design_clusters(g.des, &cl_strata, &cl_ua, &cl_ub);
 
     int64_t na = 0, nb = 0; int32_t K = 0, nc = 0;
     ob_design_shape(g.des, &na, &nb, &K, &nc);
@@ -602,6 +636,7 @@ std::vector<OaxacaResults> OaxacaBuilder::run_impl(bool rif, double tau, const s
         R.n_a = (size_t)na; R.n_b = (size_t)nb;
         R.predictor_names = has_selection_ ? rows : p.names;
         R.ms_total = r.ms_total; R.ms_gram = r.ms_gram;
+        R.cluster_strata = cl_strata; R.cluster_units_a = cl_ua; R.cluster_units_b = cl_ub;
         all.push_back(std::move(R));
     }
     return all;
@@ -685,6 +720,10 @@ void OaxacaResults::summary(std::ostream& os) const {   // display.rs:9-79
     os << "========================================\n";
     os << "Group A (Advantaged): " << n_a << " observations\n";
     os << "Group B (Reference):  " << n_b << " observations\n";
+    if (cluster_strata == OB_CLUSTER_BY_GROUP)
+        os << "Cluster bootstrap (by group): " << cluster_units_a << " units in A, " << cluster_units_b << " in B\n";
+    else if (cluster_strata == OB_CLUSTER_JOINT)
+        os << "Cluster bootstrap (joint): " << cluster_units_a << " units\n";
     os << "Total Gap: " << fmt(total_gap, 4) << "\n\n";
     os << "Two-Fold Decomposition\n";
     table(os, "Component", "Estimate", two_fold.aggregate);
@@ -733,6 +772,9 @@ std::string OaxacaResults::to_json(bool with_residuals, bool with_extra) const {
     os << "},\"three_fold\":{\"aggregate\":"; jcomps(os, three_fold.aggregate);
     os << ",\"detailed\":"; jcomps(os, three_fold.detailed);
     os << "},\"n_a\":" << n_a << ",\"n_b\":" << n_b;
+    if (cluster_strata != OB_CLUSTER_NONE)
+        os << ",\"clusters\":{\"strata\":\"" << (cluster_strata == OB_CLUSTER_JOINT ? "joint" : "group") << "\",\"units_a\":"
+           << cluster_units_a << ",\"units_b\":" << cluster_units_b << '}';
     if (with_residuals) { os << ",\"residuals\":"; jvec(os, residuals); }
     if (with_extra) {   // #[serde(skip)] fields + replicate bookkeeping, for the Python mirror and tests
         os << ",\"xa_mean\":"; jvec(os, xa_mean); os << ",\"xb_mean\":"; jvec(os, xb_mean);

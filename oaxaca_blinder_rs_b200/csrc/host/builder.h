@@ -67,6 +67,9 @@ struct OaxacaResults {     // types.rs:24-47
     int64_t bootstrap_reps = 0, successful_bootstraps = 0;
     std::vector<std::string> predictor_names;
     double ms_total = 0, ms_gram = 0;
+    // cluster bootstrap (OaxacaBuilder::cluster): ob_cluster_strata and the units resampled per replicate (JOINT: a == b)
+    int cluster_strata = OB_CLUSTER_NONE;
+    int64_t cluster_units_a = 0, cluster_units_b = 0;
 
     void summary(std::ostream& os) const;                          // display.rs:9-79
     std::string to_json(bool with_residuals, bool with_extra) const;   // display.rs to_json (serde layout) [+ extras]
@@ -106,6 +109,11 @@ public:
     OaxacaBuilder& seed(uint64_t s) { seed_ = s; return *this; }
     OaxacaBuilder& device(int d) { device_ = d; return *this; }
     OaxacaBuilder& index_stream(const uint32_t* idx_a, const uint32_t* idx_b) { idx_a_ = idx_a; idx_b_ = idx_b; return *this; }
+    // cluster bootstrap: resample whole clusters of `column` (string or numeric labels; codes follow their sorted order)
+    // with ob_cluster_strata `strata` (OB_CLUSTER_NONE: back to rows).  The column joins the null filter.
+    OaxacaBuilder& cluster(const std::string& column, int strata = OB_CLUSTER_BY_GROUP) {
+        cluster_col_ = strata == OB_CLUSTER_NONE ? std::string() : column; cluster_strata_ = strata; return *this;
+    }
 
     OaxacaResults run() const;                              // builder.rs:787-951
     // run() once per listed outcome column on one ingest: rows are cleaned over all of them, the first run fills a Gram
@@ -130,6 +138,8 @@ private:
     ReferenceCoefficients reference_coeffs_ = ReferenceCoefficients::GroupA; // builder.rs:123 (the code, not the doc comment)
     std::string weights_col_, selection_outcome_;
     bool has_weights_ = false, has_selection_ = false;
+    std::string cluster_col_;
+    int cluster_strata_ = OB_CLUSTER_NONE;
     uint64_t seed_ = 0x0B5EEDull;
     int device_ = 0;
     const uint32_t* idx_a_ = nullptr;

@@ -54,6 +54,8 @@ static void usage() {
         "      --normalize <A,B,..>           Categorical variables to Yun-normalise (builder.normalize)\n"
         "      --rif-quantile <TAU>           RIF-regression decomposition at quantile TAU (decompose_quantile)\n"
         "      --seed <N>                     Resampling seed\n"
+        "      --cluster <COLUMN>             Cluster bootstrap: resample whole clusters of COLUMN instead of rows\n"
+        "      --cluster-strata <MODE>        group (default: each group resamples its own clusters) | joint (one stratum)\n"
         "      --output-json <PATH>           Export results as JSON\n"
         "      --output-markdown <PATH>       Export results as Markdown\n";
 }
@@ -74,7 +76,17 @@ int main(int argc, char** argv) {
     unsigned long long reps = 0, seed = 0, sims = 200;                                    // main.rs:86-87
     double tau = 0.0;
     std::vector<double> quantiles = {0.1, 0.25, 0.5, 0.75, 0.9};                          // main.rs:236-239
+    int cluster_strata = OB_CLUSTER_BY_GROUP;
     try {
+        if (a.count("cluster-strata")) {
+            const std::string& cs = a["cluster-strata"];
+            if (cs == "group") cluster_strata = OB_CLUSTER_BY_GROUP;
+            else if (cs == "joint") cluster_strata = OB_CLUSTER_JOINT;
+            else throw ArgError{"invalid value '" + cs + "' for '--cluster-strata <MODE>'\n  [possible values: group, joint]"};
+            if (!a.count("cluster")) throw ArgError{"'--cluster-strata <MODE>' requires '--cluster <COLUMN>'"};
+        }
+        if (a.count("cluster") && a["analysis-type"] == "quantile")
+            throw ArgError{"'--cluster <COLUMN>' applies to the mean and RIF decompositions, not to '--analysis-type quantile'"};
         const std::string& rc = a["ref-coeffs"];
         if (rc == "group-a") ref_kind = ob::ReferenceCoefficients::GroupA;
         else if (rc == "group-b") ref_kind = ob::ReferenceCoefficients::GroupB;
@@ -126,6 +138,7 @@ int main(int argc, char** argv) {
         if (a.count("weights")) b.weights(a["weights"]);
         if (a.count("normalize")) b.normalize(split_commas(a["normalize"]));
         if (a.count("seed")) b.seed(seed);
+        if (a.count("cluster")) b.cluster(a["cluster"], cluster_strata);
         if (a.count("selection-outcome")) b.heckman_selection(a["selection-outcome"], split_commas(a["selection-predictors"]));
         const ob::OaxacaResults r = a.count("rif-quantile") ? b.decompose_quantile(tau) : b.run();
         r.summary(std::cout);

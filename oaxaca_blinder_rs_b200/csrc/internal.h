@@ -95,6 +95,8 @@ struct GroupData {               // one group's packed design in HBM (the rows t
     // Heckman selection equation (ob_design_attach_selection): Z [n][K1] row-major with the intercept first, sel [n] =
     // (selection outcome == 1), Xm [n_pad][ldx] = the design with unselected rows zeroed (operand of the outcome Gram)
     double* hk_Z = nullptr; uint8_t* hk_sel = nullptr; double* hk_Xm = nullptr;
+    // clusters (ob_design_attach_clusters): [n] resampling unit of each packed row, or nullptr (rows are resampled)
+    uint32_t* uid = nullptr;
     const double* gram_operand() const { return Xs ? Xs : X; }
 };
 
@@ -120,6 +122,22 @@ void counts_from_indices(const CountsArgs& a, const uint32_t* d_idx, int* d_over
 size_t counts_lut_bytes();
 void counts_philox_body_launch(const CountsArgs& a, long long* d_colsum, unsigned char* d_lut, cudaStream_t st);
 void counts_philox_fixup_launch(const CountsArgs& a, const long long* d_colsum, int* d_flags, cudaStream_t st);
+
+// ---- cluster.cu ----
+// attach: uid[row] = codes_frame[src[row]], present[code] = 1 (d_flags[0] |= 1 on a code outside [0, n_codes)); then
+// unit[code] = exclusive scan of present (*d_units = the stratum's unit count); then uid[row] = unit[uid[row]]
+void cluster_gather_launch(const int32_t* d_codes_frame, const uint32_t* src, int64_t n, int32_t n_codes, uint32_t* uid,
+                           uint8_t* present, int* d_flags, cudaStream_t st);
+void cluster_scan_launch(const uint8_t* present, int32_t n_codes, uint32_t* unit, long long* d_units, cudaStream_t st);
+void cluster_remap_launch(uint32_t* uid, int64_t n, const uint32_t* unit, cudaStream_t st);
+// C [panels][n_pad][BM] = U [panels][u_pad][BM] gathered through uid (rows [n, n_pad) zero); rows[slot] += the slot's row
+// count (zeroed by the caller; slots < `slots` only)
+struct ExpandArgs {
+    void* C; const void* U; const uint32_t* uid; int count_bytes;
+    int64_t n, n_pad, u_pad; int panels; int64_t slots;
+    long long* rows;
+};
+void counts_expand_launch(const ExpandArgs& a, cudaStream_t st);
 
 // ---- gram.cu ----
 constexpr int BQ = 32;            // column quantum of the Gram CTA tile: one 8-column DMMA sub-tile for each of the SM's four
@@ -217,6 +235,7 @@ struct SolveArgs {
     int n_base; int S;
     int weighted;
     double na, nb;           // group row counts (n_obs)
+    const long long* rows = nullptr;   // clustered designs: [2][slots_pad] row counts per slot (replace na / nb), else null
     // outputs
     double* stats;           // [slots][S]
     int* status;             // [slots]

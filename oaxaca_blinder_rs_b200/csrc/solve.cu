@@ -26,6 +26,7 @@ struct SolveParams {
     int n_norm; const int* norm_m; const int* norm_off; const int* norm_idx; const int* norm_has_base;
     int n_base, S, weighted;
     double na, nb;
+    const long long* rows;   // [2][slots_pad] per-slot group row counts (clustered designs), null: na / nb
     double* stats; int* status; double* beta_a; double* beta_b; double* point_extra;
     double* gscratch;        // per-slot matrix buffer in global memory when it does not fit shared memory, else null
 };
@@ -145,7 +146,14 @@ __global__ void __launch_bounds__(SOLVE_THREADS) solve_kernel(const SolveParams 
     }
     int status = OB_OK;
     // ols.rs:96-105: n_obs (row count, not sum of weights) must exceed k; group A is fitted first
-    if (p.na <= (double)K || p.nb <= (double)K) status = OB_ERR_INSUFFICIENT_DATA;
+    double na = p.na, nb = p.nb;
+    if (p.rows) {
+        // a clustered replicate: its own group sizes, checked in the reference's order -- an empty group first
+        // (builder.rs:431-435), then group A's fit, group B's n-guard at its own fit (sys == 1 below)
+        na = (double)p.rows[slot]; nb = (double)p.rows[p.slots_pad + slot];
+        if (na == 0.0 || nb == 0.0) status = OB_ERR_INVALID_GROUP;
+        else if (na <= (double)K) status = OB_ERR_INSUFFICIENT_DATA;
+    } else if (na <= (double)K || nb <= (double)K) status = OB_ERR_INSUFFICIENT_DATA;
     const int ind = 1 + p.n_cont;       // builder.rs:548-566: position of the group indicator in the pooled design
 
     for (int sys = 0; sys < (pooled ? 3 : 2); ++sys) {
@@ -153,6 +161,7 @@ __global__ void __launch_bounds__(SOLVE_THREADS) solve_kernel(const SolveParams 
         double* B = sys == 0 ? BA : (sys == 1 ? BB : BP);
         const double* g = sys == 1 ? gB : gA;
         __syncthreads();
+        if (sys == 1 && p.rows && nb <= (double)K) status = OB_ERR_INSUFFICIENT_DATA;
         if (status != OB_OK) break;
         if (sys < 2) {
             // unpack X'WX of the group from the packed columns
@@ -168,7 +177,7 @@ __global__ void __launch_bounds__(SOLVE_THREADS) solve_kernel(const SolveParams 
                 B[t * Kp + j] = g[gidx(K, T, j, j) + (K - j) + t];
             }
         } else {
-            if (p.na + p.nb <= (double)Kp) { status = OB_ERR_INSUFFICIENT_DATA; break; }
+            if (na + nb <= (double)Kp) { status = OB_ERR_INSUFFICIENT_DATA; break; }
             // rows of A and B stacked, indicator (1 on A rows) at column ind
             for (int e = tid; e < Kp * Kp; e += blockDim.x) {
                 const int i = e / Kp, j = e - i * Kp;
@@ -220,8 +229,8 @@ __global__ void __launch_bounds__(SOLVE_THREADS) solve_kernel(const SolveParams 
                 break;
             }
             default: {  // Weighted | Cotton: builder.rs:591-620
-                const double n_a = p.weighted ? sums[0] : p.na;
-                const double n_b = p.weighted ? sums[2] : p.nb;
+                const double n_a = p.weighted ? sums[0] : na;
+                const double n_b = p.weighted ? sums[2] : nb;
                 const double total = n_a + n_b;
                 if (total == 0.0) { st_t = OB_ERR_INVALID_GROUP; break; }
                 const double wA = n_a / total, wB = 1.0 - wA;
@@ -300,7 +309,7 @@ void solve_launch(const SolveArgs& a, cudaStream_t st) {
     p.K = a.K; p.n_cont = a.n_cont; p.ref_kind = a.ref_kind; p.T = a.T;
     p.n_norm = a.n_norm; p.norm_m = a.d_norm_m; p.norm_off = a.d_norm_off; p.norm_idx = a.d_norm_idx;
     p.norm_has_base = a.d_norm_has_base; p.n_base = a.n_base; p.S = a.S; p.weighted = a.weighted;
-    p.na = a.na; p.nb = a.nb;
+    p.na = a.na; p.nb = a.nb; p.rows = a.rows;
     p.stats = a.stats; p.status = a.status; p.beta_a = a.beta_a; p.beta_b = a.beta_b; p.point_extra = a.point_extra;
     const bool pooled = a.ref_kind == OB_REF_POOLED;
     const bool global = solve_scratch_bytes(a.K, pooled, a.n_norm, a.T, 1) != 0;
