@@ -244,7 +244,9 @@ typedef struct ob_boot_opts {
     int64_t rep_begin;
     int64_t rep_end;
     int32_t skip_reduce;             /* 1: stop after per-replicate statistics (multi-GPU: gather first, then ob_reduce_stats) */
-    int32_t count_bits;              /* 0 auto, 8 or 16: width of the multiplicity matrix */
+    int32_t count_bits;              /* 0 auto, 8 or 16: width of the multiplicity matrix.  16 needs K + outcomes <= 268
+                                        (the Gram kernel's shared memory; wider designs are refused, OB_ERR_UNSUPPORTED);
+                                        auto starts at 8 and widens to 16 when a count saturates, where 16 fits */
     int64_t max_workspace_bytes;     /* 0 = default (60% of free HBM); bounds the multiplicity-matrix batch */
     /* Mode R inside the library (replicate sharding; SURVEY 8e): 1 = the context carries a communicator of `world`
      * ranks (ob_comm_init_*), every rank holds the WHOLE design and makes this same call; the library computes the
@@ -475,6 +477,15 @@ ob_status ob_debug_counts(ob_ctx* ctx, const ob_design* d, uint64_t seed, int64_
  * index was >= n_global. */
 ob_status ob_debug_counts_from_indices(ob_ctx* ctx, const ob_design* d, int32_t group, const uint32_t* idx, int64_t reps,
                                        int32_t count_bits, uint16_t* counts_out, int32_t* flags_out);
+
+/* What the last successful ob_bootstrap_run_cached left in cache c (read-only; for the cell-by-cell tests of the Gram
+ * contraction): shape_out[5] = {slots, K, T, count_bytes of the fill (1 or 2), 1 if row counts are held (clustered
+ * designs) else 0}; xx_out [2][slots][K(K+1)/2] = the X'WX upper triangles, row-major; yy_out [2][slots][K T + 1] = the
+ * cells (j, y_t), j-major, then (y_0, y_0); rows_out [2][slots] = each slot's group row counts (clustered designs only,
+ * else untouched).  Slot 0 is the point estimate, slot s >= 1 replicate rep_begin + s - 1 of the run (under
+ * shard_replicates: of this rank's shard).  Any output may be NULL.  An empty cache is OB_ERR_INVALID_ARG. */
+ob_status ob_debug_gram_cache_read(ob_ctx* ctx, const ob_gram_cache* c, int64_t* shape_out, double* xx_out, double* yy_out,
+                                   int64_t* rows_out);
 
 #ifdef __cplusplus
 }

@@ -31,7 +31,8 @@ SYMBOLS = ["ob_abi_version", "ob_device_count", "ob_ctx_create", "ob_ctx_destroy
            "ob_design_redistribute_rows", "ob_design_row_shard", "ob_design_apply_rif_multi", "ob_design_num_outcomes",
            "ob_design_pack_row_shard_async", "ob_design_attach_selection", "ob_design_selection_cols", "ob_num_stats_heckman",
            "ob_mm_run", "ob_debug_gram_columns", "ob_gram_cache_create", "ob_gram_cache_destroy", "ob_gram_cache_last_use",
-           "ob_bootstrap_run_cached", "ob_debug_gram_outcome_columns", "ob_design_attach_clusters", "ob_design_clusters"]
+           "ob_bootstrap_run_cached", "ob_debug_gram_outcome_columns", "ob_design_attach_clusters", "ob_design_clusters",
+           "ob_debug_gram_cache_read"]
 
 
 class FrameView(C.Structure):
@@ -134,6 +135,7 @@ def lib() -> C.CDLL:
         L.ob_gram_cache_destroy.restype = None
         L.ob_gram_cache_last_use.argtypes = [C.c_void_p, _IP, C.POINTER(C.c_int64)]
         L.ob_bootstrap_run_cached.argtypes = [C.c_void_p, C.c_void_p, C.POINTER(BootOpts), C.c_void_p, C.POINTER(Result)]
+        L.ob_debug_gram_cache_read.argtypes = [C.c_void_p, C.c_void_p, C.POINTER(C.c_int64), _DP, _DP, C.POINTER(C.c_int64)]
         L.ob_debug_gram_outcome_columns.argtypes = [C.c_int32, C.c_int32, C.POINTER(C.c_uint16), _IP, C.c_int64, _IP]
         L.ob_debug_gram_outcome_columns.restype = C.c_int64
         L.ob_reduce_stats.argtypes = [C.c_void_p, _DP, _IP, C.c_int64, C.c_int32, _DP, C.POINTER(C.c_int64),

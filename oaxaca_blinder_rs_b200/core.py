@@ -148,6 +148,21 @@ class GramCache:
         """Device memory the cache holds."""
         return self._query()[1]
 
+    def debug_cells(self) -> dict:
+        """ob_debug_gram_cache_read: the reduced Gram cells the last cached bootstrap left here.  xx [2, slots, K(K+1)/2]
+        (X'WX upper triangle, row-major), yy [2, slots, K T + 1] ((j, y_t) j-major, then (y_0, y_0)), rows [2, slots] (group
+        row counts of a clustered design, else None), slots, K, T, count_bytes.  Slot 0 is the point estimate."""
+        shape = np.zeros(5, dtype=np.int64)
+        I64P = C.POINTER(C.c_int64)
+        self.ctx.check(N.lib().ob_debug_gram_cache_read(self.ctx._h, self._h, shape.ctypes.data_as(I64P), None, None, None))
+        slots, K, T, cb, has_rows = (int(v) for v in shape)
+        xx = np.empty((2, slots, K * (K + 1) // 2))
+        yy = np.empty((2, slots, K * T + 1))
+        rows = np.empty((2, slots), dtype=np.int64) if has_rows else None
+        self.ctx.check(N.lib().ob_debug_gram_cache_read(self.ctx._h, self._h, None, _dp(xx), _dp(yy),
+                                                        None if rows is None else rows.ctypes.data_as(I64P)))
+        return dict(xx=xx, yy=yy, rows=rows, slots=slots, K=K, T=T, count_bytes=cb)
+
     def close(self):
         if self._h:
             N.lib().ob_gram_cache_destroy(self._h)

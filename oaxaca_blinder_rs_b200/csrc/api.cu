@@ -395,6 +395,7 @@ RepRange replicate_range(const ob_ctx* ctx, const ob_design* d, const Opts* o) {
         if (o->idx_b) fail(OB_ERR_INVALID_ARG, "a JOINT cluster design takes one unit stream: idx_a [reps x M] and idx_b = NULL");
     } else if (r.index_mode && r.nrep > 0 && (!o->idx_a || !o->idx_b)) fail(OB_ERR_INVALID_ARG, "index stream needs both idx_a and idx_b");
     if (o->count_bits != 0 && o->count_bits != 8 && o->count_bits != 16) fail(OB_ERR_INVALID_ARG, "count_bits must be 0, 8 or 16");
+    if (o->count_bits == 16 && !gram_fits(d->ldx, 2)) fail(OB_ERR_UNSUPPORTED, "16-bit multiplicities need K + outcomes <= 268");
     r.count_bytes = o->count_bits == 16 ? 2 : 1;
     return r;
 }
@@ -495,11 +496,13 @@ int generate_counts(const ob_design* d, const Opts* o, const Batch& b, int count
 }
 
 // A batch's deferred error flags (multiplicity kernels): a bad index or a Poisson overshoot fails the call.  A saturated
-// count returns true when the run may widen to 16-bit counts and redo, and fails when it may not.
-bool check_batch_flags(const int flags[4], int count_bytes, int count_bits) {
+// count returns true when the run may widen to 16-bit counts and redo, and fails when it may not: already 16-bit, 8 bits
+// asked for, or a design (row stride ldx) too wide for the Gram kernel at 16 bits.
+bool check_batch_flags(const int flags[4], int count_bytes, int count_bits, int ldx) {
     if (flags[2]) fail(OB_ERR_INVALID_ARG, "resample index out of range");
     if (flags[0]) fail(OB_ERR_CUDA, "Poisson body overshot n (probability < 1e-15 per replicate); rerun with another seed");
-    if (flags[1] && (count_bytes == 2 || count_bits == 8)) fail(OB_ERR_UNSUPPORTED, "row multiplicity overflows the count width");
+    if (flags[1] && (count_bytes == 2 || count_bits == 8 || !gram_fits(ldx, 2)))
+        fail(OB_ERR_UNSUPPORTED, "row multiplicity overflows the count width");
     return flags[1] != 0;
 }
 
@@ -1790,7 +1793,7 @@ void heckman_run(ob_ctx* ctx, const ob_design* d, const ob_boot_opts* o, ob_resu
             OB_CUDA(cudaMemcpyAsync(flags, d_flags.p, sizeof flags, cudaMemcpyDeviceToHost, st));
             OB_CUDA(cudaStreamSynchronize(st));
             t_counts.collect(); t_solve.collect(); t_gram.collect(); t_solve2.collect();
-            saturated = check_batch_flags(flags, count_bytes, o->count_bits);
+            saturated = check_batch_flags(flags, count_bytes, o->count_bits, d->ldx);
         }
         if (!saturated) break;
         count_bytes = 2;
@@ -1985,7 +1988,7 @@ void mm_run(ob_ctx* ctx, const ob_design* d, const ob_mm_opts* o, ob_mm_result* 
             }
             OB_CUDA(cudaStreamSynchronize(st));
             t_counts.collect(); t_qr.collect(); t_eff.collect();
-            saturated = check_batch_flags(flags, count_bytes, o->count_bits);
+            saturated = check_batch_flags(flags, count_bytes, o->count_bits, d->ldx);
             if (saturated) break;
             if (p0 == 0 && (res->point_betas_a || res->point_betas_b))
                 for (int s_ = 0; s_ < sims; ++s_) {
@@ -2393,7 +2396,7 @@ static void bootstrap_body(ob_ctx* ctx, const ob_design* d, const ob_boot_opts* 
                 tr.mark("solve + flags", st, false);
                 t_counts.collect(); t_gram.collect(); t_solve.collect();
                 { float ms = 0; cudaEventElapsedTime(&ms, ev.a, ev.b); res->ms_gram_kernel += ms; }
-                saturated = check_batch_flags(flags, count_bytes, o->count_bits);
+                saturated = check_batch_flags(flags, count_bytes, o->count_bits, d->ldx);
             }
             if (!saturated) break;
             count_bytes = 2;  // widen and redo
@@ -2685,6 +2688,25 @@ ob_status ob_debug_counts_from_indices(ob_ctx* ctx, const ob_design* d, int32_t 
             if (v != (i < G.n ? 1u : 0u)) fail(OB_ERR_CUDA, "point-estimate slot of the multiplicity matrix is not all ones");
         }
         if (flags_out) *flags_out = (flags[1] ? 1 : 0) | (flags[2] ? 2 : 0);   // 1 = a count saturated, 2 = index out of range
+    });
+}
+
+// The reduced Gram cells a cached run left in its cache, read back (tests: cell-by-cell checks of the contraction).
+ob_status ob_debug_gram_cache_read(ob_ctx* ctx, const ob_gram_cache* c, int64_t* shape_out, double* xx_out, double* yy_out,
+                                   int64_t* rows_out) {
+    if (!ctx || !c) return OB_ERR_INVALID_ARG;
+    return guarded(ctx, [&] {
+        if (c->owner != ctx) fail(OB_ERR_INVALID_ARG, "this Gram cache belongs to another context");
+        if (!c->xx || !c->yy || !c->xx_ok || !c->y_ok) fail(OB_ERR_INVALID_ARG, "the Gram cache is empty");
+        if (shape_out) {
+            shape_out[0] = c->slots; shape_out[1] = c->K; shape_out[2] = c->T;
+            shape_out[3] = c->count_bytes; shape_out[4] = c->rows ? 1 : 0;
+        }
+        cudaStream_t st = ctx->stream;
+        if (xx_out) OB_CUDA(cudaMemcpyAsync(xx_out, c->xx, c->xx_bytes, cudaMemcpyDeviceToHost, st));
+        if (yy_out) OB_CUDA(cudaMemcpyAsync(yy_out, c->yy, c->yy_bytes, cudaMemcpyDeviceToHost, st));
+        if (rows_out && c->rows) OB_CUDA(cudaMemcpyAsync(rows_out, c->rows, c->rows_bytes, cudaMemcpyDeviceToHost, st));
+        OB_CUDA(cudaStreamSynchronize(st));
     });
 }
 

@@ -308,6 +308,10 @@ static size_t gram_ws_smem(int ldx, int count_bytes, int ring = WS_R) {
 }
 constexpr size_t GRAM_SMEM_MAX = 227 * 1024;
 
+// The Gram CTA fits in shared memory at this row stride and count width (two ring stages when three do not fit):
+// ldx <= 284 (K + outcomes <= 280) with uint8 counts, ldx <= 268 (K + outcomes <= 268) with uint16 counts.
+bool gram_fits(int ldx, int count_bytes) { return gram_ws_smem(ldx, count_bytes, 2) <= GRAM_SMEM_MAX; }
+
 // Aligned binary summation tree over LEN consecutive leaves starting at `lo` (lo < cnt): leaves >= cnt are absent
 // and skipped.  The tree shape depends on the leaf indices only, so any aligned sub-range reduced on another GPU
 // (mode N) yields the very same intermediate sums.
@@ -537,7 +541,9 @@ void gram_launch_leaves(const GramPlan& pl, const GramArgs& a, const int seg_lo[
     if (units <= 0) return;
     const int grid = (int)std::min<int64_t>(pl.grid, units);
     const size_t ws_smem = pl.smem_bytes;
-    if (ws_smem > GRAM_SMEM_MAX) throw StatusError{OB_ERR_UNSUPPORTED, "design too wide for the Gram kernel's shared-memory ring (K + outcomes <= 280)"};
+    if (!gram_fits(pl.ldx, a.count_bytes))
+        throw StatusError{OB_ERR_UNSUPPORTED, "design too wide for the Gram kernel's shared-memory ring (K + outcomes <= 280 with "
+                                              "8-bit multiplicities, <= 268 with 16-bit)"};
     auto launch_ws = [&](auto kernel) {
         OB_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ws_smem));
         kernel<<<grid, WS_THREADS, ws_smem, st>>>(p);

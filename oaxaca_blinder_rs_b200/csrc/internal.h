@@ -202,6 +202,9 @@ inline int gram_ntiles(int K, int T) { int f, q; gram_col_tiling(num_pairs(K, T)
 inline int gram_pld(int K, int T) { return (int)((num_pairs(K, T) + BQ - 1) / BQ * BQ); }
 GramPlan gram_make_plan(int K, int T, int ldx, int panels, const GroupData g[2], int count_bytes, int num_sms,
                         const GramColumns& cols);
+// whether the Gram CTA fits in shared memory at design row stride ldx with count_bytes-wide multiplicities: always at
+// 8-bit (K + outcomes <= 280), up to ldx 268 at 16-bit.  The drivers refuse or stop widening where it does not.
+bool gram_fits(int ldx, int count_bytes);
 struct GramArgs {
     const double* X[2]; const void* C[2];     // X: the (sqrt(w)-scaled when weighted) design
     int count_bytes;

@@ -84,10 +84,11 @@ struct PackKernelParams {
     long long shift[2], n_local[2], lo_add[2], hi_base[2];
     double* EX[2]; double* Ew[2]; uint32_t* Esrc[2];
     uint32_t src_add;              // frame row of the slice's first row
+    int tile_cols;                 // design columns staged per pass (all V unless [PK_ROWS][V | 1] exceeds shared memory)
 };
 
 __global__ void __launch_bounds__(PK_THREADS) pack_scatter_kernel(const PackKernelParams p) {
-    extern __shared__ __align__(16) double tile[];      // [PK_ROWS][V | 1] (odd stride: conflict-free column writes)
+    extern __shared__ __align__(16) double tile[];      // [PK_ROWS][tile_cols | 1] (odd stride: conflict-free column writes)
     __shared__ int lrank[PK_ROWS];                      // local rank within the row's group, -1 = ignored row
     __shared__ uint8_t lgrp[PK_ROWS];
     __shared__ int srcA[PK_ROWS], srcB[PK_ROWS];
@@ -124,74 +125,86 @@ __global__ void __launch_bounds__(PK_THREADS) pack_scatter_kernel(const PackKern
         cnt[0] = wcount[0][0] + wcount[1][0] + wcount[2][0] + wcount[3][0];
         cnt[1] = wcount[0][1] + wcount[1][1] + wcount[2][1] + wcount[3][1];
     }
-    // ---- stage the block's rows: column-wise coalesced reads -> tile[row][col] ----
-    // continuous predictors (the bulk of the bytes): 4 independent loads in flight per thread
-    {
-        const int lim = p.n_cont * PK_ROWS;
-        for (int base = tid; base < lim; base += PK_THREADS * 4) {
-            double v[4];
-#pragma unroll
-            for (int u = 0; u < 4; ++u) {
-                const int e = base + u * PK_THREADS;
-                const int c = e / PK_ROWS, t = e - c * PK_ROWS;
-                v[u] = (e < lim && t < rows) ? scont[c][row0 + t] : 0.0;
-            }
-#pragma unroll
-            for (int u = 0; u < 4; ++u) {
-                const int e = base + u * PK_THREADS;
-                if (e < lim) { const int c = e / PK_ROWS, t = e - c * PK_ROWS; tile[t * ts + 1 + c] = v[u]; }
-            }
-        }
-    }
-    // intercept, outcome, dummies
-    for (int t = tid; t < PK_ROWS; t += PK_THREADS) {
-        tile[t * ts] = t < rows ? 1.0 : 0.0;                                  // __ob_intercept__ (builder.rs:330)
-        tile[t * ts + p.K] = t < rows ? p.y[row0 + t] : 0.0;
-    }
-    for (int e = tid; e < p.n_cat * PK_ROWS; e += PK_THREADS) {
-        const int q = e / PK_ROWS, t = e - q * PK_ROWS;
-        const int levels = p.cat_levels[q], start = p.dummy_start[q];
-        int code = 0;
-        if (t < rows) {
-            code = p.cat[q][row0 + t];
-            if (code < 0 || code >= levels) { atomicOr(&p.flags[1], 1); code = 0; }
-        }
-        for (int lv = 1; lv < levels; ++lv)                                   // builder.rs:402-409: level lv -> column start + lv - 1
-            tile[t * ts + start + lv - 1] = (t < rows && code == lv) ? 1.0 : 0.0;
-    }
-    __syncthreads();
     const long long baseA = p.block_base[2 * blk], baseB = p.block_base[2 * blk + 1];
-    // ---- write out: one warp per packed row, lanes over its V contiguous columns; the sqrt(w)-scaled copy
-    //      (ols.rs:68-78) is written in the same pass ----
     const int warp = tid >> 5, lane = tid & 31;
-    for (int g = 0; g < 2; ++g) {
-        double* X = g ? p.XB : p.XA;
-        double* Xs = g ? p.XsB : p.XsA;
-        double* W = g ? p.wB : p.wA;
-        uint32_t* SRC = g ? p.srcB : p.srcA;
-        const int* src = g ? srcB : srcA;
-        const long long base = g ? baseB : baseA;
-        for (int r = warp; r < cnt[g]; r += PK_THREADS / 32) {
-            const int t = src[r];
-            const double wv = p.w ? p.w[row0 + t] : 1.0;
-            if (wv < 0.0 && lane == 0) atomicOr(&p.flags[0], 1);   // ols.rs:60-66 (the chunked pack has no earlier look at w)
-            const double sw = sqrt(wv);
-            long long pos = base + r + p.shift[g];
-            const bool mine = pos >= 0 && pos < p.n_local[g];
-            double* xdst = X; double* xsdst = Xs; double* wdst = W; uint32_t* sdst = SRC;
-            if (!mine) {      // another rank's row: export buffer, no scaled copy (the receiver scales what it imports)
-                pos = pos < 0 ? pos + p.lo_add[g] : p.hi_base[g] + (pos - p.n_local[g]);
-                xdst = p.EX[g]; xsdst = nullptr; wdst = p.Ew[g]; sdst = p.Esrc[g];
+    // design columns [c0, c1) per pass: all V in one pass unless the tile would not fit in shared memory (wide designs)
+    for (int c0 = 0; c0 < V; c0 += p.tile_cols) {
+        const int c1 = min(V, c0 + p.tile_cols), ts = (c1 - c0) | 1;
+        const bool last = c1 == V;
+        if (c0 > 0) __syncthreads();          // every warp has written out the previous pass's tile
+        // ---- stage the block's rows: column-wise coalesced reads -> tile[row][col - c0] ----
+        // continuous predictors (design columns 1 .. n_cont, the bulk of the bytes): 4 independent loads in flight per thread
+        {
+            const int q0 = max(c0 - 1, 0), q1 = min(c1 - 1, p.n_cont);
+            const int lim = (q1 > q0 ? q1 - q0 : 0) * PK_ROWS;
+            for (int base = tid; base < lim; base += PK_THREADS * 4) {
+                double v[4];
+#pragma unroll
+                for (int u = 0; u < 4; ++u) {
+                    const int e = base + u * PK_THREADS;
+                    const int c = q0 + e / PK_ROWS, t = e % PK_ROWS;
+                    v[u] = (e < lim && t < rows) ? scont[c][row0 + t] : 0.0;
+                }
+#pragma unroll
+                for (int u = 0; u < 4; ++u) {
+                    const int e = base + u * PK_THREADS;
+                    if (e < lim) { const int c = q0 + e / PK_ROWS, t = e % PK_ROWS; tile[t * ts + 1 + c - c0] = v[u]; }
+                }
             }
-            double* xr = xdst + pos * p.ldx;
-            for (int c = lane; c < p.ldx; c += 32) {          // pad columns [V, ldx) are written as zeros here
-                const double v = c < V ? tile[t * ts + c] : 0.0;
-                xr[c] = v;
-                if (xsdst) xsdst[pos * p.ldx + c] = sw * v;
+        }
+        // intercept, outcome, dummies
+        for (int t = tid; t < PK_ROWS; t += PK_THREADS) {
+            if (c0 == 0) tile[t * ts] = t < rows ? 1.0 : 0.0;                   // __ob_intercept__ (builder.rs:330)
+            if (last) tile[t * ts + p.K - c0] = t < rows ? p.y[row0 + t] : 0.0;
+        }
+        for (int e = tid; e < p.n_cat * PK_ROWS; e += PK_THREADS) {
+            const int q = e / PK_ROWS, t = e - q * PK_ROWS;
+            const int levels = p.cat_levels[q], start = p.dummy_start[q];
+            // no dummy of q in this pass (a one-level categorical has none: its codes are checked in the last pass)
+            if (!(last && levels <= 1) && (start + levels - 1 <= c0 || start >= c1)) continue;
+            int code = 0;
+            if (t < rows) {
+                code = p.cat[q][row0 + t];
+                if (code < 0 || code >= levels) { atomicOr(&p.flags[1], 1); code = 0; }
             }
-            if (lane == 0) {
-                if (p.w) wdst[pos] = wv;
-                sdst[pos] = p.src_add + (uint32_t)(row0 + t);      // frame row of the packed row (ob_design_update_outcome)
+            for (int lv = 1; lv < levels; ++lv) {                             // builder.rs:402-409: level lv -> column start + lv - 1
+                const int c = start + lv - 1;
+                if (c >= c0 && c < c1) tile[t * ts + c - c0] = (t < rows && code == lv) ? 1.0 : 0.0;
+            }
+        }
+        __syncthreads();
+        // ---- write out: one warp per packed row, lanes over the pass's contiguous columns; the sqrt(w)-scaled copy
+        //      (ols.rs:68-78) is written in the same pass ----
+        const int cend = last ? p.ldx : c1;                                    // pad columns [V, ldx) are written as zeros
+        for (int g = 0; g < 2; ++g) {
+            double* X = g ? p.XB : p.XA;
+            double* Xs = g ? p.XsB : p.XsA;
+            double* W = g ? p.wB : p.wA;
+            uint32_t* SRC = g ? p.srcB : p.srcA;
+            const int* src = g ? srcB : srcA;
+            const long long base = g ? baseB : baseA;
+            for (int r = warp; r < cnt[g]; r += PK_THREADS / 32) {
+                const int t = src[r];
+                const double wv = p.w ? p.w[row0 + t] : 1.0;
+                if (last && wv < 0.0 && lane == 0) atomicOr(&p.flags[0], 1);   // ols.rs:60-66 (the chunked pack has no earlier look at w)
+                const double sw = sqrt(wv);
+                long long pos = base + r + p.shift[g];
+                const bool mine = pos >= 0 && pos < p.n_local[g];
+                double* xdst = X; double* xsdst = Xs; double* wdst = W; uint32_t* sdst = SRC;
+                if (!mine) {      // another rank's row: export buffer, no scaled copy (the receiver scales what it imports)
+                    pos = pos < 0 ? pos + p.lo_add[g] : p.hi_base[g] + (pos - p.n_local[g]);
+                    xdst = p.EX[g]; xsdst = nullptr; wdst = p.Ew[g]; sdst = p.Esrc[g];
+                }
+                double* xr = xdst + pos * p.ldx;
+                for (int c = c0 + lane; c < cend; c += 32) {
+                    const double v = c < V ? tile[t * ts + c - c0] : 0.0;
+                    xr[c] = v;
+                    if (xsdst) xsdst[pos * p.ldx + c] = sw * v;
+                }
+                if (last && lane == 0) {
+                    if (p.w) wdst[pos] = wv;
+                    sdst[pos] = p.src_add + (uint32_t)(row0 + t);      // frame row of the packed row (ob_design_update_outcome)
+                }
             }
         }
     }
@@ -226,8 +239,13 @@ void pack_scatter(const PackArgs& a, const long long* d_block_base, GroupData ga
         p.EX[g] = win ? win->EX[g] : nullptr; p.Ew[g] = win ? win->Ew[g] : nullptr; p.Esrc[g] = win ? win->Esrc[g] : nullptr;
     }
     p.src_add = win ? win->src_add : 0u;
+    // the widest odd tile row that fits next to the kernel's static shared memory; wider designs are staged in passes
+    cudaFuncAttributes fa;
+    OB_CUDA(cudaFuncGetAttributes(&fa, pack_scatter_kernel));
+    const int max_ts = (int)((227 * 1024 - fa.sharedSizeBytes) / (sizeof(double) * PK_ROWS));
     const int V = a.K + 1;
-    const size_t smem = sizeof(double) * (size_t)PK_ROWS * (V | 1);
+    p.tile_cols = std::min(V, (max_ts - 1) | 1);
+    const size_t smem = sizeof(double) * (size_t)PK_ROWS * (p.tile_cols | 1);
     OB_CUDA(cudaFuncSetAttribute(pack_scatter_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     pack_scatter_kernel<<<nb, PK_THREADS, smem, st>>>(p);
     OB_CUDA(cudaGetLastError());
