@@ -325,6 +325,30 @@ ob_status ob_gram_cache_last_use(const ob_gram_cache* c, int32_t* use, int64_t* 
 ob_status ob_bootstrap_run_cached(ob_ctx* ctx, const ob_design* design, const ob_boot_opts* opts, ob_gram_cache* cache,
                                   ob_result* res);
 
+/* ---- Bayesian bootstrap (Rubin 1981): Dirichlet-weighted replicates instead of multinomial counts ---------------------
+ * Replicate b gives row i of group g the weight pi_i = n_g E_i / sum_{j in g} E_j with E_i ~ iid Exp(1): Dirichlet(1, .., 1)
+ * scaled to n_g, stratified by group like the row bootstrap.  A replicate is the reference's single pass (builder.rs:420-699)
+ * with the multiplicity c_i replaced by pi_i: WLS on the weights pi_i w_i, means sum(pi w x) / sum(pi w), Cotton / Weighted
+ * omega from sum_g pi w when weighted and n_g when not, Pooled stacks the two pi-weighted groups, and the n-guards use n_g
+ * (every row is present).  No replicate can lose a row, so none loses a categorical level the way a row-bootstrap draw can
+ * (an all-zero dummy column makes X'WX singular and the replicate is dropped).  The point estimate (slot 0, weight 1) is the
+ * unchanged point pass.
+ * Native stream (wt_a = wt_b = NULL, or bayes = NULL): E = -log U, U in (0, 1) from Philox4x32-10 keyed by (seed; global
+ * row, group, global replicate id, a stream tag of its own), E rounded to fp32: results do not depend on batching, grid shape,
+ * replicate sharding (mode R) or row sharding (mode N).  Explicit stream (test-only, like idx_a / idx_b): wt_a [reps x n_a]
+ * and wt_b [reps x n_b], positive unnormalised E in the group's frame order; the library applies the same normalisation.
+ * The weights are fp32 A operands of the FP64 Gram contraction (4 bytes per row and replicate of workspace), which bounds
+ * the design at K + outcomes <= 236.  opts->idx_a / idx_b must be NULL and count_bits 0 (OB_ERR_INVALID_ARG).  cache may be
+ * NULL; with a cache the native stream fills and reuses it like ob_bootstrap_run_cached (the scheme is part of its key).
+ * Refused (OB_ERR_UNSUPPORTED): clustered designs, designs with a selection equation, K + outcomes > 236, and a cache with
+ * an explicit stream. */
+typedef struct ob_bayes_opts {
+    const float* wt_a;               /* [reps x n_a] or NULL (native stream) */
+    const float* wt_b;               /* [reps x n_b] or NULL */
+} ob_bayes_opts;
+ob_status ob_bootstrap_run_bayes(ob_ctx* ctx, const ob_design* design, const ob_boot_opts* opts, const ob_bayes_opts* bayes,
+                                 ob_gram_cache* cache, ob_result* res);
+
 /* Reduction alone, on host arrays gathered from several shards, in replicate order
  * (process_component, builder.rs:849-865): out arrays [S] each. */
 ob_status ob_reduce_stats(ob_ctx* ctx, const double* rep_stats, const int32_t* rep_status, int64_t reps, int32_t S,
@@ -470,6 +494,9 @@ int64_t ob_debug_gram_outcome_columns(int32_t K, int32_t T, uint16_t* pairs_out,
 ob_status ob_debug_counts(ob_ctx* ctx, const ob_design* d, uint64_t seed, int64_t rep, int32_t group,
                           uint16_t* counts_out);
 
+/* The native Bayesian-bootstrap weights E (unnormalised, fp32) of global replicate `rep` of `group`, [n_group] in row
+ * order, from the production kernel (tests; not on row-sharded designs). */
+ob_status ob_debug_bayes_weights(ob_ctx* ctx, const ob_design* d, uint64_t seed, int64_t rep, int32_t group, float* out);
 /* The multiplicity matrix ob_bootstrap_run builds from an explicit index stream (same kernel), read back for the
  * bit-exactness tests: idx [reps x n_global] (host; global row positions within the group), counts_out
  * [reps x n_local] (row-major by replicate; n_local = the rows of the group this design holds, all of them unless

@@ -52,6 +52,9 @@ ob_status ob_builder_index_stream(ob_builder* b, const uint32_t* idx_a, const ui
  * again.  run, run_outcomes and decompose_quantile honour it; an index stream then draws units (joint: idx_b = NULL).
  * The results gain a summary line and a "clusters" JSON key {strata, units_a, units_b}. */
 ob_status ob_builder_cluster(ob_builder* b, const char* column, int32_t strata);
+/* Bayesian bootstrap (ob_bootstrap_run_bayes) when on != 0: Dirichlet row weights instead of multinomial counts; run,
+ * run_outcomes and decompose_quantile honour it.  The results gain a summary line and "bootstrap_scheme": "bayes" in JSON. */
+ob_status ob_builder_bayesian(ob_builder* b, int32_t on);
 
 ob_status ob_builder_run(ob_builder* b, ob_results** out);
 /* run() once per outcome column names[n] (f64 columns) on ONE ingest: rows are cleaned over every listed column (plus the

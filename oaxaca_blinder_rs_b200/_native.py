@@ -32,6 +32,7 @@ SYMBOLS = ["ob_abi_version", "ob_device_count", "ob_ctx_create", "ob_ctx_destroy
            "ob_design_pack_row_shard_async", "ob_design_attach_selection", "ob_design_selection_cols", "ob_num_stats_heckman",
            "ob_mm_run", "ob_debug_gram_columns", "ob_gram_cache_create", "ob_gram_cache_destroy", "ob_gram_cache_last_use",
            "ob_bootstrap_run_cached", "ob_debug_gram_outcome_columns", "ob_design_attach_clusters", "ob_design_clusters",
+           "ob_bootstrap_run_bayes", "ob_debug_bayes_weights",
            "ob_debug_gram_cache_read"]
 
 
@@ -57,6 +58,10 @@ class RawFrame(C.Structure):
 
 class SelectionView(C.Structure):
     _fields_ = [("n_pred", C.c_int32), ("pred", C.POINTER(_DP)), ("outcome", _DP)]
+
+
+class BayesOpts(C.Structure):
+    _fields_ = [("wt_a", C.POINTER(C.c_float)), ("wt_b", C.POINTER(C.c_float))]
 
 
 class BootOpts(C.Structure):
@@ -135,6 +140,9 @@ def lib() -> C.CDLL:
         L.ob_gram_cache_destroy.restype = None
         L.ob_gram_cache_last_use.argtypes = [C.c_void_p, _IP, C.POINTER(C.c_int64)]
         L.ob_bootstrap_run_cached.argtypes = [C.c_void_p, C.c_void_p, C.POINTER(BootOpts), C.c_void_p, C.POINTER(Result)]
+        L.ob_bootstrap_run_bayes.argtypes = [C.c_void_p, C.c_void_p, C.POINTER(BootOpts), C.POINTER(BayesOpts), C.c_void_p,
+                                             C.POINTER(Result)]
+        L.ob_debug_bayes_weights.argtypes = [C.c_void_p, C.c_void_p, C.c_uint64, C.c_int64, C.c_int32, C.POINTER(C.c_float)]
         L.ob_debug_gram_cache_read.argtypes = [C.c_void_p, C.c_void_p, C.POINTER(C.c_int64), _DP, _DP, C.POINTER(C.c_int64)]
         L.ob_debug_gram_outcome_columns.argtypes = [C.c_int32, C.c_int32, C.POINTER(C.c_uint16), _IP, C.c_int64, _IP]
         L.ob_debug_gram_outcome_columns.restype = C.c_int64

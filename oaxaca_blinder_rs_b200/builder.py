@@ -57,6 +57,7 @@ def _blib():
         L.ob_builder_reference_coefficients.argtypes = [vp, i32]
         L.ob_builder_heckman_selection.argtypes = [vp, cp, C.POINTER(cp), i32]
         L.ob_builder_cluster.argtypes = [vp, cp, i32]
+        L.ob_builder_bayesian.argtypes = [vp, i32]
         L.ob_builder_seed.argtypes = [vp, C.c_uint64]
         L.ob_builder_device.argtypes = [vp, i32]
         L.ob_builder_index_stream.argtypes = [vp, N._U32P, N._U32P]
@@ -97,7 +98,7 @@ BUILDER_SYMBOLS = ["ob_frame_new", "ob_frame_free", "ob_frame_add_f64", "ob_fram
                    "ob_builder_new", "ob_builder_from_formula", "ob_builder_free", "ob_builder_predictors",
                    "ob_builder_categorical_predictors", "ob_builder_normalize", "ob_builder_weights",
                    "ob_builder_bootstrap_reps", "ob_builder_reference_coefficients", "ob_builder_heckman_selection",
-                   "ob_builder_cluster", "ob_builder_seed", "ob_builder_device", "ob_builder_index_stream", "ob_builder_run", "ob_builder_run_outcomes",
+                   "ob_builder_cluster", "ob_builder_bayesian", "ob_builder_seed", "ob_builder_device", "ob_builder_index_stream", "ob_builder_run", "ob_builder_run_outcomes",
                    "ob_builder_decompose_quantile", "ob_builder_get_data_matrices", "ob_builder_describe", "ob_builder_last_error", "ob_builder_last_status",
                    "ob_results_free", "ob_results_json", "ob_results_summary", "ob_results_markdown",
                    "ob_results_residuals",
@@ -216,6 +217,7 @@ class OaxacaResults:
         self.predictor_names = d["predictor_names"]
         self.timings_ms = dict(total=d["ms_total"], gram=d["ms_gram"])
         self.clusters = d.get("clusters")        # dict(strata, units_a, units_b) on a cluster bootstrap, else None
+        self.bootstrap_scheme = d.get("bootstrap_scheme", "multinomial")
         n = L.ob_results_residuals(handle, None)
         self.residuals = np.empty(n)
         L.ob_results_residuals(handle, self.residuals.ctypes.data_as(N._DP))
@@ -309,6 +311,12 @@ class OaxacaBuilder:
         if strata not in CLUSTER_STRATA:
             raise ValueError(f"strata must be 'group', 'joint' or None, not {strata!r}")
         return self._check(_blib().ob_builder_cluster(self._h, column.encode(), CLUSTER_STRATA[strata]))
+
+    def bayesian_bootstrap(self, on: bool = True):
+        """Bayesian bootstrap: every row keeps a Dirichlet weight n_g E_i / sum E (E ~ Exp(1)) in every replicate instead of
+        a multinomial count, so no replicate loses a rare categorical level.  run, run_outcomes and decompose_quantile
+        honour it."""
+        return self._check(_blib().ob_builder_bayesian(self._h, int(bool(on))))
 
     def device(self, device: int):
         return self._check(_blib().ob_builder_device(self._h, int(device)))

@@ -360,6 +360,14 @@ class Design:
                                                out.ctypes.data_as(C.POINTER(C.c_uint16))))
         return out
 
+    def debug_bayes_weights(self, seed: int, rep: int, group: int) -> np.ndarray:
+        """ob_debug_bayes_weights: the native Bayesian-bootstrap weights E (fp32, unnormalised) of global replicate `rep`
+        of `group`, in row order."""
+        out = np.empty(self.n_a if group == 0 else self.n_b, dtype=np.float32)
+        self.ctx.check(N.lib().ob_debug_bayes_weights(self.ctx._h, self._h, seed, rep, group,
+                                                      out.ctypes.data_as(C.POINTER(C.c_float))))
+        return out
+
     def debug_counts_from_indices(self, idx, group: int, count_bits: int = 8):
         """ob_debug_counts_from_indices: (counts [reps, n_local] uint16, flags) of an explicit index stream
         idx [reps, n_global] through the production histogram kernel."""
@@ -524,8 +532,12 @@ def bootstrap(design: Design, reps: int, ref_kind: int = REF_GROUP_A, norm: Sequ
               seed: int = 0, idx_a=None, idx_b=None, rep_begin: int = 0, rep_end: int = 0,
               skip_reduce: bool = False, count_bits: int = 0, max_workspace_bytes: int = 0,
               want_rep: bool = False, want_residuals: bool = True, residuals_out: Optional[np.ndarray] = None,
-              shard_replicates: bool = False, cache: Optional[GramCache] = None) -> dict:
+              shard_replicates: bool = False, cache: Optional[GramCache] = None, scheme: str = "multinomial",
+              wt_a=None, wt_b=None) -> dict:
     """ob_bootstrap_run (ob_bootstrap_run_cached with a GramCache: same results, and `cache_use` in the dict).  Returns point estimates, per-statistic SE/p/CI/t and (optionally) replicate detail.
+    scheme "bayes": the Bayesian bootstrap (ob_bootstrap_run_bayes): every row keeps a Dirichlet weight n_g E_i / sum E
+    with E ~ Exp(1) in every replicate.  wt_a [reps x n_a] / wt_b [reps x n_b]: a test-only explicit stream of E (float32);
+    None = the native stream.
     On a clustered design (Design.attach_clusters) idx_a / idx_b draw units: [reps x units_a] / [reps x units_b], or
     idx_a [reps x M] with idx_b=None under joint strata.
     residuals_out: optional preallocated float64 [n_b] buffer for OaxacaResults.residuals (reusing one across calls
@@ -550,6 +562,18 @@ def bootstrap(design: Design, reps: int, ref_kind: int = REF_GROUP_A, norm: Sequ
     hb = np.array([int(v.has_base) for v in norm] + [0], dtype=np.int32)
     o.norm_m, o.norm_off, o.norm_idx, o.norm_has_base = _ip(m), _ip(off), _ip(idx), _ip(hb)
     o.reps, o.seed = reps, seed
+    if scheme not in ("multinomial", "bayes"):
+        raise ValueError(f"scheme must be 'multinomial' or 'bayes', not {scheme!r}")
+    bo = None
+    if scheme == "bayes":
+        bo = N.BayesOpts()
+        if wt_a is not None or wt_b is not None:
+            wt_a = np.ascontiguousarray(wt_a, dtype=np.float32)
+            wt_b = np.ascontiguousarray(wt_b, dtype=np.float32)
+            assert wt_a.shape == (reps, design.n_a_global) and wt_b.shape == (reps, design.n_b_global)
+            bo.wt_a, bo.wt_b = wt_a.ctypes.data_as(C.POINTER(C.c_float)), wt_b.ctypes.data_as(C.POINTER(C.c_float))
+    elif wt_a is not None or wt_b is not None:
+        raise ValueError("wt_a / wt_b are weight streams of scheme='bayes'")
     cl = design.clusters
     if idx_a is not None and cl is not None and cl["strata"] == "joint":
         # one unit stream over both groups
@@ -589,7 +613,10 @@ def bootstrap(design: Design, reps: int, ref_kind: int = REF_GROUP_A, norm: Sequ
     for k, v in a.items():
         setattr(r, k, _ip(v) if v.dtype == np.int32 else _dp(v))
     try:
-        if cache is None:
+        if bo is not None:
+            ctx.check(N.lib().ob_bootstrap_run_bayes(ctx._h, design._h, C.byref(o), C.byref(bo),
+                                                     None if cache is None else cache._h, C.byref(r)))
+        elif cache is None:
             ctx.check(N.lib().ob_bootstrap_run(ctx._h, design._h, C.byref(o), C.byref(r)))
         else:
             ctx.check(N.lib().ob_bootstrap_run_cached(ctx._h, design._h, C.byref(o), cache._h, C.byref(r)))

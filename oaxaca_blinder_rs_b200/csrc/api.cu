@@ -88,12 +88,14 @@ struct ob_gram_cache {
     double* xx = nullptr; size_t xx_bytes = 0;   // [2][slots][K(K+1)/2]
     double* yy = nullptr; size_t yy_bytes = 0;   // [2][slots][K T + 1]
     long long* rows = nullptr; size_t rows_bytes = 0;   // clustered designs: [2][slots] group row counts (a SOLVE_ONLY run draws none)
+    double* esum = nullptr; size_t esum_bytes = 0;      // Bayesian bootstrap: [2][slots] sums of the raw weights per slot
     // key of xx (valid while xx_ok): what decides the resamples and the design's X'WX
     bool xx_ok = false;
     uint64_t design_id = 0, x_gen = 0, seed = 0;
     int64_t reps = 0, rep_begin = 0, rep_end = 0, slots = 0;
     int shard_reps = 0, rep_world = 1, rep_rank = 0, row_world = 1, row_rank = 0, K = 0;
     int count_bytes = 1;             // multiplicity width the fill ended with (a saturation already known)
+    bool bayes = false;              // resampling scheme of the fill: Bayesian (Dirichlet) weights or multinomial counts
     // key of yy (valid while y_ok): the design's outcome generation and outcome count
     bool y_ok = false;
     uint64_t y_gen = 0; int T = 0;
@@ -281,8 +283,9 @@ void cache_release_device(ob_gram_cache* c) {
         if (c->xx) cudaFreeAsync(c->xx, st);
         if (c->yy) cudaFreeAsync(c->yy, st);
         if (c->rows) cudaFreeAsync(c->rows, st);
+        if (c->esum) cudaFreeAsync(c->esum, st);
     }
-    c->xx = c->yy = nullptr; c->rows = nullptr; c->xx_bytes = c->yy_bytes = c->rows_bytes = 0;
+    c->xx = c->yy = nullptr; c->rows = nullptr; c->esum = nullptr; c->xx_bytes = c->yy_bytes = c->rows_bytes = c->esum_bytes = 0;
     c->xx_ok = c->y_ok = false;
 }
 
@@ -495,11 +498,59 @@ int generate_counts(const ob_design* d, const Opts* o, const Batch& b, int count
     return launches;
 }
 
+// The batch's Bayesian-bootstrap weights of both groups (resample.cu: native stream, or the caller's explicit fp32 stream
+// uploaded per batch into wt) and their per-slot sums esum [2][b.pn * BM]: leaf partials into part, summed by the Gram's
+// aligned leaf tree.  Mode N: each rank sums its aligned subtree into esum_local, the per-rank sums are gathered and the top
+// of the tree evaluated on every rank (gram_combine_launch), so esum is bit-identical to the single-GPU sums.
+struct BayesWork {
+    DevBuf wt[2], part, esum, esum_local, gathered;
+    int ranks_with_rows[2];
+};
+int generate_weights(const ob_design* d, const ob_boot_opts* o, const ob_bayes_opts* bo, const Batch& b, DevBuf (&C)[2],
+                     BayesWork& w, int* flags, Comm* row_comm, double* ms_comm, cudaStream_t st) {
+    const int64_t spad = b.pn * BM;
+    int segs[2];
+    int64_t leaf0 = 0;
+    for (int g = 0; g < 2; ++g) {
+        const GroupData& G = d->g[g];
+        BayesArgs a;
+        a.C = C[g].as<float>(); a.n = G.n; a.n_pad = G.n_pad; a.panels = (int)b.pn;
+        a.n_global = G.shard.n_global; a.row_begin = G.shard.row_begin;
+        a.slots = b.bslots; a.first_slot = b.first_slot; a.rep0 = b.rep0; a.group = g; a.seed = o->seed;
+        a.segs = segs[g] = G.shard.leaf_hi - G.shard.leaf_lo; a.seg_rows = G.shard.seg_rows;
+        a.wt = nullptr; a.flags = flags;
+        a.part = w.part.as<double>() + (size_t)leaf0 * spad;
+        leaf0 += a.segs;
+        const float* h = bo ? (g == 0 ? bo->wt_a : bo->wt_b) : nullptr;
+        if (h) {
+            const size_t nb = sizeof(float) * (size_t)std::max<int64_t>(b.brep, 1) * a.n_global;
+            if (w.wt[g].bytes < nb) w.wt[g].alloc(nb);
+            if (b.brep > 0)
+                OB_CUDA(cudaMemcpyAsync(w.wt[g].p, h + (size_t)(b.rep0 + b.first_slot) * a.n_global,
+                                        sizeof(float) * (size_t)b.brep * a.n_global, cudaMemcpyHostToDevice, st));
+            a.wt = w.wt[g].as<float>();
+        }
+        bayes_weights_launch(a, st);
+    }
+    const int span = d->g[0].shard.leaf_span;
+    leaf_sum_launch(w.part.as<double>(), segs, spad, span, row_comm ? w.esum_local.as<double>() : w.esum.as<double>(), st);
+    int launches = 3;
+    if (row_comm) {
+        Timer t_c(st, ms_comm);
+        row_comm->allgather(w.esum_local.p, w.gathered.p, sizeof(double) * 2 * (size_t)spad, st);
+        gram_combine_launch(w.gathered.as<double>(), row_comm->world, w.ranks_with_rows, spad, w.esum.as<double>(), st);
+        t_c.stop(); OB_CUDA(cudaStreamSynchronize(st)); t_c.collect();
+        launches += 1;
+    }
+    return launches;
+}
+
 // A batch's deferred error flags (multiplicity kernels): a bad index or a Poisson overshoot fails the call.  A saturated
 // count returns true when the run may widen to 16-bit counts and redo, and fails when it may not: already 16-bit, 8 bits
 // asked for, or a design (row stride ldx) too wide for the Gram kernel at 16 bits.
 bool check_batch_flags(const int flags[4], int count_bytes, int count_bits, int ldx) {
     if (flags[2]) fail(OB_ERR_INVALID_ARG, "resample index out of range");
+    if (flags[3]) fail(OB_ERR_INVALID_ARG, "explicit Bayesian weight that is not a positive normal float");
     if (flags[0]) fail(OB_ERR_CUDA, "Poisson body overshot n (probability < 1e-15 per replicate); rerun with another seed");
     if (flags[1] && (count_bytes == 2 || count_bits == 8 || !gram_fits(ldx, 2)))
         fail(OB_ERR_UNSUPPORTED, "row multiplicity overflows the count width");
@@ -2054,8 +2105,24 @@ ob_status ob_mm_run(ob_ctx* ctx, const ob_design* d, const ob_mm_opts* o, ob_mm_
 // ob_bootstrap_run, and with a cache ob_bootstrap_run_cached: the batch loop contracts the full Gram (no cache, or a
 // cache that is (re)filled), only its outcome columns (OB_CACHE_OUTCOME_ONLY: X'WX comes from the cache) or nothing
 // (OB_CACHE_SOLVE_ONLY: the whole Gram comes from the cache, no multiplicities are generated)
-static void bootstrap_body(ob_ctx* ctx, const ob_design* d, const ob_boot_opts* o, ob_gram_cache* cache, ob_result* res) {
+// bayes: the Bayesian bootstrap (ob_bootstrap_run_bayes; bo null or null streams = the native stream)
+static void bootstrap_body(ob_ctx* ctx, const ob_design* d, const ob_boot_opts* o, ob_gram_cache* cache, ob_result* res,
+                           bool bayes = false, const ob_bayes_opts* bo = nullptr) {
         design_alive(d);
+        const bool bayes_explicit = bayes && bo && (bo->wt_a || bo->wt_b);
+        if (bayes) {
+            if (d->cl_strata != OB_CLUSTER_NONE)
+                fail(OB_ERR_UNSUPPORTED, "Bayesian bootstrap on a clustered design: cluster weights are not built (detach the clusters)");
+            if (d->K1 > 0)
+                fail(OB_ERR_UNSUPPORTED, "Bayesian bootstrap on a design with a selection equation: the Heckman estimator is not built for it");
+            if (o->idx_a || o->idx_b)
+                fail(OB_ERR_INVALID_ARG, "the Bayesian bootstrap takes no index stream (idx_a / idx_b must be NULL; explicit weights go in ob_bayes_opts)");
+            if (o->count_bits != 0) fail(OB_ERR_INVALID_ARG, "the Bayesian bootstrap has fp32 weights: count_bits must be 0");
+            if (!gram_fits(d->ldx, 4))
+                fail(OB_ERR_UNSUPPORTED, "design too wide for the Bayesian bootstrap: K + outcomes <= 236 with fp32 weights");
+            if (cache && bayes_explicit)
+                fail(OB_ERR_UNSUPPORTED, "a Gram cache needs the native weight stream (explicit weight streams cannot be keyed)");
+        }
         if (cache && d->K1 > 0) fail(OB_ERR_UNSUPPORTED, "a Gram cache does not apply to designs with a selection equation (Heckman)");
         if (cache && (o->idx_a || o->idx_b)) fail(OB_ERR_UNSUPPORTED, "a Gram cache needs the native resampling stream (explicit index streams cannot be keyed)");
         if (d->K1 > 0) {                 // a selection equation is attached: the Heckman two-step estimator per replicate
@@ -2089,7 +2156,7 @@ static void bootstrap_body(ob_ctx* ctx, const ob_design* d, const ob_boot_opts* 
             const bool xx_hit = cache->xx_ok && cache->design_id == d->id && cache->x_gen == d->x_gen && cache->seed == o->seed &&
                                 cache->reps == o->reps && cache->rep_begin == rr.rb && cache->rep_end == rr.re &&
                                 cache->shard_reps == (rr.shard_reps ? 1 : 0) && cache->rep_world == rep_world && cache->rep_rank == rep_rank &&
-                                cache->row_world == d->world && cache->row_rank == d->rank && cache->K == d->K &&
+                                cache->row_world == d->world && cache->row_rank == d->rank && cache->K == d->K && cache->bayes == bayes &&
                                 !(o->count_bits == 8 && cache->count_bytes == 2);   // that run saturates 8-bit counts: let it fail
             mode = !xx_hit ? OB_CACHE_FILLED : (cache->y_ok && cache->y_gen == d->y_gen && cache->T == d->T) ? OB_CACHE_SOLVE_ONLY
                                                                                                            : OB_CACHE_OUTCOME_ONLY;
@@ -2106,8 +2173,10 @@ static void bootstrap_body(ob_ctx* ctx, const ob_design* d, const ob_boot_opts* 
             if (o->norm_idx[t] < 0 || o->norm_idx[t] >= K) fail(OB_ERR_INVALID_ARG, "norm_idx outside the design");
         const int D = K + n_base, S = 5 + 2 * D;
         const int SE = T * S, KE = T * K;     // per slot: T outcomes (a quantile sweep) x S statistics / K coefficients
-        int count_bytes = rr.count_bytes;
+        int count_bytes = bayes ? 4 : rr.count_bytes;                                // fp32 weights: 4 bytes a cell
         if (outcome_only && o->count_bits == 0) count_bytes = cache->count_bytes;   // start where the fill ended
+        if (bayes && rr.nrep > 0 && bayes_explicit && (!bo->wt_a || !bo->wt_b))
+            fail(OB_ERR_INVALID_ARG, "an explicit weight stream needs both wt_a and wt_b");
 
         res->ms_counts = res->ms_gram = res->ms_solve = res->ms_reduce = res->ms_total = res->ms_gram_kernel = res->ms_comm = 0.0;
         res->gpu_launches = 0;
@@ -2147,6 +2216,11 @@ static void bootstrap_body(ob_ctx* ctx, const ob_design* d, const ob_boot_opts* 
                 OB_CUDA(cudaMallocFromPoolAsync((void**)&cache->rows, cache->rows_bytes, ctx->pool_design, st));
                 cache_new_bytes += cache->rows_bytes;
             }
+            if (bayes) {
+                cache->esum_bytes = sizeof(double) * 2 * (size_t)slots;
+                OB_CUDA(cudaMallocFromPoolAsync((void**)&cache->esum, cache->esum_bytes, ctx->pool_design, st));
+                cache_new_bytes += cache->esum_bytes;
+            }
         }
         if (mode == OB_CACHE_FILLED || outcome_only) {
             cache->y_ok = false;
@@ -2180,8 +2254,12 @@ static void bootstrap_body(ob_ctx* ctx, const ob_design* d, const ob_boot_opts* 
         // workspace of one panel: multiplicities (+ index stream), reduced Gram (+ the mode-N exchange), partial tiles, column
         // sums; a run that only solves needs the reduced Gram alone
         // (clustered: + the unit matrices and the per-slot row counts)
+        // (Bayesian: + the per-slot weight sums, their leaf partials and mode-N exchange, and an explicit stream's upload)
         auto per_panel_bytes = [&](int cb) {
-            const double cl = clustered ? (solve_only ? 0.0 : (double)u_pad_all * BM * cb) + 2.0 * BM * 8.0 : 0.0;
+            double cl = clustered ? (solve_only ? 0.0 : (double)u_pad_all * BM * cb) + 2.0 * BM * 8.0 : 0.0;
+            if (bayes)
+                cl = 2.0 * BM * 8.0 + (solve_only ? 0.0 : (double)local_leaves * BM * 8.0 + (comm ? world + 1 : 0) * 2.0 * BM * 8.0 +
+                                                          (bayes_explicit ? (double)(n_glob[0] + n_glob[1]) * BM * 4.0 : 0.0));
             if (solve_only) return 2.0 * BM * Pld * 8.0 + cl;
             return (double)(n_pad[0] + n_pad[1]) * BM * cb + (rr.index_mode ? (double)idx_len * BM * 4.0 : 0.0) +
                    2.0 * BM * Pld * 8.0 * (comm ? world + 2 : 1) + (double)local_leaves * ntiles * (BM * BN * 8.0) + 2.0 * BM * 8.0 + cl;
@@ -2216,17 +2294,24 @@ static void bootstrap_body(ob_ctx* ctx, const ob_design* d, const ob_boot_opts* 
             tr.mark("setup", st, true);
             DevBuf d_C[2], d_idx[2], d_colsum, d_gram, d_gram_local, d_gathered, d_rows;
             ClusterWork cw;
+            BayesWork bw;
+            bw.ranks_with_rows[0] = ranks_with_rows[0]; bw.ranks_with_rows[1] = ranks_with_rows[1];
             const size_t gram_elems = 2 * (size_t)ppb * BM * Pld;      // [2][slots_pad][Pld]
             bool saturated = false;
             GramPlan plan; int64_t plan_panels = -1;
             DevBuf d_partials, d_pairs, d_colmap, d_cmap;
             auto allocate_workspace = [&] {
                 if (!solve_only) {
-                    d_colsum.alloc(sizeof(long long) * 2 * (size_t)ppb * BM);
+                    if (!bayes) d_colsum.alloc(sizeof(long long) * 2 * (size_t)ppb * BM);
                     for (int g = 0; g < 2; ++g) d_C[g].alloc((size_t)ppb * n_pad[g] * BM * count_bytes);
                     for (int m = 0; m < mats; ++m) cw.U[m].alloc((size_t)ppb * pad_rows(d->cl_units[m]) * BM * count_bytes);
                 }
                 if (clustered) { d_rows.alloc(sizeof(long long) * 2 * (size_t)ppb * BM); cw.rows = d_rows.as<long long>(); }
+                if (bayes) {
+                    bw.esum.alloc(sizeof(double) * 2 * (size_t)ppb * BM);
+                    if (!solve_only) bw.part.alloc(sizeof(double) * (size_t)std::max<int64_t>(local_leaves, 1) * ppb * BM);
+                    if (!solve_only && comm) { bw.esum_local.alloc(sizeof(double) * 2 * (size_t)ppb * BM); bw.gathered.alloc(sizeof(double) * 2 * (size_t)ppb * BM * world); }
+                }
                 d_gram.alloc(sizeof(double) * gram_elems);
                 if (cache) {
                     const std::vector<int32_t> cmap = gram_cache_map(K, T);
@@ -2256,7 +2341,9 @@ static void bootstrap_body(ob_ctx* ctx, const ob_design* d, const ob_boot_opts* 
 
                 // (2) replicate generation (none when the cache holds every Gram cell of these slots)
                 Timer t_counts(st, &res->ms_counts);
-                if (!solve_only)
+                if (!solve_only && bayes)
+                    res->gpu_launches += generate_weights(d, o, bo, b, d_C, bw, d_flags.as<int>(), comm, &res->ms_comm, st);
+                else if (!solve_only)
                     res->gpu_launches += generate_counts(d, o, b, count_bytes, ppb, d_C, d_idx, d_colsum, d_lut, d_flags.as<int>(), comm,
                                                          &res->ms_comm, st, clustered ? &cw : nullptr);
                 t_counts.stop();
@@ -2357,6 +2444,13 @@ static void bootstrap_body(ob_ctx* ctx, const ob_design* d, const ob_boot_opts* 
                         OB_CUDA(cudaMemcpyAsync(solve_only ? batch_rows : kept, solve_only ? kept : batch_rows, sizeof(long long) * (size_t)bslots,
                                                 cudaMemcpyDeviceToDevice, st));
                     }
+                    // Bayesian: so do the per-slot weight sums
+                    for (int g = 0; bayes && g < 2 && (mode == OB_CACHE_FILLED || solve_only); ++g) {
+                        double* batch_esum = bw.esum.as<double>() + (size_t)g * pn * BM;
+                        double* kept = cache->esum + (size_t)g * slots + b.slot_lo;
+                        OB_CUDA(cudaMemcpyAsync(solve_only ? batch_esum : kept, solve_only ? kept : batch_esum, sizeof(double) * (size_t)bslots,
+                                                cudaMemcpyDeviceToDevice, st));
+                    }
                     if (mode == OB_CACHE_FILLED) gram_cache_extract_launch(cc, st);
                     else if (solve_only) gram_cache_assemble_launch(cc, st);
                     else {
@@ -2378,6 +2472,7 @@ static void bootstrap_body(ob_ctx* ctx, const ob_design* d, const ob_boot_opts* 
                 sa.n_base = n_base; sa.S = S; sa.weighted = d->weighted ? 1 : 0;
                 sa.na = (double)n_glob[0]; sa.nb = (double)n_glob[1];
                 sa.rows = clustered ? d_rows.as<long long>() : nullptr;     // [2][pn * BM]
+                sa.esum = bayes ? bw.esum.as<double>() : nullptr;           // [2][pn * BM]
                 sa.stats = d_stats.as<double>() + (size_t)b.slot_lo * SE;
                 sa.status = d_status.as<int>() + b.slot_lo;
                 sa.beta_a = want_beta ? d_ba.as<double>() + (size_t)b.slot_lo * KE : nullptr;
@@ -2420,6 +2515,7 @@ static void bootstrap_body(ob_ctx* ctx, const ob_design* d, const ob_boot_opts* 
                 cache->reps = o->reps; cache->rep_begin = rr.rb; cache->rep_end = rr.re; cache->slots = slots;
                 cache->shard_reps = rr.shard_reps ? 1 : 0; cache->rep_world = rep_world; cache->rep_rank = rep_rank;
                 cache->row_world = d->world; cache->row_rank = d->rank; cache->K = K; cache->count_bytes = count_bytes;
+                cache->bayes = bayes;
                 cache->xx_ok = true;
             }
             if (!solve_only) { cache->y_gen = d->y_gen; cache->T = T; cache->y_ok = true; }
@@ -2531,7 +2627,7 @@ void ob_gram_cache_destroy(ob_gram_cache* c) {
 ob_status ob_gram_cache_last_use(const ob_gram_cache* c, int32_t* use, int64_t* bytes) {
     if (!c) return OB_ERR_INVALID_ARG;
     if (use) *use = c->last_use;
-    if (bytes) *bytes = (int64_t)(c->xx_bytes + c->yy_bytes + c->rows_bytes);
+    if (bytes) *bytes = (int64_t)(c->xx_bytes + c->yy_bytes + c->rows_bytes + c->esum_bytes);
     return OB_OK;
 }
 
@@ -2541,6 +2637,22 @@ ob_status ob_bootstrap_run_cached(ob_ctx* ctx, const ob_design* d, const ob_boot
         if (cache->owner != ctx) fail(OB_ERR_INVALID_ARG, "this Gram cache belongs to another context");
         try {
             bootstrap_body(ctx, d, o, cache, res);
+        } catch (...) {          // whatever failed, the next call fills the cache anew
+            cache_release_device(cache);
+            cache->last_use = OB_CACHE_NONE;
+            throw;
+        }
+    });
+}
+
+ob_status ob_bootstrap_run_bayes(ob_ctx* ctx, const ob_design* d, const ob_boot_opts* o, const ob_bayes_opts* bo,
+                                 ob_gram_cache* cache, ob_result* res) {
+    if (!ctx || !d || !o || !res) return OB_ERR_INVALID_ARG;
+    return guarded(ctx, [&] {
+        if (!cache) { bootstrap_body(ctx, d, o, nullptr, res, true, bo); return; }
+        if (cache->owner != ctx) fail(OB_ERR_INVALID_ARG, "this Gram cache belongs to another context");
+        try {
+            bootstrap_body(ctx, d, o, cache, res, true, bo);
         } catch (...) {          // whatever failed, the next call fills the cache anew
             cache_release_device(cache);
             cache->last_use = OB_CACHE_NONE;
@@ -2644,6 +2756,28 @@ ob_status ob_debug_counts(ob_ctx* ctx, const ob_design* d, uint64_t seed, int64_
         // slot 1 column of the single panel
         OB_CUDA(cudaMemcpy2DAsync(counts_out, sizeof(uint16_t), d_C.as<uint16_t>() + 1, sizeof(uint16_t) * BM,
                                   sizeof(uint16_t), (size_t)G.n, cudaMemcpyDeviceToHost, st));
+        OB_CUDA(cudaStreamSynchronize(st));
+    });
+}
+
+// The native Bayesian-bootstrap weights E of one replicate of one group, read back (the production kernel, one panel).
+ob_status ob_debug_bayes_weights(ob_ctx* ctx, const ob_design* d, uint64_t seed, int64_t rep, int32_t group, float* out) {
+    if (!ctx || !d || !out || group < 0 || group > 1 || rep < 0) return OB_ERR_INVALID_ARG;
+    return guarded(ctx, [&] {
+        design_ready(d);
+        if (d->world > 1) fail(OB_ERR_UNSUPPORTED, "ob_debug_bayes_weights on a row-sharded design");
+        cudaStream_t st = ctx->stream;
+        const GroupData& G = d->g[group];
+        const int segs = G.shard.leaf_hi - G.shard.leaf_lo;
+        DevBuf d_C((size_t)G.n_pad * BM * sizeof(float)), d_part(sizeof(double) * (size_t)std::max(segs, 1) * BM);
+        BayesArgs a;
+        a.C = d_C.as<float>(); a.n = G.n; a.n_pad = G.n_pad; a.panels = 1;
+        a.n_global = G.shard.n_global; a.row_begin = G.shard.row_begin;
+        a.slots = 2; a.first_slot = 1; a.rep0 = rep - 1; a.group = group; a.seed = seed;
+        a.segs = segs; a.seg_rows = G.shard.seg_rows; a.wt = nullptr; a.part = d_part.as<double>();
+        bayes_weights_launch(a, st);
+        OB_CUDA(cudaMemcpy2DAsync(out, sizeof(float), d_C.as<float>() + 1, sizeof(float) * BM, sizeof(float), (size_t)G.n,
+                                  cudaMemcpyDeviceToHost, st));
         OB_CUDA(cudaStreamSynchronize(st));
     });
 }

@@ -27,6 +27,7 @@
 
 #include <algorithm>
 #include <cstdlib>
+#include <type_traits>
 
 namespace ob {
 
@@ -62,11 +63,19 @@ struct GramKernelParams {
 // of the current stage's DMMA loop.  uint8 counts go through a 256-entry fp64 table in shared memory (no FP64-pipe
 // work: that pipe is what the DMMAs need); uint16 counts use the exact magic-number conversion (2^52 + c) - 2^52.
 // Sample weights are NOT applied here: the design rows are already sqrt(w)-scaled (ols.rs:68-78), so A is the
-// bare multiplicity.
+// bare multiplicity.  fp32 Bayesian-bootstrap weights (resample.cu) are widened by integer bit operations alone: for a
+// positive normal float the fp64 exponent is the fp32 one rebiased by 1023 - 127 = 896 and the 23 mantissa bits move up
+// by 29, so the value is exact and the FP64 pipe stays free for the DMMAs; 0.0f (padding rows, empty slots) stays 0.0.
 template <typename CountT>
-__device__ __forceinline__ double count_to_f64(unsigned c, const double* __restrict__ tab) {
-    if (sizeof(CountT) == 1) return tab[c];
-    return __hiloint2double(0x43300000, (int)c) - 4503599627370496.0;
+__device__ __forceinline__ double count_to_f64(CountT c, const double* __restrict__ tab) {
+    if constexpr (std::is_same<CountT, float>::value) {
+        const uint32_t f = __float_as_uint(c);
+        return __hiloint2double(f ? (int)((f >> 3) + (896u << 20)) : 0, (int)(f << 29));
+    } else if constexpr (sizeof(CountT) == 1) {
+        return tab[(unsigned)c];
+    } else {
+        return __hiloint2double(0x43300000, (int)(unsigned)c) - 4503599627370496.0;
+    }
 }
 
 // ------------------------------------------------------------------------------------------------------------------
@@ -302,14 +311,17 @@ __global__ void __launch_bounds__(WS_THREADS, 1) gram_ws_kernel(const GramKernel
     }
 }
 
-static size_t gram_ws_smem(int ldx, int count_bytes, int ring = WS_R) {
+static constexpr size_t gram_ws_smem(int ldx, int count_bytes, int ring = WS_R) {
     return sizeof(double) * ((size_t)ring * A_TILE + 256 + (size_t)ring * KT * ldx) + (size_t)ring * KT * BM * count_bytes +
            sizeof(uint64_t) * 3 * ring;
 }
 constexpr size_t GRAM_SMEM_MAX = 227 * 1024;
+// ring depth of the fp32-weight kernel at a specialised row stride: three stages up to ldx 84, two beyond
+constexpr int gram_ring_f32(int ldx) { return gram_ws_smem(ldx, 4, WS_R) <= GRAM_SMEM_MAX ? WS_R : 2; }
 
 // The Gram CTA fits in shared memory at this row stride and count width (two ring stages when three do not fit):
-// ldx <= 284 (K + outcomes <= 280) with uint8 counts, ldx <= 268 (K + outcomes <= 268) with uint16 counts.
+// ldx <= 284 (K + outcomes <= 280) with uint8 counts, ldx <= 268 (K + outcomes <= 268) with uint16 counts, ldx <= 236
+// (K + outcomes <= 236) with fp32 Bayesian-bootstrap weights.
 bool gram_fits(int ldx, int count_bytes) { return gram_ws_smem(ldx, count_bytes, 2) <= GRAM_SMEM_MAX; }
 
 // Aligned binary summation tree over LEN consecutive leaves starting at `lo` (lo < cnt): leaves >= cnt are absent
@@ -383,6 +395,19 @@ __global__ void __launch_bounds__(256) gram_reduce_kernel(const double* __restri
         const int c0 = colmap[nt * BN + n], c1 = colmap[nt * BN + n + 1];
         if (c0 >= 0) dst[c0] = s.x;
         if (c1 >= 0) dst[c1] = s.y;
+    }
+}
+
+// Per-slot sums of the Bayesian-bootstrap weights: out[g][slot] = tree sum over the group's leaf partials held here,
+// part [segs0 + segs1][slots_pad] (group 0's leaves first).  The same aligned tree as gram_reduce, so the sums do not
+// depend on batching, and mode N combines the per-rank sums with gram_combine_kernel into the single-GPU values.
+__global__ void __launch_bounds__(256) leaf_sum_kernel(const double* __restrict__ part, int segs0, int segs1, long long half,
+                                                       int span, double* __restrict__ out) {
+    for (long long e = (long long)blockIdx.x * blockDim.x + threadIdx.x; e < 2 * half; e += (long long)gridDim.x * blockDim.x) {
+        const int g = e >= half ? 1 : 0;
+        const int cnt = g ? segs1 : segs0;
+        const double2* base = reinterpret_cast<const double2*>(part + (g ? (size_t)segs0 * 2 * half : 0)) + (e - (g ? half : 0));
+        reinterpret_cast<double2*>(out)[e] = cnt > 0 ? tree_sum_span(base, (size_t)half, cnt, span) : make_double2(0.0, 0.0);
     }
 }
 
@@ -543,18 +568,20 @@ void gram_launch_leaves(const GramPlan& pl, const GramArgs& a, const int seg_lo[
     const size_t ws_smem = pl.smem_bytes;
     if (!gram_fits(pl.ldx, a.count_bytes))
         throw StatusError{OB_ERR_UNSUPPORTED, "design too wide for the Gram kernel's shared-memory ring (K + outcomes <= 280 with "
-                                              "8-bit multiplicities, <= 268 with 16-bit)"};
+                                              "8-bit multiplicities, <= 268 with 16-bit, <= 236 with fp32 Bayesian weights)"};
     auto launch_ws = [&](auto kernel) {
         OB_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ws_smem));
         kernel<<<grid, WS_THREADS, ws_smem, st>>>(p);
     };
     // row stride specialisations (ldx = 4 mod 8): the common design widths get immediate shared-memory offsets
-#define OB_GRAM_WS_CASE(L) case L: if (a.count_bytes == 1) launch_ws(gram_ws_kernel<uint8_t, L>); else launch_ws(gram_ws_kernel<uint16_t, L>); break;
+#define OB_GRAM_WS_CASE(L) case L: if (a.count_bytes == 4) launch_ws(gram_ws_kernel<float, L, gram_ring_f32(L)>); \
+                                   else if (a.count_bytes == 1) launch_ws(gram_ws_kernel<uint8_t, L>); else launch_ws(gram_ws_kernel<uint16_t, L>); break;
     switch (pl.ldx) {
         OB_GRAM_WS_CASE(12) OB_GRAM_WS_CASE(20) OB_GRAM_WS_CASE(28) OB_GRAM_WS_CASE(36) OB_GRAM_WS_CASE(44) OB_GRAM_WS_CASE(52)
         OB_GRAM_WS_CASE(60) OB_GRAM_WS_CASE(68) OB_GRAM_WS_CASE(76) OB_GRAM_WS_CASE(84) OB_GRAM_WS_CASE(92)
         default:      // wider designs: run-time row stride; two ring stages when three do not fit
-            if (pl.ring == WS_R) { if (a.count_bytes == 1) launch_ws(gram_ws_kernel<uint8_t, 0, WS_R>); else launch_ws(gram_ws_kernel<uint16_t, 0, WS_R>); }
+            if (a.count_bytes == 4) { if (pl.ring == WS_R) launch_ws(gram_ws_kernel<float, 0, WS_R>); else launch_ws(gram_ws_kernel<float, 0, 2>); }
+            else if (pl.ring == WS_R) { if (a.count_bytes == 1) launch_ws(gram_ws_kernel<uint8_t, 0, WS_R>); else launch_ws(gram_ws_kernel<uint16_t, 0, WS_R>); }
             else { if (a.count_bytes == 1) launch_ws(gram_ws_kernel<uint8_t, 0, 2>); else launch_ws(gram_ws_kernel<uint16_t, 0, 2>); }
     }
 #undef OB_GRAM_WS_CASE
@@ -576,6 +603,13 @@ void gram_launch(const GramPlan& pl, const GramArgs& a, cudaStream_t st, cudaEve
     gram_launch_leaves(pl, a, nullptr, nullptr, st);
     if (ev_main_end) OB_CUDA(cudaEventRecord(ev_main_end, st));
     gram_reduce_launch(pl, a, st);
+}
+
+void leaf_sum_launch(const double* part, const int segs[2], int64_t slots_pad, int span, double* out, cudaStream_t st) {
+    const long long half = slots_pad / 2;
+    const unsigned blocks = (unsigned)std::min<long long>((2 * half + 255) / 256, 148 * 8);
+    leaf_sum_kernel<<<std::max(blocks, 1u), 256, 0, st>>>(part, segs[0], segs[1], half, span, out);
+    OB_CUDA(cudaGetLastError());
 }
 
 void gram_combine_launch(const double* gathered, int world, const int ranks_with_rows[2], int64_t per_group_elems,

@@ -607,7 +607,8 @@ std::vector<OaxacaResults> OaxacaBuilder::run_impl(bool rif, double tau, const s
         r.point_stats = point.data(); r.xa_mean = R.xa_mean.data(); r.xb_mean = R.xb_mean.data(); r.beta_star = R.beta_star.data();
         r.residuals_b = R.residuals.data();
         r.std_err = se.data(); r.p_value = pv.data(); r.ci_lower = lo.data(); r.ci_upper = hi.data(); r.t_stat = t.data();
-        check(g.ctx, cache.c ? ob_bootstrap_run_cached(g.ctx, g.des, &o, cache.c, &r) : ob_bootstrap_run(g.ctx, g.des, &o, &r));
+        if (bayesian_) check(g.ctx, ob_bootstrap_run_bayes(g.ctx, g.des, &o, nullptr, cache.c, &r));
+        else check(g.ctx, cache.c ? ob_bootstrap_run_cached(g.ctx, g.des, &o, cache.c, &r) : ob_bootstrap_run(g.ctx, g.des, &o, &r));
 
         R.bootstrap_reps = (int64_t)bootstrap_reps_;
         R.successful_bootstraps = r.n_ok;
@@ -637,6 +638,7 @@ std::vector<OaxacaResults> OaxacaBuilder::run_impl(bool rif, double tau, const s
         R.predictor_names = has_selection_ ? rows : p.names;
         R.ms_total = r.ms_total; R.ms_gram = r.ms_gram;
         R.cluster_strata = cl_strata; R.cluster_units_a = cl_ua; R.cluster_units_b = cl_ub;
+        R.bayesian = bayesian_;
         all.push_back(std::move(R));
     }
     return all;
@@ -724,6 +726,7 @@ void OaxacaResults::summary(std::ostream& os) const {   // display.rs:9-79
         os << "Cluster bootstrap (by group): " << cluster_units_a << " units in A, " << cluster_units_b << " in B\n";
     else if (cluster_strata == OB_CLUSTER_JOINT)
         os << "Cluster bootstrap (joint): " << cluster_units_a << " units\n";
+    if (bayesian) os << "Bootstrap scheme: Bayesian (Dirichlet row weights)\n";
     os << "Total Gap: " << fmt(total_gap, 4) << "\n\n";
     os << "Two-Fold Decomposition\n";
     table(os, "Component", "Estimate", two_fold.aggregate);
@@ -775,6 +778,7 @@ std::string OaxacaResults::to_json(bool with_residuals, bool with_extra) const {
     if (cluster_strata != OB_CLUSTER_NONE)
         os << ",\"clusters\":{\"strata\":\"" << (cluster_strata == OB_CLUSTER_JOINT ? "joint" : "group") << "\",\"units_a\":"
            << cluster_units_a << ",\"units_b\":" << cluster_units_b << '}';
+    if (bayesian) os << ",\"bootstrap_scheme\":\"bayes\"";
     if (with_residuals) { os << ",\"residuals\":"; jvec(os, residuals); }
     if (with_extra) {   // #[serde(skip)] fields + replicate bookkeeping, for the Python mirror and tests
         os << ",\"xa_mean\":"; jvec(os, xa_mean); os << ",\"xb_mean\":"; jvec(os, xb_mean);

@@ -70,6 +70,7 @@ struct OaxacaResults {     // types.rs:24-47
     // cluster bootstrap (OaxacaBuilder::cluster): ob_cluster_strata and the units resampled per replicate (JOINT: a == b)
     int cluster_strata = OB_CLUSTER_NONE;
     int64_t cluster_units_a = 0, cluster_units_b = 0;
+    bool bayesian = false;     // OaxacaBuilder::bayesian_bootstrap: Dirichlet-weighted replicates
 
     void summary(std::ostream& os) const;                          // display.rs:9-79
     std::string to_json(bool with_residuals, bool with_extra) const;   // display.rs to_json (serde layout) [+ extras]
@@ -115,6 +116,10 @@ public:
         cluster_col_ = strata == OB_CLUSTER_NONE ? std::string() : column; cluster_strata_ = strata; return *this;
     }
 
+    // Bayesian bootstrap (ob_bootstrap_run_bayes): every row keeps a Dirichlet weight in every replicate instead of a
+    // multinomial count; run, run_outcomes and decompose_quantile honour it
+    OaxacaBuilder& bayesian_bootstrap(bool on = true) { bayesian_ = on; return *this; }
+
     OaxacaResults run() const;                              // builder.rs:787-951
     // run() once per listed outcome column on one ingest: rows are cleaned over all of them, the first run fills a Gram
     // cache and the others only contract their outcome columns (ob_bootstrap_run_cached)
@@ -140,6 +145,7 @@ private:
     bool has_weights_ = false, has_selection_ = false;
     std::string cluster_col_;
     int cluster_strata_ = OB_CLUSTER_NONE;
+    bool bayesian_ = false;
     uint64_t seed_ = 0x0B5EEDull;
     int device_ = 0;
     const uint32_t* idx_a_ = nullptr;

@@ -116,6 +116,7 @@ ob_status ob_builder_cluster(ob_builder* b, const char* column, int32_t strata) 
     if (strata < OB_CLUSTER_NONE || strata > OB_CLUSTER_JOINT || (strata != OB_CLUSTER_NONE && !column)) return OB_ERR_INVALID_ARG;
     return guarded(b, [&] { b->b->cluster(column ? column : "", strata); });
 }
+ob_status ob_builder_bayesian(ob_builder* b, int32_t on) { return guarded(b, [&] { b->b->bayesian_bootstrap(on != 0); }); }
 ob_status ob_builder_seed(ob_builder* b, uint64_t seed) { return guarded(b, [&] { b->b->seed(seed); }); }
 ob_status ob_builder_device(ob_builder* b, int32_t device) { return guarded(b, [&] { b->b->device(device); }); }
 ob_status ob_builder_index_stream(ob_builder* b, const uint32_t* idx_a, const uint32_t* idx_b) {

@@ -56,6 +56,7 @@ static void usage() {
         "      --seed <N>                     Resampling seed\n"
         "      --cluster <COLUMN>             Cluster bootstrap: resample whole clusters of COLUMN instead of rows\n"
         "      --cluster-strata <MODE>        group (default: each group resamples its own clusters) | joint (one stratum)\n"
+        "      --bootstrap-scheme <SCHEME>    multinomial (default: resample rows) | bayes (Bayesian bootstrap: Dirichlet row weights)\n"
         "      --output-json <PATH>           Export results as JSON\n"
         "      --output-markdown <PATH>       Export results as Markdown\n";
 }
@@ -77,7 +78,16 @@ int main(int argc, char** argv) {
     double tau = 0.0;
     std::vector<double> quantiles = {0.1, 0.25, 0.5, 0.75, 0.9};                          // main.rs:236-239
     int cluster_strata = OB_CLUSTER_BY_GROUP;
+    bool bayesian = false;
     try {
+        if (a.count("bootstrap-scheme")) {
+            const std::string& bs = a["bootstrap-scheme"];
+            if (bs == "bayes") bayesian = true;
+            else if (bs != "multinomial")
+                throw ArgError{"invalid value '" + bs + "' for '--bootstrap-scheme <SCHEME>'\n  [possible values: multinomial, bayes]"};
+            if (bayesian && a["analysis-type"] == "quantile")
+                throw ArgError{"'--bootstrap-scheme bayes' applies to the mean and RIF decompositions, not to '--analysis-type quantile'"};
+        }
         if (a.count("cluster-strata")) {
             const std::string& cs = a["cluster-strata"];
             if (cs == "group") cluster_strata = OB_CLUSTER_BY_GROUP;
@@ -139,6 +149,7 @@ int main(int argc, char** argv) {
         if (a.count("normalize")) b.normalize(split_commas(a["normalize"]));
         if (a.count("seed")) b.seed(seed);
         if (a.count("cluster")) b.cluster(a["cluster"], cluster_strata);
+        if (bayesian) b.bayesian_bootstrap(true);
         if (a.count("selection-outcome")) b.heckman_selection(a["selection-outcome"], split_commas(a["selection-predictors"]));
         const ob::OaxacaResults r = a.count("rif-quantile") ? b.decompose_quantile(tau) : b.run();
         r.summary(std::cout);

@@ -123,6 +123,23 @@ size_t counts_lut_bytes();
 void counts_philox_body_launch(const CountsArgs& a, long long* d_colsum, unsigned char* d_lut, cudaStream_t st);
 void counts_philox_fixup_launch(const CountsArgs& a, const long long* d_colsum, int* d_flags, cudaStream_t st);
 
+// Bayesian bootstrap (Rubin 1981): C [panels][n_pad][BM] of fp32 E_i ~ iid Exp(1) per (row, replicate) -- the point slot
+// holds 1.0 on valid rows, padding rows and slots outside [first_slot, slots) hold 0 -- and part [segs][panels*BM]: each
+// (leaf segment, slot)'s sum of E in a fixed order (leaf_sum_launch then sums the leaves by the Gram's aligned tree).  Native
+// stream: E = -log U, U in (0, 1) from Philox4x32-10 keyed by (seed; global row, group, global replicate id, stream tag);
+// explicit stream: wt [replicates of the batch][n_global], the caller's E in the group's row order.
+struct BayesArgs {
+    float* C; int64_t n, n_pad; int panels;      // rows held here
+    int64_t n_global, row_begin;
+    int64_t slots; int first_slot; int64_t rep0; // as CountsArgs
+    int group; uint64_t seed;
+    int segs, seg_rows;                          // leaves held here (RowShard) and rows per leaf
+    const float* wt;                             // explicit stream on the device, or null (native)
+    double* part;                                // [segs][panels * BM]
+    int* flags = nullptr;                        // flags[3] |= 1: an explicit weight that is not a positive normal float
+};
+void bayes_weights_launch(const BayesArgs& a, cudaStream_t st);
+
 // ---- cluster.cu ----
 // attach: uid[row] = codes_frame[src[row]], present[code] = 1 (d_flags[0] |= 1 on a code outside [0, n_codes)); then
 // unit[code] = exclusive scan of present (*d_units = the stratum's unit count); then uid[row] = unit[uid[row]]
@@ -203,7 +220,8 @@ inline int gram_pld(int K, int T) { return (int)((num_pairs(K, T) + BQ - 1) / BQ
 GramPlan gram_make_plan(int K, int T, int ldx, int panels, const GroupData g[2], int count_bytes, int num_sms,
                         const GramColumns& cols);
 // whether the Gram CTA fits in shared memory at design row stride ldx with count_bytes-wide multiplicities: always at
-// 8-bit (K + outcomes <= 280), up to ldx 268 at 16-bit.  The drivers refuse or stop widening where it does not.
+// 8-bit (K + outcomes <= 280), up to ldx 268 at 16-bit, up to ldx 236 with fp32 Bayesian weights (count_bytes 4).  The
+// drivers refuse or stop widening where it does not.
 bool gram_fits(int ldx, int count_bytes);
 struct GramArgs {
     const double* X[2]; const void* C[2];     // X: the (sqrt(w)-scaled when weighted) design
@@ -221,6 +239,9 @@ void gram_launch(const GramPlan& plan, const GramArgs& args, cudaStream_t st, cu
 // fixed-tree reduction of the partial tiles (once every leaf has been contracted)
 void gram_launch_leaves(const GramPlan& plan, const GramArgs& args, const int seg_lo[2], const int seg_n[2], cudaStream_t st);
 void gram_reduce_launch(const GramPlan& plan, const GramArgs& args, cudaStream_t st);
+// out [2][slots_pad] = per slot, the aligned-tree sum of part [segs[0] + segs[1]][slots_pad] over each group's leaves held
+// here (span = MAX_SEGS / world); mode N then combines the per-rank sums with gram_combine_launch
+void leaf_sum_launch(const double* part, const int segs[2], int64_t slots_pad, int span, double* out, cudaStream_t st);
 // mode N: gram = aligned-tree sum over ranks of gathered [world][2][slots_pad*Pld] per-rank sums; ranks_with_rows[g]
 // = number of leading ranks that hold leaves of group g
 void gram_combine_launch(const double* gathered, int world, const int ranks_with_rows[2], int64_t per_group_elems,
@@ -239,6 +260,7 @@ struct SolveArgs {
     int weighted;
     double na, nb;           // group row counts (n_obs)
     const long long* rows = nullptr;   // clustered designs: [2][slots_pad] row counts per slot (replace na / nb), else null
+    const double* esum = nullptr;      // Bayesian bootstrap: [2][slots_pad] sums of the raw weights E per slot, else null
     // outputs
     double* stats;           // [slots][S]
     int* status;             // [slots]

@@ -20,6 +20,7 @@
 //               reference's unweighted means require (estimation.rs:66, ols.rs:83).
 //      Every draw is keyed by global ids, so counts do not depend on grid shape, batch split or on
 //      how replicates/rows are sharded over GPUs.
+//  (c) bayes_weights: the Bayesian bootstrap's fp32 weights E_i ~ Exp(1) in the same layout (see BayesArgs).
 #include "common.cuh"
 #include "internal.h"
 
@@ -259,6 +260,96 @@ __global__ void __launch_bounds__(256) counts_index_kernel(CountT* __restrict__ 
         if (row < 0 || row >= n) continue;             // drawn row lives on another GPU
         if (bump_count<CountT>(C, (panel * n_pad + row) * BM + col)) atomicOr(&flags[1], 1);
     }
+}
+
+// ---- Bayesian bootstrap weights ----
+constexpr uint32_t STREAM_BAYES = 0x0BA7E5u;
+
+// E = -log U with U = (u >> 9 + 1/2) 2^-23 in [2^-24, 1 - 2^-24]: exact in fp32, open at both ends, so E is a positive
+// normal float (5.96e-8 <= E <= 16.6)
+__device__ __forceinline__ float exp1_from_u32(uint32_t u) {
+    return -logf(((float)(u >> 9) + 0.5f) * 0x1p-23f);
+}
+
+// Block = (leaf segment held here, panel); thread = (row lane rl = tid / 32, slot quad q = tid % 32): rows rl, rl + 8, ..
+// of the leaf, slots 4q .. 4q + 3 of the panel (one 16-byte store per row).  Replicate r draws the 32-bit word of stream
+// id sid = r + 1 (the slot of r when unsharded) from the Philox call keyed by sid / 4; SH = sid of the thread's first
+// slot mod 4, uniform over the launch: the thread's four slots span one (SH == 0) or two calls.  Each (leaf, slot) sum
+// adds the thread's rows in order, then the eight row lanes in order: fixed by the leaf alone.
+template <int SH, bool EXPLICIT>
+__global__ void __launch_bounds__(256) bayes_weights_kernel(const BayesArgs a, uint32_t k0, uint32_t k1) {
+    __shared__ double red[8][BM];
+    const int leaf = blockIdx.x, panel = blockIdx.y;
+    const int q = threadIdx.x & 31, rl = threadIdx.x >> 5;
+    const long long slot0 = (long long)panel * BM + 4 * q;
+    const long long r_lo = (long long)leaf * a.seg_rows;
+    const long long r_hi = r_lo + a.seg_rows < a.n_pad ? r_lo + a.seg_rows : a.n_pad;
+    unsigned valid = 0;
+#pragma unroll
+    for (int e = 0; e < 4; ++e)
+        if (slot0 + e >= a.first_slot && slot0 + e < a.slots) valid |= 1u << e;
+    const bool point_slot = slot0 == 0 && a.first_slot == 1;
+    const long long quad0 = (a.rep0 + 1 + slot0 - SH) >> 2;
+    constexpr int NQ = SH ? 2 : 1;
+    const uint32_t c1base = (uint32_t)a.group << 8;
+    double acc[4] = {0.0, 0.0, 0.0, 0.0};
+    for (long long row = r_lo + rl; row < r_hi; row += 8) {
+        float E[4] = {0.f, 0.f, 0.f, 0.f};
+        if (row < a.n) {
+            const unsigned long long grow = (unsigned long long)(row + a.row_begin);   // keyed by the GLOBAL row
+            if (EXPLICIT) {
+#pragma unroll
+                for (int e = 0; e < 4; ++e) {
+                    if (!(valid & (1u << e))) continue;
+                    E[e] = a.wt[(size_t)(slot0 + e - a.first_slot) * a.n_global + grow];
+                    // the Gram kernel widens positive normal floats only; a caller's zero, denormal, negative, inf or NaN
+                    // fails the call
+                    if (!(E[e] >= 1.17549435e-38f && E[e] <= 3.40282347e38f)) { atomicOr(&a.flags[3], 1); E[e] = 0.f; }
+                }
+            } else if (valid) {
+                const uint32_t c1 = c1base | (uint32_t)(grow >> 32);
+                uint32_t w[4 * NQ];
+#pragma unroll
+                for (int h = 0; h < NQ; ++h) {
+                    const long long qd = quad0 + h;
+                    const Philox4 r = philox4x32_10((uint32_t)grow, c1, (uint32_t)qd, STREAM_BAYES ^ (uint32_t)((unsigned long long)qd >> 32), k0, k1);
+                    w[4 * h] = r.x; w[4 * h + 1] = r.y; w[4 * h + 2] = r.z; w[4 * h + 3] = r.w;
+                }
+#pragma unroll
+                for (int e = 0; e < 4; ++e) E[e] = (valid & (1u << e)) ? exp1_from_u32(w[SH + e]) : 0.f;
+            }
+            if (point_slot) E[0] = 1.f;
+        }
+        *reinterpret_cast<float4*>(a.C + ((long long)panel * a.n_pad + row) * BM + 4 * q) = make_float4(E[0], E[1], E[2], E[3]);
+#pragma unroll
+        for (int e = 0; e < 4; ++e) acc[e] += (double)E[e];
+    }
+#pragma unroll
+    for (int e = 0; e < 4; ++e) red[rl][4 * q + e] = acc[e];
+    __syncthreads();
+    if (threadIdx.x < BM) {
+        double s = red[0][threadIdx.x];
+#pragma unroll
+        for (int l = 1; l < 8; ++l) s += red[l][threadIdx.x];
+        a.part[(size_t)leaf * a.panels * BM + (size_t)panel * BM + threadIdx.x] = s;
+    }
+}
+
+void bayes_weights_launch(const BayesArgs& a, cudaStream_t st) {
+    if (a.segs <= 0 || a.panels <= 0) return;
+    const uint32_t k0 = (uint32_t)a.seed, k1 = (uint32_t)(a.seed >> 32);
+    const dim3 grid((unsigned)a.segs, (unsigned)a.panels);
+    if (a.wt) {
+        bayes_weights_kernel<0, true><<<grid, 256, 0, st>>>(a, k0, k1);
+    } else {
+        switch ((int)(((a.rep0 + 1) % 4 + 4) % 4)) {
+        case 0: bayes_weights_kernel<0, false><<<grid, 256, 0, st>>>(a, k0, k1); break;
+        case 1: bayes_weights_kernel<1, false><<<grid, 256, 0, st>>>(a, k0, k1); break;
+        case 2: bayes_weights_kernel<2, false><<<grid, 256, 0, st>>>(a, k0, k1); break;
+        default: bayes_weights_kernel<3, false><<<grid, 256, 0, st>>>(a, k0, k1); break;
+        }
+    }
+    OB_CUDA(cudaGetLastError());
 }
 
 void counts_clear(const CountsArgs& a, cudaStream_t st) {

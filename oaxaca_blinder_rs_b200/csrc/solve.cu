@@ -27,6 +27,7 @@ struct SolveParams {
     int n_base, S, weighted;
     double na, nb;
     const long long* rows;   // [2][slots_pad] per-slot group row counts (clustered designs), null: na / nb
+    const double* esum;      // [2][slots_pad] per-slot sums of the raw Bayesian weights E, null: multiplicities
     double* stats; int* status; double* beta_a; double* beta_b; double* point_extra;
     double* gscratch;        // per-slot matrix buffer in global memory when it does not fit shared memory, else null
 };
@@ -155,6 +156,11 @@ __global__ void __launch_bounds__(SOLVE_THREADS) solve_kernel(const SolveParams 
         else if (na <= (double)K) status = OB_ERR_INSUFFICIENT_DATA;
     } else if (na <= (double)K || nb <= (double)K) status = OB_ERR_INSUFFICIENT_DATA;
     const int ind = 1 + p.n_cont;       // builder.rs:548-566: position of the group indicator in the pooled design
+    // Bayesian bootstrap: the Gram holds sums over raw weights E; the replicate's weights are pi = n_g E / sum_g E.  beta
+    // and the means of one group do not change when its weights scale by a common factor; where the groups meet (the
+    // stacked Pooled system, the weighted Cotton / Weighted omega) each group's cells are scaled by s_g = n_g / sum_g E.
+    double sA = 1.0, sB = 1.0;
+    if (p.esum) { sA = na / p.esum[slot]; sB = nb / p.esum[p.slots_pad + slot]; }
 
     for (int sys = 0; sys < (pooled ? 3 : 2); ++sys) {
         const int N = sys == 2 ? Kp : K, ldm = sys == 2 ? ldp : ld;
@@ -186,14 +192,17 @@ __global__ void __launch_bounds__(SOLVE_THREADS) solve_kernel(const SolveParams 
                 if (i == ind && j == ind) v = gA[0];
                 else if (i == ind) v = gA[sj];        // sum over A rows of w * 1 * x_sj
                 else if (j == ind) v = gA[si];
-                else v = gsym(gA, K, T, si, sj) + gsym(gB, K, T, si, sj);
+                else v = p.esum ? sA * gsym(gA, K, T, si, sj) + sB * gsym(gB, K, T, si, sj) : gsym(gA, K, T, si, sj) + gsym(gB, K, T, si, sj);
+                if (p.esum && (i == ind || j == ind)) v *= sA;
                 M[i * ldm + j] = v;
             }
             for (int e = tid; e < T * Kp; e += blockDim.x) {
                 const int t = e / Kp, i = e - t * Kp;
                 const int si = i < ind ? i : i - 1;
                 const long long ya = gidx(K, T, 0, 0) + K + t;             // (0, y_t): sum over A rows of w y_t
-                B[e] = (i == ind) ? gA[ya] : gA[gidx(K, T, si, si) + (K - si) + t] + gB[gidx(K, T, si, si) + (K - si) + t];
+                const double a = gA[gidx(K, T, si, si) + (K - si) + t], b = gB[gidx(K, T, si, si) + (K - si) + t];
+                if (p.esum) B[e] = (i == ind) ? sA * gA[ya] : sA * a + sB * b;
+                else B[e] = (i == ind) ? gA[ya] : a + b;
             }
         }
         __syncthreads();
@@ -229,8 +238,8 @@ __global__ void __launch_bounds__(SOLVE_THREADS) solve_kernel(const SolveParams 
                 break;
             }
             default: {  // Weighted | Cotton: builder.rs:591-620
-                const double n_a = p.weighted ? sums[0] : na;
-                const double n_b = p.weighted ? sums[2] : nb;
+                const double n_a = p.weighted ? (p.esum ? sA * sums[0] : sums[0]) : na;
+                const double n_b = p.weighted ? (p.esum ? sB * sums[2] : sums[2]) : nb;
                 const double total = n_a + n_b;
                 if (total == 0.0) { st_t = OB_ERR_INVALID_GROUP; break; }
                 const double wA = n_a / total, wB = 1.0 - wA;
@@ -309,7 +318,7 @@ void solve_launch(const SolveArgs& a, cudaStream_t st) {
     p.K = a.K; p.n_cont = a.n_cont; p.ref_kind = a.ref_kind; p.T = a.T;
     p.n_norm = a.n_norm; p.norm_m = a.d_norm_m; p.norm_off = a.d_norm_off; p.norm_idx = a.d_norm_idx;
     p.norm_has_base = a.d_norm_has_base; p.n_base = a.n_base; p.S = a.S; p.weighted = a.weighted;
-    p.na = a.na; p.nb = a.nb; p.rows = a.rows;
+    p.na = a.na; p.nb = a.nb; p.rows = a.rows; p.esum = a.esum;
     p.stats = a.stats; p.status = a.status; p.beta_a = a.beta_a; p.beta_b = a.beta_b; p.point_extra = a.point_extra;
     const bool pooled = a.ref_kind == OB_REF_POOLED;
     const bool global = solve_scratch_bytes(a.K, pooled, a.n_norm, a.T, 1) != 0;
