@@ -371,7 +371,10 @@ ob_status ob_reduce_stats(ob_ctx* ctx, const double* rep_stats, const int32_t* r
  * builder has neither weights nor a RIF), K <= 47 columns; row-sharded designs are refused.
  * Test-only explicit streams (the reference's are unseeded thread_rng draws): idx_a / idx_b as in ob_boot_opts; taus
  * [(reps + 1) x simulations], pass 0 = point estimates; draw_a / draw_b [(reps + 1) x simulations] = position of the
- * simulated row in the pass's (resampled) group frame (needs idx_* when reps > 0).  NULL = native Philox streams. */
+ * simulated row in the pass's (resampled) group frame (needs idx_* when reps > 0).  NULL = native Philox streams.
+ * idx_* without draw_a / draw_b: the simulated rows are drawn natively against the explicit multiplicities, which is
+ * exact (row i with probability c_i / n) only while every multiplicity is <= 64; a replicate of [rep_begin, rep_end)
+ * that draws a row more than 64 times is refused with OB_ERR_UNSUPPORTED (pass draw_a / draw_b with such streams). */
 typedef struct ob_mm_opts {
     int32_t simulations;             /* builder default 200 (quantile_decomposition.rs:58), <= 4096 */
     int32_t n_quantiles;

@@ -1922,6 +1922,25 @@ void mm_run(ob_ctx* ctx, const ob_design* d, const ob_mm_opts* o, ob_mm_result* 
     if (draws_given && (!o->draw_a || !o->draw_b)) fail(OB_ERR_INVALID_ARG, "simulated-row stream needs both draw_a and draw_b");
     if (draws_given && rr.nrep > 0 && !rr.index_mode)
         fail(OB_ERR_INVALID_ARG, "draw_a / draw_b are positions in the resampled frames: they need the explicit resample stream idx_a / idx_b");
+    // Without draw_a / draw_b the simulated rows of an explicit resample are drawn natively (mm_streams_kernel), by
+    // rejection with acceptance min(c_i, 64) / 64: that is row i with probability c_i / n only while every multiplicity is
+    // <= 64.  Native multiplicities never get there; an explicit stream that does is refused.
+    if (rr.index_mode && !draws_given) {
+        for (int g = 0; g < 2; ++g) {
+            const uint32_t* ix = g == 0 ? o->idx_a : o->idx_b;
+            const int64_t n = d->g[g].n;
+            std::vector<uint32_t> cnt((size_t)n);
+            for (int64_t r = rr.rb; r < rr.re; ++r) {
+                std::fill(cnt.begin(), cnt.end(), 0u);
+                for (int64_t i = 0; i < n; ++i) {
+                    const uint32_t row = ix[(size_t)r * n + i];
+                    if (row < n && ++cnt[row] > 64)
+                        fail(OB_ERR_UNSUPPORTED, "an explicit resample draws a row more than 64 times: the native simulated-row "
+                                                 "draw is exact only up to 64; pass draw_a / draw_b explicitly");
+                }
+            }
+        }
+    }
     for (int q = 0; q < nq; ++q)
         if (!(o->quantiles[q] >= 0.0 && o->quantiles[q] <= 1.0)) fail(OB_ERR_INVALID_ARG, "target quantiles must lie in [0, 1]");
     int count_bytes = rr.count_bytes;
